@@ -18,7 +18,9 @@ Input bytes are the synthetic source's xorshift stream, a pure function of
           compared (a) for sweep 0 alone with the reference-generated known-answer hash of
           SURVEY.md 8(c) and (b) for the whole interval with a 1-rank run of the same bytes.
   value : inputs already resident in HBM, CUDA-event timed on the launching stream,
-          max over ranks; rounds of --steps steps are repeated until >= 50 ms are timed.
+          max over ranks, over exactly --steps steps.
+  --dump-outputs DIR: the report of the last timed step (what a caller of the timed path
+          receives) as DIR/avg.npy, db.npy, samples.npy in float64 (about 32 MiB in all).
   e2e   : the same interval through the public C ABI with HOST buffers:
           rtlsdr_gpu_scan_submit_batch() from pinned memory (H2D inside the timed
           region), the exchange, and the gathered report copied to host memory on rank 0.
@@ -37,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the bench leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -295,9 +298,10 @@ class ShardedSweep:
         self.pinned.free()
 
 
-def time_device(D, sw, steps, warmup, min_ms=MIN_TIMED_MS, sampler=None):
+def time_device(D, sw, steps, warmup, min_ms=MIN_TIMED_MS, sampler=None, last=None):
     """rounds of exactly `steps` device-resident steps, CUDA events on the launching stream, max over ranks;
-    repeated until >= min_ms have been timed.  Returns (ms_per_step, timed_steps, kernel_ms, kernel_launches, launches)."""
+    repeated until >= min_ms have been timed (min_ms = 0: one round).  Returns (ms_per_step, timed_steps, kernel_ms,
+    kernel_launches, launches, issue_ms).  last: a list that receives rank 0's report of the last timed step."""
     torch = D.torch
     for i in range(warmup):
         sw.step_device(i)
@@ -333,6 +337,9 @@ def time_device(D, sw, steps, warmup, min_ms=MIN_TIMED_MS, sampler=None):
     s1 = sw.g.stats()
     k_ms, k_n = sw.g.kernel_time()
     sw.g.set_timing(0)
+    if last is not None and D.rank == 0:
+        # before the sampler's untimed launches below rewrite report buffer 0
+        last.append(device_report(sw.gather, (i0 - 1) & 1))
     if sampler:
         # nvidia-smi ticks every 10 ms: keep the same kernels running on THIS rank, untimed and WITHOUT the
         # exchange (a collective that the other ranks do not join would never complete), until a few clock
@@ -345,6 +352,22 @@ def time_device(D, sw, steps, warmup, min_ms=MIN_TIMED_MS, sampler=None):
             torch.cuda.synchronize()
     return (total_ms / (rounds * steps), rounds * steps, k_ms / max(k_n, 1), k_n,
             s1["kernel_launches"] - s0["kernel_launches"], D.max(issue_ms))
+
+
+def device_report(gather, k):
+    """rank 0, after a synchronise: the gathered report in exchange buffer k where the device left it (timed steps
+    publish without the copy to pinned host memory that fetch() reads)"""
+    bufs = gather.send[k].view(1, gather.words) if gather.world == 1 else gather.recv[k]
+    return gather.unpack(bufs.cpu().numpy())
+
+
+def dump_outputs(path, rep):
+    """avg (int64 bins, exact in float64 below 2^53), db and samples of one report as float64 .npy files"""
+    import numpy as np
+    assert int(np.abs(rep.avg).max()) < 1 << 53, "bins beyond float64's exact integers"
+    os.makedirs(path, exist_ok=True)
+    for name in ("avg", "db", "samples"):
+        np.save(os.path.join(path, f"{name}.npy"), getattr(rep, name).astype(np.float64))
 
 
 def verify_sharded(D, sw, kat_p1, full_interval=True):
@@ -660,8 +683,12 @@ def run_gpu(args):
     sw = ShardedSweep(D, rs, RANGE, CROP, WINDOW, FIR, args.sweeps)
     verify = verify_sharded(D, sw, KAT_P1)
     sampler = ClockSampler(D.local) if D.rank == 0 else None
-    ms_step, timed_steps, k_ms, k_n, launches, issue_ms = time_device(D, sw, args.steps, args.warmup, sampler=sampler)
+    last = []
+    ms_step, timed_steps, k_ms, k_n, launches, issue_ms = time_device(D, sw, args.steps, args.warmup, min_ms=0.0,
+                                                                      sampler=sampler, last=last)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
     # ---- end to end from host buffers: hop shares proportional to each GPU's host-to-device bandwidth ----
     e2e_steps = max(4, min(args.steps, 24))
     h2d = probe_h2d(D)
@@ -722,8 +749,7 @@ def run_gpu(args):
                        "input": "synthetic source xorshift stream, bytes a pure function of (hop, sweep): "
                                 "identical job at every N",
                        "cache": f"inputs larger than L2: every step streams this rank's whole {sw.bytes_rank >> 20} MiB cube from HBM",
-                       "timing": f"rounds of {args.steps} steps repeated until >= {MIN_TIMED_MS:.0f} ms "
-                                 f"({timed_steps} steps timed)",
+                       "timing": f"{timed_steps} steps between two CUDA events",
                        "exchange": sw.gather.describe(), "host_pinning": pin},
             "per_gpu_value": value / D.world,
             "host_issue_ms_per_step": issue_ms,
@@ -822,14 +848,18 @@ def pin_to_gpu_numa(gpu_index):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of the headline workload")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="graft", choices=["graft", "reference"])
     ap.add_argument("--sweeps", type=int, default=SWEEPS,
                     help="sweeps per step (default = the benchmark's 256; tests shrink it, the line says so)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-companions", action="store_true", help="skip the other-configuration measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's report of the last timed step to DIR/{avg,db,samples}.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)

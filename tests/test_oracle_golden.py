@@ -74,7 +74,7 @@ def test_rms(port_oracle, gold):
 
 
 def test_scans_and_csv_rows(port_oracle, gold):
-    """whole hop visits + the text rows csv_dbm printed for them"""
+    """whole hop visits + the text rows csv_dbm printed for them; the host planner's whole plan == the reference's"""
     from rtlsdr_b200.planner import plan_scan
     vec, meta = gold
     for c in meta["scan"]:
@@ -86,20 +86,22 @@ def test_scans_and_csv_rows(port_oracle, gold):
         assert np.array_equal(avg, vec[c["key"] + "_avg"]), c["freq"]
         assert np.array_equal(smp, vec[c["key"] + "_samples"])
         p = plan_scan(c["freq"], c["crop"], None if c["fir"] < 0 else c["fir"])
-        assert p.as_dict()["freqs"] == plan["freqs"]
+        mine = p.as_dict()
+        for k, v in c["plan"].items():
+            assert mine[k] == v, (c["freq"], k, mine[k], v)
         for h in range(plan["tune_count"]):
             assert p.csv_row(h, int(smp[h]), db[h]) == c["csv"][h], (c["freq"], h)
 
 
 def test_known_answer_hashes(port_oracle):
-    """SURVEY.md 8(c) rows (cheap ones on CPU; the GPU suite runs all of them)."""
+    """SURVEY.md 8(c) rows, all of them (about a second of CPU): the 2^17-bin row checks the restatement's large
+    fix_fft, the 512 / 623-hop rows the wideband plans, against the reference's own bins."""
     from rtlsdr_b200.planner import plan_scan
     with open(os.path.join(GOLD, "kat.json")) as f:
         kat = json.load(f)
+    assert len(kat) == 11
     for c in kat:
         plan = plan_scan(c["freq"], c["crop"], None if c["fir"] < 0 else c["fir"]).as_dict()
-        if plan["tune_count"] > 16 or plan["bin_e"] > 12:
-            continue
         plan["peak_hold"] = c["peak"]
         w = port_oracle.window_coefs(c["window"], 1 << plan["bin_e"])
         reads, hops = make_reads(port_oracle.lib, plan, c["passes"], c["mode"], 0, 0)
