@@ -423,6 +423,26 @@ struct TwSmall {
 	}
 };
 
+/* the compact twiddles and the window -> shared memory, shared by the threads t = 0, 1, .. stride-1: asynchronous
+ * 16-byte copies (the host pre-arranges the per-stage compact twiddle layout), so the caller's first input copies
+ * overlap them; the caller waits for them and puts a barrier before the first use */
+template <int L>
+SCAN_DEV void load_tables(int2 *tws, uint16_t *wins, const int2 *twc, const uint16_t *win, int t, int stride)
+{
+	constexpr int N = 1 << L;
+	if constexpr (N > 16) {
+		for (int i = t; i < (N - 16) / 2; i += stride)
+			cp_async16((uint8_t *)tws + 16 * i, (const uint8_t *)twc + 16 * i);
+	}
+	if constexpr (N >= 8) {
+		for (int i = t; i < N / 8; i += stride)
+			cp_async16((uint8_t *)wins + 16 * i, (const uint8_t *)win + 16 * i);
+	} else {
+		for (int i = t; i < N; i += stride)
+			wins[i] = win[i];
+	}
+}
+
 SCAN_DEV long long entry_offset(const SmallParams &prm, int e)
 {
 	return prm.read_off ? prm.read_off[e] : (long long)(e - prm.entry_base) * prm.regular_stride;
@@ -532,10 +552,12 @@ SCAN_DEV void front_u8(X2 (&x)[kPts], const uint8_t *st, int ws, int kI, int kQ,
 	}
 }
 
-/* one hop's sums / peaks of this CTA -> tunes[hop].avg (64-bit RED); `bins` = N x u64 of shared memory that no
- * thread is using (only touched when N < 4096, where several registers of the CTA share a bin) */
-template <int L, bool PEAK>
-SCAN_DEV void flush_bins(unsigned long long (&acc)[kPts], long long *out, unsigned long long *bins, int t)
+/* one hop's sums / peaks of the kThreads transform threads synchronised by `bar` -> tunes[hop].avg (64-bit RED);
+ * `bins` = N x u64 of shared memory that none of them is using (only touched when N < 4096, where several
+ * registers share a bin) */
+template <int L, bool PEAK, class BAR = BlockBar>
+SCAN_DEV void flush_bins(unsigned long long (&acc)[kPts], long long *out, unsigned long long *bins, int t,
+			 const BAR &bar = BAR())
 {
 	constexpr int N = 1 << L;
 	if constexpr (L == 12) {
@@ -548,10 +570,10 @@ SCAN_DEV void flush_bins(unsigned long long (&acc)[kPts], long long *out, unsign
 				atomicAdd((unsigned long long *)(out + bin), acc[r]);
 		}
 	} else {
-		__syncthreads();
+		bar.sync();
 		for (int i = t; i < N; i += kThreads)
 			bins[i] = 0ull;
-		__syncthreads();
+		bar.sync();
 #pragma unroll
 		for (int r = 0; r < kPts; ++r) {
 			const int bin = last_pos<L>(t, r) & (N - 1);
@@ -560,14 +582,14 @@ SCAN_DEV void flush_bins(unsigned long long (&acc)[kPts], long long *out, unsign
 			else
 				atomicAdd(bins + bin, acc[r]);
 		}
-		__syncthreads();
+		bar.sync();
 		for (int i = t; i < N; i += kThreads) {
 			if constexpr (PEAK)
 				atomicMax(out + i, (long long)bins[i]);
 			else
 				atomicAdd((unsigned long long *)(out + i), bins[i]);
 		}
-		__syncthreads();
+		bar.sync();
 	}
 }
 
@@ -593,19 +615,7 @@ scan_small_kernel(const SCAN_GRID_CONSTANT SmallParams prm)
 	int *red = (int *)(smem + SM::off_red); /* [8 warps][2] */
 
 	const int t = threadIdx.x;
-	/* tables: asynchronous 16-byte copies (the host pre-arranges the per-stage compact
-	 * twiddle layout), overlapped with the first read's prefetch */
-	if constexpr (N > 16) {
-		for (int i = t; i < (N - 16) / 2; i += kThreads)
-			cp_async16((uint8_t *)tws + 16 * i, (const uint8_t *)prm.twc + 16 * i);
-	}
-	if constexpr (N >= 8) {
-		for (int i = t; i < N / 8; i += kThreads)
-			cp_async16((uint8_t *)wins + 16 * i, (const uint8_t *)prm.win + 16 * i);
-	} else {
-		for (int i = t; i < N; i += kThreads)
-			wins[i] = prm.win[i];
-	}
+	load_tables<L>(tws, wins, prm.twc, prm.win, t, kThreads); /* overlapped with the first read's prefetch */
 
 	TwSmall<L> tw;
 	tw.tws = tws;
@@ -1601,6 +1611,30 @@ struct FusedSmem {
 	static int bytes(int ds, int slots) { return off_stage + slots * 512 * ds; }
 };
 
+/* producer lane of a warp-specialised narrow-scan kernel: the CPR chunks of each of the n reads first, first + 1, ..
+ * go into the ring of nslots slots in order, one bulk copy each; (slot, ph) is the ring position and phase */
+template <int CPR>
+SCAN_DEV void produce_reads(const FusedBoxcarParams &prm, int first, int n, uint8_t *stage, uint64_t *full,
+			    uint64_t *empty, int chunk_bytes, int nslots, int &slot, unsigned &ph)
+{
+	long long off = prm.read_off[first];
+	for (int rd = 0; rd < n; ++rd) {
+		const uint8_t *src = prm.base + off;
+		if (rd + 1 < n)
+			off = prm.read_off[first + rd + 1]; /* in flight while this read's copies are issued */
+		for (int c = 0; c < CPR; ++c) {
+			mbar_wait(empty + slot, ph ^ 1u);
+			mbar_arrive_expect_tx(full + slot, (unsigned)chunk_bytes);
+			bulk_copy_g2s(stage + slot * chunk_bytes, src + (long long)c * chunk_bytes, (unsigned)chunk_bytes,
+				      full + slot);
+			if (++slot == nslots) {
+				slot = 0;
+				ph ^= 1u;
+			}
+		}
+	}
+}
+
 /*
  * Requirements (checked by the host): boxcar, 2 <= ds <= 64, buf_len = 2 * N * ds (so every
  * read is exactly one FFT block and remove_dc covers all of it), 256 <= N <= 4096.
@@ -1628,10 +1662,7 @@ scan_boxcar_fused_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 
 	const int t = threadIdx.x, ds = prm.ds;
 	const int chunk_bytes = 512 * ds;
-	for (int i = t; i < (N - 16) / 2; i += kThreads)
-		cp_async16((uint8_t *)tws + 16 * i, (const uint8_t *)prm.twc + 16 * i);
-	for (int i = t; i < N / 8; i += kThreads)
-		cp_async16((uint8_t *)wins + 16 * i, (const uint8_t *)prm.win + 16 * i);
+	load_tables<L>(tws, wins, prm.twc, prm.win, t, kThreads);
 
 	TwSmall<L> tw;
 	tw.tws = tws;
@@ -1767,39 +1798,8 @@ scan_boxcar_fused_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 		pdl_wait();
 		if (t == 0)
 			atomicAdd((unsigned long long *)(prm.samples + hop), (unsigned long long)((long long)count * ds));
-		long long *out = prm.avg + ((long long)hop << L);
-		if constexpr (L == 12) {
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(t, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(out + bin, (long long)acc[r]);
-				else
-					atomicAdd((unsigned long long *)(out + bin), acc[r]);
-			}
-		} else {
-			unsigned long long *bins = (unsigned long long *)xch; /* 2 * kXchWords * 4 >= N * 8 */
-			__syncthreads();
-			for (int i = t; i < N; i += kThreads)
-				bins[i] = 0ull;
-			__syncthreads();
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(t, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(bins + bin, acc[r]);
-				else
-					atomicAdd(bins + bin, acc[r]);
-			}
-			__syncthreads();
-			for (int i = t; i < N; i += kThreads) {
-				if constexpr (PEAK)
-					atomicMax(out + i, (long long)bins[i]);
-				else
-					atomicAdd((unsigned long long *)(out + i), bins[i]);
-			}
-			__syncthreads();
-		}
+		/* the transpose buffers are idle here: 2 * kXchWords * 4 >= N * 8 */
+		flush_bins<L, PEAK>(acc, prm.avg + ((long long)hop << L), (unsigned long long *)xch, t);
 	}
 }
 
@@ -1947,22 +1947,7 @@ scan_boxcar_stream_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 		unsigned ph = 0;
 		for (int seg = blockIdx.x; seg < prm.n_segs; seg += gridDim.x) {
 			const int4 sg = prm.segs[seg];
-			long long off = prm.read_off[sg.y];
-			for (int rd = 0; rd < sg.z; ++rd) {
-				const uint8_t *src = prm.base + off;
-				if (rd + 1 < sg.z)
-					off = prm.read_off[sg.y + rd + 1]; /* in flight while this read's copies are issued */
-				for (int c = 0; c < CPR; ++c) {
-					mbar_wait(empty + slot, ph ^ 1u);
-					mbar_arrive_expect_tx(full + slot, (unsigned)chunk_bytes);
-					bulk_copy_g2s(stage + slot * chunk_bytes, src + (long long)c * chunk_bytes,
-						      (unsigned)chunk_bytes, full + slot);
-					if (++slot == nslots) {
-						slot = 0;
-						ph ^= 1u;
-					}
-				}
-			}
+			produce_reads<CPR>(prm, sg.y, sg.z, stage, full, empty, chunk_bytes, nslots, slot, ph);
 		}
 		return;
 	}
@@ -2108,41 +2093,9 @@ scan_boxcar_stream_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 		pdl_wait();
 		if (t == 0)
 			atomicAdd((unsigned long long *)(prm.samples + hop), (unsigned long long)((long long)count * ds));
-		long long *out = prm.avg + ((long long)hop << L);
-		if constexpr (L == 12) {
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(tf, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(out + bin, (long long)acc[r]);
-				else
-					atomicAdd((unsigned long long *)(out + bin), acc[r]);
-			}
-		} else {
-			/* both transpose buffers are idle here: every transform thread is past its last exchange
-			 * read once it has passed the first barrier below */
-			unsigned long long *bins = (unsigned long long *)xch; /* 2 * kXchWords * 4 >= N * 8 */
-			fft_bar.sync();
-			for (int i = tf; i < N; i += kThreads)
-				bins[i] = 0ull;
-			fft_bar.sync();
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(tf, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(bins + bin, acc[r]);
-				else
-					atomicAdd(bins + bin, acc[r]);
-			}
-			fft_bar.sync();
-			for (int i = tf; i < N; i += kThreads) {
-				if constexpr (PEAK)
-					atomicMax(out + i, (long long)bins[i]);
-				else
-					atomicAdd((unsigned long long *)(out + i), bins[i]);
-			}
-			fft_bar.sync();
-		}
+		/* both transpose buffers are idle here (2 * kXchWords * 4 >= N * 8): every transform thread is past its
+		 * last exchange read once it has passed the first barrier in flush_bins */
+		flush_bins<L, PEAK, GroupBar>(acc, prm.avg + ((long long)hop << L), (unsigned long long *)xch, tf, fft_bar);
 	}
 }
 
@@ -2257,22 +2210,7 @@ scan_boxcar_sym_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 				if ((wsn & (kSymGroups - 1)) != pg)
 					continue;
 				const int nvalid = (sg.z - rd0 < RPW) ? sg.z - rd0 : RPW;
-				long long off = prm.read_off[sg.y + rd0];
-				for (int rw = 0; rw < nvalid; ++rw) {
-					const uint8_t *src = prm.base + off;
-					if (rw + 1 < nvalid)
-						off = prm.read_off[sg.y + rd0 + rw + 1]; /* in flight while this read's copies are issued */
-					for (int c = 0; c < CPR; ++c) {
-						mbar_wait(empty + slot, ph ^ 1u);
-						mbar_arrive_expect_tx(full + slot, (unsigned)chunk_bytes);
-						bulk_copy_g2s(stage + slot * chunk_bytes, src + (long long)c * chunk_bytes,
-							      (unsigned)chunk_bytes, full + slot);
-						if (++slot == nslots) {
-							slot = 0;
-							ph ^= 1u;
-						}
-					}
-				}
+				produce_reads<CPR>(prm, sg.y + rd0, nvalid, stage, full, empty, chunk_bytes, nslots, slot, ph);
 			}
 		}
 		return;
@@ -2284,10 +2222,7 @@ scan_boxcar_sym_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 	c16 *xch = (c16 *)(smem + SM::off_xch) + fg * 2 * kXchWords;
 	int *red = (int *)(smem + SM::off_red) + fg * 32;
 	const GroupBar bar = { 1 + fg, kThreads };
-	for (int i = t; i < (N - 16) / 2; i += kSymGroups * kThreads)
-		cp_async16((uint8_t *)tws + 16 * i, (const uint8_t *)prm.twc + 16 * i);
-	for (int i = t; i < N / 8; i += kSymGroups * kThreads)
-		cp_async16((uint8_t *)wins + 16 * i, (const uint8_t *)prm.win + 16 * i);
+	load_tables<L>(tws, wins, prm.twc, prm.win, t, kSymGroups * kThreads);
 	cp_async_commit();
 	cp_async_wait_all();
 	named_bar_sync(3, kSymGroups * kThreads); /* tables complete for every worker */
@@ -2390,39 +2325,8 @@ scan_boxcar_sym_kernel(const SCAN_GRID_CONSTANT FusedBoxcarParams prm)
 		pdl_wait();
 		if (t == 0)
 			atomicAdd((unsigned long long *)(prm.samples + hop), (unsigned long long)((long long)count * ds));
-		long long *out = prm.avg + ((long long)hop << L);
-		if constexpr (L == 12) {
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(tf, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(out + bin, (long long)acc[r]);
-				else
-					atomicAdd((unsigned long long *)(out + bin), acc[r]);
-			}
-		} else {
-			unsigned long long *bins = (unsigned long long *)xch; /* 2 * kXchWords * 4 >= N * 8 */
-			bar.sync();
-			for (int i = tf; i < N; i += kThreads)
-				bins[i] = 0ull;
-			bar.sync();
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int bin = last_pos<L>(tf, r) & (N - 1);
-				if constexpr (PEAK)
-					atomicMax(bins + bin, acc[r]);
-				else
-					atomicAdd(bins + bin, acc[r]);
-			}
-			bar.sync();
-			for (int i = tf; i < N; i += kThreads) {
-				if constexpr (PEAK)
-					atomicMax(out + i, (long long)bins[i]);
-				else
-					atomicAdd((unsigned long long *)(out + i), bins[i]);
-			}
-			bar.sync();
-		}
+		/* the group's transpose buffers are idle here: 2 * kXchWords * 4 >= N * 8 */
+		flush_bins<L, PEAK, GroupBar>(acc, prm.avg + ((long long)hop << L), (unsigned long long *)xch, tf, bar);
 	}
 }
 
