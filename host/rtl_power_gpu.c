@@ -12,7 +12,8 @@
  *     dB..." in hop order                              (:989-1003, :722-760)
  *   - SIGINT: first = finish the pass and exit, second = abort (:182-211, :651)
  * What is replaced: the DSP between the read and the row (:660-718, :730-764)
- * is rtlsdr_gpu_scan_submit() / rtlsdr_gpu_scan_collect_all().
+ * is rtlsdr_gpu_scan_submit() / rtlsdr_gpu_scan_collect_csv(), which also formats
+ * the rows on the GPU (byte-identical to rp_csv_row's printf).
  *
  * Three items of the reference's TODO list (rtl_power.c:29-36) that the GPU makes cheap:
  *   -t workers   "multiple FFT workers": the hops are dealt in contiguous ranges to `workers`
@@ -216,6 +217,26 @@ static int sweep(rtlsdr_dev_t *dev, const struct workers *ws, const rp_plan_t *p
 	return 0;
 }
 
+/* the row table of a worker: the plan's hops [first, first + rows) */
+static int set_columns(rtlsdr_gpu_scan_t *gpu, const rp_plan_t *plan, int first, int rows)
+{
+	int32_t *low = (int32_t *)malloc(sizeof(int32_t) * (size_t)rows);
+	int32_t *high = (int32_t *)malloc(sizeof(int32_t) * (size_t)rows);
+	double step = 0.0;
+	int i, l, h, rc = RTLSDR_GPU_ERR_NOMEM;
+	if (low && high) {
+		for (i = 0; i < rows; i++) {
+			rp_csv_columns(plan, first + i, &l, &h, &step);
+			low[i] = l;
+			high[i] = h;
+		}
+		rc = rtlsdr_gpu_scan_set_csv_columns(gpu, rows, low, high, step);
+	}
+	free(low);
+	free(high);
+	return rc;
+}
+
 /* the device list of -t: RTLSDR_GPU_DEVICES=0,2,3 or RTLSDR_GPU_DEVICE, RTLSDR_GPU_DEVICE + 1, ... */
 static int device_list(int workers, int *devices)
 {
@@ -240,7 +261,7 @@ int main(int argc, char **argv)
 	int opt, interval = 10, single = 0, peak_hold = 0, boxcar = 1, comp_fir_size = 0;
 	int passes_per_report = env_int("RTL_POWER_PASSES", 0), passes = 0, rc = 0, hop, w;
 	int max_reports = env_int("RTL_POWER_REPORTS", 0), reports = 0;
-	int want_workers = 1, smooth_iir = 0, shuffle = 0, db_count, devices[MAX_WORKERS];
+	int want_workers = 1, smooth_iir = 0, shuffle = 0, devices[MAX_WORKERS];
 	uint8_t *parts = NULL;      /* by_pass: raw bins + counts of workers 1.., pinned (device-readable) */
 	size_t part_avg_bytes = 0, part_bytes = 0;
 	const int use_async = getenv("RTL_POWER_ASYNC") != NULL;
@@ -254,10 +275,9 @@ int main(int argc, char **argv)
 	rtlsdr_gpu_scan_cfg_t cfg;
 	int32_t *window_coefs = NULL;
 	uint8_t *buf8, *replay = NULL;
-	double *db;
-	int *samples, *order;
-	char *row, stamp[64];
-	size_t row_cap;
+	int *order;
+	char *text, stamp[80];
+	size_t text_cap = 0, text_len = 0;
 	FILE *out;
 	struct sigaction sa;
 
@@ -385,10 +405,15 @@ int main(int argc, char **argv)
 		cfg.device = devices[w];
 		cfg.tune_count = ws.by_pass ? plan->tune_count : ws.first[w + 1] - ws.first[w];
 		rc = rtlsdr_gpu_scan_init(&cfg, &ws.gpu[w]);
+		if (!rc)
+			rc = set_columns(ws.gpu[w], plan, ws.first[w], cfg.tune_count);
 		if (rc) {
 			fprintf(stderr, "rtlsdr_gpu_scan_init (device %d): %s\n", devices[w], rtlsdr_gpu_scan_strerror(rc));
 			return 1;
 		}
+		/* text buffer for the longest stamp this program prints */
+		if ((size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > text_cap)
+			text_cap = (size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1);
 	}
 	if (ws.count > 1 && ws.by_pass)
 		fprintf(stderr, "GPU workers: %d (all %d hops each, every %d-th sweep; accumulators merged per report)\n",
@@ -406,15 +431,11 @@ int main(int argc, char **argv)
 		}
 	}
 
-	db_count = rtlsdr_gpu_scan_db_count(ws.gpu[0]);
 	buf8 = (uint8_t *)malloc((size_t)plan->buf_len);
-	/* report landing area: pinned, so every worker's device-to-host copies are plain DMA */
-	db = (double *)rtlsdr_gpu_scan_host_alloc(sizeof(double) * (size_t)db_count * (size_t)plan->tune_count);
-	samples = (int *)rtlsdr_gpu_scan_host_alloc(sizeof(int) * (size_t)plan->tune_count);
+	/* report landing area: pinned, so every worker's device-to-host copy is plain DMA */
+	text = (char *)rtlsdr_gpu_scan_host_alloc(text_cap);
 	order = (int *)malloc(sizeof(int) * (size_t)plan->tune_count);
-	row_cap = (size_t)db_count * 16 + 256;
-	row = (char *)malloc(row_cap);
-	if (!buf8 || !db || !samples || !order || !row) {
+	if (!buf8 || !text || !order) {
 		fprintf(stderr, "Out of memory.\n");
 		return 1;
 	}
@@ -434,13 +455,14 @@ int main(int argc, char **argv)
 		if (passes_per_report ? (passes % passes_per_report) != 0 : now < next_tick)
 			continue;
 		if (fixed_stamp) {
-			snprintf(stamp, sizeof(stamp), "%s", fixed_stamp);
+			snprintf(stamp, sizeof(stamp) - 2, "%s", fixed_stamp);
 		} else {
 			struct tm *cal = localtime(&now);
-			strftime(stamp, sizeof(stamp), "%Y-%m-%d, %H:%M:%S", cal);
+			strftime(stamp, sizeof(stamp) - 2, "%Y-%m-%d, %H:%M:%S", cal);
 		}
-		/* one report per worker: ONE epilogue launch, one copy, one synchronisation each
-		 * (csv_dbm's reads and zeroing, rtl_power.c:730-764), then the rows in hop order (:995-1000) */
+		strcat(stamp, ", ");
+		/* one report per worker (csv_dbm's reads and zeroing, rtl_power.c:730-764): the epilogue and the
+		 * row formatter run on the worker's GPU, its rows' text is written out in hop order (:995-1000) */
 		if (ws.by_pass) {
 			/* the other workers' raw int64 bins and counts land in pinned memory, worker 0 folds them into its
 			 * own accumulators (sums, or maxima under -P: exact in any grouping) and reports alone */
@@ -451,24 +473,20 @@ int main(int argc, char **argv)
 				rc = rtlsdr_gpu_scan_merge_device(ws.gpu[0], parts, parts + part_avg_bytes, ws.count - 1,
 								  (int64_t)part_bytes);
 			if (!rc)
-				rc = rtlsdr_gpu_scan_collect_all(ws.gpu[0], NULL, samples, db);
+				rc = rtlsdr_gpu_scan_collect_csv(ws.gpu[0], stamp, text, text_cap, &text_len);
+			if (!rc)
+				fwrite(text, 1, text_len, out);
 			if (rc)
 				fprintf(stderr, "merging the workers' accumulators: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
 					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[0]));
 		}
 		for (w = 0; w < ws.count && !rc && !ws.by_pass; w++) {
-			rc = rtlsdr_gpu_scan_collect_all(ws.gpu[w], NULL, samples + ws.first[w],
-							 db + (size_t)ws.first[w] * (size_t)db_count);
+			rc = rtlsdr_gpu_scan_collect_csv(ws.gpu[w], stamp, text, text_cap, &text_len);
 			if (rc)
-				fprintf(stderr, "rtlsdr_gpu_scan_collect_all: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
+				fprintf(stderr, "rtlsdr_gpu_scan_collect_csv: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
 					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
-		}
-		for (hop = 0; hop < plan->tune_count && !rc; hop++) {
-			if (rp_csv_row(row, row_cap, plan, hop, samples[hop], db + (size_t)hop * (size_t)db_count, db_count) < 0) {
-				rc = 1;
-				break;
-			}
-			fprintf(out, "%s, %s", stamp, row);
+			else
+				fwrite(text, 1, text_len, out);
 		}
 		fflush(out);
 		if (rc)
@@ -491,11 +509,9 @@ int main(int argc, char **argv)
 		rtlsdr_gpu_scan_close(ws.gpu[w]);
 	rtlsdr_close(dev);
 	free(buf8);
-	rtlsdr_gpu_scan_host_free(db);
-	rtlsdr_gpu_scan_host_free(samples);
+	rtlsdr_gpu_scan_host_free(text);
 	rtlsdr_gpu_scan_host_free(parts);
 	free(order);
-	free(row);
 	free(window_coefs);
 	free(replay);
 	free(plan);

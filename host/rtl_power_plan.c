@@ -168,16 +168,24 @@ int rp_db_count(const rp_plan_t *p)
 	return i2 - i1 + 2;
 }
 
-int rp_csv_row(char *out, size_t cap, const rp_plan_t *p, int hop, int samples,
-	       const double *db, int db_count)
+void rp_csv_columns(const rp_plan_t *p, int hop, int *low, int *high, double *step)
 {
 	const int len = 1 << p->bin_e, ds = p->downsample;
 	const int bin_count = (int)((double)len * (1.0 - p->crop));
 	const int bw2 = (int)(((double)p->rate * (double)bin_count) / (len * 2 * ds));
+	*low = p->freq[hop] - bw2;
+	*high = p->freq[hop] + bw2;
+	*step = (double)p->rate / (double)(len * ds);
+}
+
+int rp_csv_row(char *out, size_t cap, const rp_plan_t *p, int hop, int samples,
+	       const double *db, int db_count)
+{
 	size_t used = 0;
-	int i, n;
-	n = snprintf(out, cap, "%i, %i, %.2f, %i, ", p->freq[hop] - bw2, p->freq[hop] + bw2,
-		     (double)p->rate / (double)(len * ds), samples);
+	int i, n, low, high;
+	double step;
+	rp_csv_columns(p, hop, &low, &high, &step);
+	n = snprintf(out, cap, "%i, %i, %.2f, %i, ", low, high, step, samples);
 	if (n < 0 || (size_t)n >= cap)
 		return -1;
 	used = (size_t)n;

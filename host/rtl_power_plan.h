@@ -56,6 +56,10 @@ void rp_plan_report(const rp_plan_t *p, void *file /* FILE* */);
 int rp_csv_row(char *out, size_t cap, const rp_plan_t *p, int hop, int samples,
 	       const double *db, int db_count);
 
+/* The first three columns of hop `hop`'s row (rtl_power.c:739-746): low and high edge in Hz and the
+ * bin step.  rp_csv_row() prints these, and rtlsdr_gpu_scan_set_csv_columns() takes them. */
+void rp_csv_columns(const rp_plan_t *p, int hop, int *low, int *high, double *step);
+
 /* number of doubles per row = i2 - i1 + 2 (rtl_power.c:747-748) */
 int rp_db_count(const rp_plan_t *p);
 

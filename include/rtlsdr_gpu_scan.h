@@ -51,7 +51,8 @@ enum rtlsdr_gpu_scan_error {
 	RTLSDR_GPU_ERR_NULL      = -1,  /* NULL handle / argument (librtlsdr returns -1 for !dev) */
 	RTLSDR_GPU_ERR_CONFIG    = -2,  /* inconsistent or unsupported configuration */
 	RTLSDR_GPU_ERR_HOP       = -3,  /* hop index outside [0, tune_count) */
-	RTLSDR_GPU_ERR_LENGTH    = -4,  /* submit length != buf_len (short read, see submit) */
+	RTLSDR_GPU_ERR_LENGTH    = -4,  /* submit length != buf_len (short read, see submit), or a text buffer
+	                                 * smaller than rtlsdr_gpu_scan_csv_capacity() */
 	RTLSDR_GPU_ERR_NO_DEVICE = -5,  /* no CUDA device / device is not sm_100 */
 	RTLSDR_GPU_ERR_CUDA      = -6,  /* a CUDA runtime call or kernel failed */
 	RTLSDR_GPU_ERR_NOMEM     = -7,  /* host or device allocation failed */
@@ -237,6 +238,49 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void
  */
 RTLSDR_GPU_API int rtlsdr_gpu_scan_level_stats(rtlsdr_gpu_scan_t *h, int hop, uint64_t *overload,
 		uint64_t *high_level, uint64_t *bytes);
+
+/* ---- CSV rows ------------------------------------------------------------ */
+
+/*
+ * The report as rtl_power prints it, formatted on the GPU: per row
+ * "<stamp>low, high, step, samples, dB, ..., dB\n" (rtl_power.c:739-760, 995-998), byte-identical to the host's
+ * printf("%i, %i, %.2f, %i, " "%.2f, " ... "%.2f\n") of the same values (host/rtl_power_plan.c rp_csv_row).
+ * `stamp` is copied verbatim in front of every row (rtl_power prints "date, time, ", so pass it with the
+ * separator); it is a NUL-terminated string of fewer than 128 bytes.
+ *
+ * The formatter prints what it is given: -inf for a bin of 0, nan / -nan with the sign bit of the NaN (a hop
+ * without samples), -0.00 for values that round to zero from below.  A dB value whose text would be wider than
+ * 7 characters (wider than "-999.99" or "9999.99") does not occur in a report, whose dB values lie in (-187, 190);
+ * met in a caller's buffer it is an error, never text.
+ */
+
+/* The row table: row r prints low[r], high[r] and `step` (rtl_power_plan.c rp_csv_columns; 0 <= step < 2^31).
+ * Copied to the device once.  collect_csv() prints rows [0, tune_count); the table may have more rows for
+ * format_csv_device() (e.g. rank 0 of a sharded sweep prints every rank's hops).  Synchronous. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_set_csv_columns(rtlsdr_gpu_scan_t *h, int rows, const int32_t *low,
+		const int32_t *high, double step);
+/* Bytes that `rows` rows with a stamp of stamp_len bytes can take at most: the text buffer size collect_csv() and
+ * format_csv_device() require.  rows * (stamp_len + 56 + 9 * db_count); negative = error. */
+RTLSDR_GPU_API int64_t rtlsdr_gpu_scan_csv_capacity(const rtlsdr_gpu_scan_t *h, int rows, size_t stamp_len);
+/*
+ * collect_all()'s read-and-zero of every hop, returning the rows' text instead of the dB doubles: `text`
+ * receives *len bytes (no NUL).  cap is checked against csv_capacity(tune_count) before anything is touched
+ * (RTLSDR_GPU_ERR_LENGTH); without a table of at least tune_count rows the call is RTLSDR_GPU_ERR_CONFIG.  On
+ * any error the accumulators are left as they were.  Blocks until the text is in `text`.
+ */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap,
+		size_t *len);
+/*
+ * The rows [row_first, row_first + rows) of the table for a report in device memory: dB row r at
+ * dev_db + r * db_stride doubles (db_stride >= db_count, 8-byte aligned), its count at dev_samples[r] (int32) --
+ * the layout collect_device() writes for a handle with the same configuration.  The text goes to dev_text
+ * (cap >= csv_capacity(rows), else RTLSDR_GPU_ERR_LENGTH) and its length to *dev_len (int64, 8-byte aligned);
+ * a value outside the formatter's domain makes *dev_len = -1 (all ones).  Asynchronous on the handle's stream;
+ * the caller orders it after the writer of the report and before the reader of the text.
+ */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first,
+		int rows, const void *dev_db, int64_t db_stride, const void *dev_samples, void *dev_text, size_t cap,
+		void *dev_len);
 
 /* ---- multi-GPU report hand-off ----------------------------------------- */
 

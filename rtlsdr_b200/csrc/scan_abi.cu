@@ -12,6 +12,7 @@
  *    the number of reads, so it is counted on the host.
  */
 #include "../../include/rtlsdr_gpu_scan.h"
+#include "csv_text.cuh"
 #include "scan_kernels.cuh"
 #include "scan_large.cuh"
 
@@ -140,6 +141,19 @@ struct rtlsdr_gpu_scan {
 	/* bulk H2D staging for submit_batch */
 	uint8_t *d_bulk = nullptr;
 	size_t bulk_bytes = 0;
+
+	/* CSV rows (csv_text.cuh): column table of set_csv_columns(), per-row slots and lengths, and for
+	 * collect_csv() the packed text and its length */
+	int2 *d_csv_cols = nullptr;
+	int csv_rows = 0;
+	double csv_step = 0.0;
+	char *d_csv_slots = nullptr;
+	size_t csv_slot_bytes = 0;
+	int *d_csv_lens = nullptr;
+	char *d_csv_text = nullptr;
+	size_t csv_text_bytes = 0;
+	long long *d_csv_len = nullptr;
+	long long *h_csv_len = nullptr; /* pinned */
 
 	/* true while the last operation this handle put on its OWN stream was the report epilogue:
 	 * only then may the next transform kernel be launched programmatically dependent (it reads
@@ -1195,6 +1209,13 @@ void free_all(rtlsdr_gpu_scan *h)
 	cudaFree(h->d_samples);
 	cudaFree(h->d_scratch);
 	cudaFree(h->d_bulk);
+	cudaFree(h->d_csv_cols);
+	cudaFree(h->d_csv_slots);
+	cudaFree(h->d_csv_lens);
+	cudaFree(h->d_csv_text);
+	cudaFree(h->d_csv_len);
+	if (h->h_csv_len)
+		cudaFreeHost(h->h_csv_len);
 	for (auto &c : h->reg_cache)
 		cudaFree(c.d_desc);
 	for (int i = 0; i < 2; i++) {
@@ -1274,6 +1295,52 @@ int run_epilogue(rtlsdr_gpu_scan *h, int hop0, int nhops, double *db, long long 
 	epilogue_kernel<<<grid, 256, 0, h->stream>>>(p);
 	h->last_was_epilogue = zero_after; /* nothing else follows it on the stream in the fused-zero case */
 	return check_launch(h, "epilogue_kernel");
+}
+
+/* bytes of `rows` CSV rows at their widest (csv_text.cuh) */
+size_t csv_bound(const rtlsdr_gpu_scan *h, int rows, size_t stamp_len)
+{
+	return (size_t)rows * (stamp_len + kCsvRowFixed + (size_t)kCsvValueMax * (size_t)h->db_count);
+}
+
+/* rows [row_first, row_first + rows) of the column table, from dB rows and int32 counts in device memory, into
+ * `text` (csv_bound() bytes) and `len` (-1 = a value outside the formatter's domain), on the handle's stream */
+int run_csv(rtlsdr_gpu_scan *h, const char *stamp, size_t stamp_len, int row_first, int rows, const double *db,
+	    long long db_stride, const int *samples, char *text, long long *len)
+{
+	const size_t slot = csv_bound(h, 1, stamp_len), need = slot * (size_t)rows;
+	if (need > h->csv_slot_bytes) {
+		cudaFree(h->d_csv_slots);
+		h->d_csv_slots = nullptr;
+		h->csv_slot_bytes = 0;
+		CU(cudaMalloc(&h->d_csv_slots, need));
+		h->csv_slot_bytes = need;
+	}
+	CsvRowParams p;
+	p.db = db;
+	p.db_stride = db_stride;
+	p.samples = samples;
+	p.cols = h->d_csv_cols;
+	p.step = h->csv_step;
+	p.row_first = row_first;
+	p.db_count = h->db_count;
+	p.slots = h->d_csv_slots;
+	p.slot_bytes = (long long)slot;
+	p.lens = h->d_csv_lens;
+	p.stamp_len = (int)stamp_len;
+	memcpy(p.stamp, stamp, stamp_len);
+	h->last_was_epilogue = false;
+	csv_rows_kernel<<<rows, kCsvThreads, 0, h->stream>>>(p);
+	if (int rc = check_launch(h, "csv_rows_kernel"))
+		return rc;
+	CsvPackParams q;
+	q.slots = h->d_csv_slots;
+	q.slot_bytes = (long long)slot;
+	q.lens = h->d_csv_lens;
+	q.text = text;
+	q.len = len;
+	csv_pack_kernel<<<rows, kCsvThreads, 0, h->stream>>>(q);
+	return check_launch(h, "csv_pack_kernel");
 }
 
 } // namespace
@@ -2108,6 +2175,116 @@ int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *de
 	std::fill(h->samples.begin(), h->samples.end(), 0);
 	h->samples_on_device = false;
 	return 0;
+}
+
+int rtlsdr_gpu_scan_set_csv_columns(rtlsdr_gpu_scan_t *h, int rows, const int32_t *low, const int32_t *high, double step)
+{
+	if (!h || !low || !high)
+		return RTLSDR_GPU_ERR_NULL;
+	if (rows < 1 || !(step >= 0.0 && step < kCsvStepLimit))
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	std::vector<int2> cols((size_t)rows);
+	for (int i = 0; i < rows; i++)
+		cols[i] = make_int2(low[i], high[i]);
+	if (rows > h->csv_rows) {
+		cudaFree(h->d_csv_cols); /* implicit device synchronisation: no kernel still reads the old table */
+		cudaFree(h->d_csv_lens);
+		h->d_csv_cols = nullptr;
+		h->d_csv_lens = nullptr;
+		h->csv_rows = 0;
+		CU(cudaMalloc(&h->d_csv_cols, (size_t)rows * sizeof(int2)));
+		CU(cudaMalloc(&h->d_csv_lens, (size_t)rows * sizeof(int)));
+	} else {
+		CU(cudaStreamSynchronize(h->stream));
+	}
+	h->last_was_epilogue = false;
+	CU(cudaMemcpyAsync(h->d_csv_cols, cols.data(), (size_t)rows * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
+	CU(cudaStreamSynchronize(h->stream));
+	h->h2d += (uint64_t)rows * sizeof(int2);
+	h->csv_rows = rows;
+	h->csv_step = step;
+	return 0;
+}
+
+int64_t rtlsdr_gpu_scan_csv_capacity(const rtlsdr_gpu_scan_t *h, int rows, size_t stamp_len)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (rows < 0 || stamp_len >= (size_t)kCsvStampMax)
+		return RTLSDR_GPU_ERR_CONFIG;
+	return (int64_t)csv_bound(h, rows, stamp_len);
+}
+
+int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len)
+{
+	if (!h || !stamp || !text || !len)
+		return RTLSDR_GPU_ERR_NULL;
+	const size_t stamp_len = strlen(stamp);
+	const int tc = h->cfg.tune_count;
+	if (stamp_len >= (size_t)kCsvStampMax || h->csv_rows < tc)
+		return RTLSDR_GPU_ERR_CONFIG;
+	const size_t bound = csv_bound(h, tc, stamp_len);
+	if (cap < bound)
+		return RTLSDR_GPU_ERR_LENGTH;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc = flush_ring(h);
+	if (rc)
+		return rc;
+	if (!h->d_csv_len) {
+		CU(cudaMalloc(&h->d_csv_len, sizeof(long long)));
+		CU(cudaMallocHost(&h->h_csv_len, sizeof(long long)));
+	}
+	if (bound > h->csv_text_bytes) {
+		cudaFree(h->d_csv_text);
+		h->d_csv_text = nullptr;
+		h->csv_text_bytes = 0;
+		CU(cudaMalloc(&h->d_csv_text, bound));
+		h->csv_text_bytes = bound;
+	}
+	/* the epilogue's dB rows and counts stay on the device: only the text crosses PCIe */
+	if ((rc = run_epilogue(h, 0, tc, h->d_db, nullptr, h->d_samples)))
+		return rc;
+	if ((rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_db, h->db_count, h->d_samples, h->d_csv_text, h->d_csv_len)))
+		return rc;
+	CU(cudaMemcpyAsync(h->h_csv_len, h->d_csv_len, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+	CU(cudaStreamSynchronize(h->stream));
+	const long long n = *h->h_csv_len;
+	if (n < 0 || (size_t)n > bound)
+		return RTLSDR_GPU_ERR_CONFIG; /* cannot happen for the epilogue's values; the accumulators are kept */
+	CU(cudaMemcpyAsync(text, h->d_csv_text, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+	h->d2h += (uint64_t)n + sizeof(long long);
+	/* read-and-zero, like csv_dbm (rtl_power.c:761-764) */
+	CU(cudaMemsetAsync(h->d_avg, 0, ((size_t)tc * h->N + (size_t)tc) * sizeof(long long), h->stream));
+	if (h->d_level)
+		CU(cudaMemsetAsync(h->d_level, 0, (size_t)tc * 2 * sizeof(unsigned long long), h->stream));
+	CU(cudaStreamSynchronize(h->stream));
+	std::fill(h->samples.begin(), h->samples.end(), 0);
+	if (h->d_level)
+		std::fill(h->level_bytes.begin(), h->level_bytes.end(), 0);
+	h->samples_on_device = false;
+	*len = (size_t)n;
+	return 0;
+}
+
+int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first, int rows,
+				      const void *dev_db, int64_t db_stride, const void *dev_samples, void *dev_text,
+				      size_t cap, void *dev_len)
+{
+	if (!h || !stamp || !dev_db || !dev_samples || !dev_text || !dev_len)
+		return RTLSDR_GPU_ERR_NULL;
+	if (((uintptr_t)dev_db & 7) || ((uintptr_t)dev_samples & 3) || ((uintptr_t)dev_len & 7))
+		return RTLSDR_GPU_ERR_ALIGN;
+	const size_t stamp_len = strlen(stamp);
+	if (stamp_len >= (size_t)kCsvStampMax || !h->d_csv_cols || db_stride < h->db_count)
+		return RTLSDR_GPU_ERR_CONFIG;
+	if (rows < 1 || row_first < 0 || row_first > h->csv_rows - rows)
+		return RTLSDR_GPU_ERR_HOP;
+	if (cap < csv_bound(h, rows, stamp_len))
+		return RTLSDR_GPU_ERR_LENGTH;
+	CU(cudaSetDevice(h->cfg.device));
+	return run_csv(h, stamp, stamp_len, row_first, rows, (const double *)dev_db, (long long)db_stride,
+		       (const int *)dev_samples, (char *)dev_text, (long long *)dev_len);
 }
 
 int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, const void *dev_samples, int sets,

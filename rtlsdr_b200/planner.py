@@ -32,6 +32,9 @@ def host_library():
         L.rp_csv_row.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(_RpPlan), ctypes.c_int,
                                  ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
         L.rp_db_count.argtypes = [ctypes.POINTER(_RpPlan)]
+        L.rp_csv_columns.argtypes = [ctypes.POINTER(_RpPlan), ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                     ctypes.c_void_p]
+        L.rp_csv_columns.restype = None
         for fn in (L.rp_atofs, L.rp_atoft, L.rp_atofp):
             fn.argtypes = [ctypes.c_char_p]
             fn.restype = ctypes.c_double
@@ -72,6 +75,20 @@ class Plan:
     @property
     def db_count(self):
         return host_library().rp_db_count(ctypes.byref(self._c))
+
+    def csv_columns(self, hops=None):
+        """(low int32 [rows], high int32 [rows], step) of the rows of `hops` (default: all), the table
+        GpuScan.set_csv_columns() takes (rp_csv_columns, the numbers csv_row() prints)"""
+        import numpy as np
+        hops = range(self.tune_count) if hops is None else hops
+        low = np.zeros(len(hops), dtype=np.int32)
+        high = np.zeros(len(hops), dtype=np.int32)
+        lo, hi, step = ctypes.c_int(), ctypes.c_int(), ctypes.c_double()
+        for i, h in enumerate(hops):
+            host_library().rp_csv_columns(ctypes.byref(self._c), h, ctypes.byref(lo), ctypes.byref(hi),
+                                          ctypes.byref(step))
+            low[i], high[i] = lo.value, hi.value
+        return low, high, step.value
 
     def csv_row(self, hop, samples, db):
         """'low, high, step, samples, dB...' exactly as csv_dbm prints it (rtl_power.c:739-760)."""

@@ -57,6 +57,11 @@ def load_library():
     L.rtlsdr_gpu_scan_collect_all.argtypes = [vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_collect_device.argtypes = [vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_merge_device.argtypes = [vp, vp, vp, i, i64]
+    L.rtlsdr_gpu_scan_set_csv_columns.argtypes = [vp, i, vp, vp, ctypes.c_double]
+    L.rtlsdr_gpu_scan_csv_capacity.argtypes = [vp, i, ctypes.c_size_t]
+    L.rtlsdr_gpu_scan_csv_capacity.restype = i64
+    L.rtlsdr_gpu_scan_collect_csv.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]
+    L.rtlsdr_gpu_scan_format_csv_device.argtypes = [vp, ctypes.c_char_p, i, i, vp, i64, vp, vp, ctypes.c_size_t, vp]
     L.rtlsdr_gpu_scan_db_count.argtypes = [vp]
     L.rtlsdr_gpu_scan_host_alloc.argtypes = [ctypes.c_size_t]
     L.rtlsdr_gpu_scan_host_alloc.restype = vp
@@ -251,6 +256,39 @@ class GpuScan:
         """fold `sets` external accumulator sets (raw int64 bins + int32 counts as collect_device writes them,
         `set_stride` bytes apart; may be peer memory) into this handle's: sums, or maxima under peak hold"""
         self._check(self.lib.rtlsdr_gpu_scan_merge_device(self.h, dev_avg, dev_samples, sets, set_stride), "merge_device")
+
+    def set_csv_columns(self, low, high, step):
+        """row table of the CSV formatter: row r prints low[r], high[r], step (Plan.csv_columns())"""
+        lo = np.ascontiguousarray(low, dtype=np.int32)
+        hi = np.ascontiguousarray(high, dtype=np.int32)
+        assert lo.size == hi.size
+        self._check(self.lib.rtlsdr_gpu_scan_set_csv_columns(self.h, lo.size, lo.ctypes.data, hi.ctypes.data,
+                                                             float(step)), "set_csv_columns")
+
+    def csv_capacity(self, rows, stamp_len):
+        """bytes `rows` CSV rows with a stamp of `stamp_len` bytes can take at most"""
+        n = self.lib.rtlsdr_gpu_scan_csv_capacity(self.h, rows, stamp_len)
+        self._check(n if n < 0 else 0, "csv_capacity")
+        return n
+
+    def collect_csv(self, stamp, out=None):
+        """collect_all()'s read-and-zero, returning the rows' text (bytes), formatted on the GPU.  `stamp` is
+        printed verbatim before every row; out: optional writable uint8 buffer (e.g. PinnedBuffer.array)."""
+        s = stamp.encode() if isinstance(stamp, str) else bytes(stamp)
+        if out is None:
+            out = np.empty(max(1, self.csv_capacity(self.tune_count, len(s))), dtype=np.uint8)
+        n = ctypes.c_size_t(0)
+        self._check(self.lib.rtlsdr_gpu_scan_collect_csv(self.h, s, out.ctypes.data, out.nbytes, ctypes.byref(n)),
+                    "collect_csv")
+        return out[: n.value].tobytes()
+
+    def format_csv_device(self, stamp, row_first, rows, dev_db, db_stride, dev_samples, dev_text, cap, dev_len):
+        """rows [row_first, row_first + rows) of a collect_device() report (dB rows db_stride doubles apart,
+        int32 counts) into dev_text / *dev_len (int64, -1 = value outside the domain), async on the handle's stream"""
+        s = stamp.encode() if isinstance(stamp, str) else bytes(stamp)
+        self._check(self.lib.rtlsdr_gpu_scan_format_csv_device(self.h, s, row_first, rows, dev_db, db_stride,
+                                                               dev_samples, dev_text, cap, dev_len),
+                    "format_csv_device")
 
     def set_stream(self, cuda_stream):
         self._check(self.lib.rtlsdr_gpu_scan_set_stream(self.h, cuda_stream), "set_stream")

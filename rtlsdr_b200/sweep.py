@@ -329,6 +329,15 @@ class SpectrumGather:
             bufs = self.host[k].numpy()
         return self.unpack(bufs)
 
+    def wait(self, k):
+        """block until the exchange of buffer k is done; raises if a rank's report did not arrive (peer mode)"""
+        if self.cuda:
+            self.gathered[k].synchronize()
+        if self.rank == 0 and self.mode == "peer" and self.world > 1:
+            flags = self.peer[0][SLOTS * self.world * self.words:].view(torch.int32)
+            if int(flags[SLOTS * self.world + SLOTS].item()) != 0:
+                raise RuntimeError("SpectrumGather: a rank's report did not arrive within the flag wait's time-out")
+
     def partial_sets(self, k):
         """rank 0, replicated mode: (device address of set 0's raw bins, of its int32 counts, number of sets, bytes
         between sets) of the gathered buffer k, for rtlsdr_gpu_scan_merge_device() on a stream that has waited for
@@ -337,6 +346,21 @@ class SpectrumGather:
         base = self.dev_copy[k].data_ptr()
         smp = base + (self.hmax * self.n + self.hmax * self.db_count) * 8
         return base, smp, self.world, self.words * 8
+
+    def keep_device_copy(self):
+        """rank 0, CUDA: from now on every exchange also leaves a private device copy of the gathered buffer (made
+        on the second stream before any rank may rewrite its slot; from the host buffer in host mode), for readers
+        on another stream such as the CSV formatter.  They call release_copy() behind their last read."""
+        if self.rank == 0 and self.cuda and self.dev_copy is None:
+            self.dev_copy = [torch.zeros(self.world, self.words, dtype=torch.int64, device=self.device)
+                             for _ in range(SLOTS)]
+
+    def slot_rows(self, k, r):
+        """rank 0: (device address of the dB rows, of the int32 counts) of rank r's slot in the private copy of
+        buffer k (keep_device_copy); the dB rows are db_count doubles apart"""
+        base = self.dev_copy[k].data_ptr() + r * self.words * 8
+        p_db = base + self.hmax * self.n * 8
+        return p_db, p_db + self.hmax * self.db_count * 8
 
     def release_copy(self, k, stream):
         """rank 0, replicated mode: everything enqueued so far on `stream` (the merge) is the last reader of the
@@ -373,9 +397,3 @@ class SpectrumGather:
                         "with the next interval's transform",
                 "host": "reports staged through host memory and gathered with torch.distributed (gloo)"}[self.mode] \
             if self.world > 1 else "none (one rank)"
-
-
-def format_rows(plan, report: IntervalReport, stamp: str) -> List[str]:
-    """rank 0: 'date, time, low, high, step, samples, dB...' rows in hop order"""
-    return [f"{stamp}, " + plan.csv_row(h, int(report.samples[h]), report.db[h])
-            for h in range(plan.tune_count)]

@@ -8,8 +8,9 @@ Every rank plans the same scan (host/rtl_power_plan.c), takes a contiguous range
 function of (hop, sweep), so the result does not depend on N), and once per integration interval
 bins + dB rows + sample counts reach rank 0 -- written by every rank's report epilogue straight
 into rank 0's buffer over NVLink (symmetric-memory peer mapping, one barrier per interval), or by
-ONE NCCL gather where peer mapping is unavailable / RTLSDR_B200_NCCL_GATHER=1 -- and rank 0 prints
-the reference's CSV rows in hop order (rtl_power.c:995-1000).  With N = 1 no process group is created.
+ONE NCCL gather where peer mapping is unavailable / RTLSDR_B200_NCCL_GATHER=1 -- and rank 0 formats
+the reference's CSV rows in hop order (rtl_power.c:995-1000) on its GPU (rtlsdr_gpu_scan_format_csv_device, once
+per rank slot) and copies only the text to the host.  With N = 1 no process group is created.
 Scans with fewer hops than GPUs (BASELINE configs 1 and 4 are ONE hop) shard the READS instead (--shard reads):
 every rank transforms its share of each hop's reads into its own accumulators, the raw int64 bins and counts
 reach rank 0 the same way, and rank 0 folds them into its handle (rtlsdr_gpu_scan_merge_device: int64 sums, or
@@ -54,7 +55,7 @@ def main(argv=None):
 
     from . import scan as rs
     from .planner import host_library, plan_scan, synth_cube
-    from .sweep import IntervalReport, SpectrumGather, format_rows, shard_hops
+    from .sweep import SpectrumGather, shard_hops
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -78,7 +79,7 @@ def main(argv=None):
     mode = ["xorshift", "counter", "const", "biased", "tone"].index(args.synth)
     if args.shard == "reads":
         return _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch, dist,
-                                  IntervalReport, SpectrumGather, format_rows, shard_hops, synth_cube)
+                                  SpectrumGather, shard_hops, synth_cube)
 
     g = None
     if len(mine):
@@ -90,6 +91,19 @@ def main(argv=None):
     if rank == 0 and world > 1:
         print("sweep_main: interval reports: " + gather.describe(), file=sys.stderr)
     stream = torch.cuda.ExternalStream(g.get_stream()) if g else torch.cuda.current_stream()
+    stamp = args.stamp + ", "
+    if rank == 0:
+        # rank 0 formats every rank's rows from a private device copy of the gathered report, on its handle's
+        # stream behind the exchange; one text region and one int64 length per rank slot, copied out together
+        gather.keep_device_copy()
+        g.set_csv_columns(*plan.csv_columns())
+        caps = [g.csv_capacity(len(r), len(stamp.encode())) for r in gather.ranges]
+        offs = [0] + [int(x) for x in np.cumsum(caps)]
+        lens_at = (offs[-1] + 7) // 8 * 8
+        dev = torch.device("cuda", local)
+        text_dev = [torch.empty(lens_at + 8 * world, dtype=torch.uint8, device=dev) for _ in range(2)]
+        text_host = [torch.empty(lens_at + 8 * world, dtype=torch.uint8).pin_memory() for _ in range(2)]
+        text_ready = [torch.cuda.Event() for _ in range(2)]
     # Two pinned input cubes alternate: rtlsdr_gpu_scan_submit_batch() returns while its host-to-device copies
     # are still queued, and `buf` must stay untouched until an event recorded on the handle's stream after the
     # call has completed (include/rtlsdr_gpu_scan.h) -- `consumed[k]` below.
@@ -100,10 +114,31 @@ def main(argv=None):
     rows_out = []
     pending = None          # exchange buffer of the interval whose report has not been printed yet
 
+    def format_rows(k):
+        """rank 0: the rows of exchange buffer k into text_dev[k] on the handle's stream, then to pinned memory"""
+        stream.wait_event(gather.gathered[k])
+        lens = text_dev[k].data_ptr() + lens_at
+        for r, hops in enumerate(gather.ranges):
+            if len(hops):
+                p_db, p_smp = gather.slot_rows(k, r)
+                g.format_csv_device(stamp, hops.start, len(hops), p_db, g.db_count, p_smp,
+                                    text_dev[k].data_ptr() + offs[r], caps[r], lens + 8 * r)
+        gather.release_copy(k, stream)
+        with torch.cuda.stream(stream):
+            text_host[k].copy_(text_dev[k], non_blocking=True)
+        text_ready[k].record(stream)
+
     def print_pending():
-        report = gather.fetch(pending)
+        gather.wait(pending)
         if rank == 0:
-            rows_out.extend(format_rows(plan, report, args.stamp))
+            text_ready[pending].synchronize()
+            buf = text_host[pending].numpy()
+            lens = buf[lens_at:].view(np.int64)
+            for r, hops in enumerate(gather.ranges):
+                if len(hops):
+                    if lens[r] < 0:
+                        raise RuntimeError("sweep_main: a report value is outside the CSV formatter's domain")
+                    rows_out.append(buf[offs[r]: offs[r] + lens[r]].tobytes().decode())
 
     for interval in range(args.intervals):
         k = interval & 1
@@ -130,7 +165,9 @@ def main(argv=None):
             consumed[k].record(stream)
         # one exchange per interval (asynchronous, second stream); the previous interval's rows are
         # printed while this one is on the GPU
-        gather.publish(k, stream, to_host=True)
+        gather.publish(k, stream)
+        if rank == 0:
+            format_rows(k)
         if pending is not None:
             print_pending()
         pending = k
@@ -143,6 +180,11 @@ def main(argv=None):
         else:
             with open(args.out, "w") as f:
                 f.write(text)
+    if rank == 0:
+        # torch's pinned-memory allocator records an event on the stream of the last copy when it frees a block:
+        # the text buffers go before the handle's stream does
+        stream.synchronize()
+        text_host.clear()
     if g:
         g.close()
     if world > 1:
@@ -152,7 +194,7 @@ def main(argv=None):
 
 
 def _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch, dist,
-                       IntervalReport, SpectrumGather, format_rows, shard_hops, synth_cube):
+                       SpectrumGather, shard_hops, synth_cube):
     """--shard reads: rank r transforms sweeps [S*r/W, S*(r+1)/W) of every interval for ALL hops; rank 0 merges"""
     tc, b, n = pd["tune_count"], pd["buf_len"], 1 << pd["bin_e"]
     sweeps = shard_hops(args.sweeps, world, rank)            # the same balanced split, over sweeps
@@ -164,6 +206,8 @@ def _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch
         print("sweep_main: reads sharded %s over %d ranks; partial accumulators: %s" % (
             [len(shard_hops(args.sweeps, world, r)) for r in range(world)], world, gather.describe()), file=sys.stderr)
     stream = torch.cuda.ExternalStream(g.get_stream())
+    if rank == 0:
+        g.set_csv_columns(*plan.csv_columns())
     pinned = [rs.PinnedBuffer(max(1, len(sweeps) * tc * b)) for _ in range(2)]
     consumed = [None, None]
     rows_out = []
@@ -184,8 +228,7 @@ def _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch
         if rank == 0:
             stream.wait_event(gather.gathered[k])
             g.merge_device(*gather.partial_sets(k))
-            avg, smp, db = g.collect_all()
-            rows_out.extend(format_rows(plan, IntervalReport(avg, db, smp), args.stamp))
+            rows_out.append(g.collect_csv(args.stamp + ", ").decode())
     if rank == 0:
         text = "".join(rows_out)
         if args.out == "-":
