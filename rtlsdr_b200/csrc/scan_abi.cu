@@ -13,6 +13,7 @@
  */
 #include "../../include/rtlsdr_gpu_scan.h"
 #include "csv_text.cuh"
+#include "scan_host.cuh"
 #include "scan_kernels.cuh"
 #include "scan_large.cuh"
 
@@ -33,11 +34,8 @@ constexpr int kDescSlots = 4;
 constexpr size_t kDefaultRing = 32u << 20;
 constexpr size_t kScratchBudget = 512ull << 20; /* device bytes for decimation / large-FFT scratch */
 constexpr int kChainMaxPasses = 7;           /* fused fifth_order chain up to 128x decimation */
-constexpr int kChainCap0 = 8192;             /* level-0 samples a chain tile may span (32 KiB) */
 constexpr int kDecimChunks = 4;              /* only for batches >= kDecimOverlapBytes (measured: a loss below) */
 constexpr size_t kDecimOverlapBytes = 1ull << 30;
-
-enum Path { PATH_RMS, PATH_SMALL_U8, PATH_SMALL_DECIM, PATH_LARGE };
 
 struct DescSlot {
 	void *h = nullptr; /* pinned */
@@ -64,11 +62,7 @@ struct RegularKey {
 
 struct rtlsdr_gpu_scan {
 	rtlsdr_gpu_scan_cfg_t cfg;
-	int N = 1;
-	Path path = PATH_SMALL_U8;
-	int l_len = 0, n_blocks = 0, blocks_padded = 0, samples_per_read = 0;
-	long long image_stride = 0; /* c16 per decimated image */
-	int db_i1 = 0, db_i2 = 0, db_count = 2;
+	ScanShape shape;
 	int num_sms = 148, ctas_per_sm = 2;
 
 	cudaStream_t own_stream = nullptr, stream = nullptr;
@@ -97,7 +91,6 @@ struct rtlsdr_gpu_scan {
 	int *h_samples_pinned = nullptr;
 	std::vector<int> samples;
 	PassTw tw0;
-	std::vector<int2> tw_host;
 
 	/* staging ring: two halves, each host pinned + device mirror */
 	size_t ring_bytes = 0;
@@ -266,6 +259,51 @@ const int kCic9[11][5] = {
 	{ -199, -362, 5303, -25505, 77489 },
 };
 
+/* ---- init ------------------------------------------------------------- */
+
+/* the handle's debug / A-B switches (see rtlsdr_gpu_scan), read from the environment */
+int read_debug_switches(rtlsdr_gpu_scan *h)
+{
+	if (const char *f = getenv("RTLSDR_GPU_BOXCAR_STREAM")) {
+		const int m = atoi(f);
+		if (m != 0 && m != 1 && m != 2 && m != 3 && m != 5)
+			return RTLSDR_GPU_ERR_CONFIG; /* not a kernel variant */
+		h->dbg_boxcar_mode = m;
+	}
+	h->dbg_no_fused_boxcar = getenv("RTLSDR_GPU_NO_FUSED_BOXCAR") != nullptr;
+	if (const char *f = getenv("RTLSDR_GPU_STAGGER_NS"))
+		h->dbg_stagger_ns = atoi(f);
+	h->dbg_no_hb_stream = getenv("RTLSDR_GPU_NO_HB_STREAM") != nullptr;
+	if (const char *f = getenv("RTLSDR_GPU_LARGE_PIPE")) /* A/B switch: 0 = one-tile-per-CTA round B for N >= 2^17 */
+		h->dbg_large_pipe = atoi(f) != 0;
+	h->dbg_rms_warp = getenv("RTLSDR_GPU_RMS_WARP") != nullptr; /* 1-bin hops: warp-per-read kernel instead of CTA-per-read */
+	return 0;
+}
+
+/* device buffer of `bytes`, each set to `byte` on stream s.  A failed allocation sets *rc. */
+template <class T>
+bool alloc_fill(T **dst, size_t bytes, int byte, cudaStream_t s, int *rc)
+{
+	if (cudaMalloc(dst, bytes) != cudaSuccess) {
+		*rc = RTLSDR_GPU_ERR_NOMEM;
+		return false;
+	}
+	return cudaMemsetAsync(*dst, byte, bytes, s) == cudaSuccess;
+}
+
+/* device copy of a host table; an empty table stays nullptr.  A failed allocation sets *rc. */
+template <class T>
+bool upload(T **dst, const std::vector<T> &v, int *rc)
+{
+	if (v.empty())
+		return true;
+	if (cudaMalloc(dst, v.size() * sizeof(T)) != cudaSuccess) {
+		*rc = RTLSDR_GPU_ERR_NOMEM;
+		return false;
+	}
+	return cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice) == cudaSuccess;
+}
+
 /* ---- events for kernel timing ----------------------------------------- */
 
 cudaEvent_t get_event(rtlsdr_gpu_scan *h)
@@ -368,7 +406,7 @@ int build_desc(rtlsdr_gpu_scan *h, const std::vector<long long> &offs, const std
 	       std::vector<long long> &s_offs, std::vector<int> &s_hops, std::vector<int4> &segs)
 {
 	const int n = (int)offs.size(), tc = h->cfg.tune_count;
-	if (h->path == PATH_RMS) {
+	if (h->shape.path == PATH_RMS) {
 		/* 1-bin hops: every read is reduced on its own (one atomic per read), so the reads keep their
 		 * submission order = address order; sorting them by hop would turn the resident CTAs' working window
 		 * from one contiguous stretch into 16 KiB pieces a whole sweep apart */
@@ -391,10 +429,10 @@ int build_desc(rtlsdr_gpu_scan *h, const std::vector<long long> &offs, const std
 		s_hops[p] = hops[i];
 	}
 	segs.clear();
-	if (h->path == PATH_SMALL_U8 || h->path == PATH_RMS || h->path == PATH_LARGE)
+	if (h->shape.path == PATH_SMALL_U8 || h->shape.path == PATH_RMS || h->shape.path == PATH_LARGE)
 		return 0; /* these kernels walk the hop-sorted reads themselves (equal runs per CTA / per-read work) */
 	/* the decimating path runs in kDecimChunks chunks, each should still fill the GPU */
-	const bool big_decim = h->path == PATH_SMALL_DECIM && (size_t)n * (size_t)h->cfg.buf_len >= kDecimOverlapBytes;
+	const bool big_decim = h->shape.path == PATH_SMALL_DECIM && (size_t)n * (size_t)h->cfg.buf_len >= kDecimOverlapBytes;
 	const int target = std::max(1, h->num_sms * h->ctas_per_sm) * (big_decim ? kDecimChunks : 1);
 	int chunk = std::max(1, (n + target - 1) / target);
 	/*
@@ -694,8 +732,8 @@ int launch_fused_boxcar(rtlsdr_gpu_scan *h, const FusedBoxcarParams &prm)
 bool fused_boxcar_ok(const rtlsdr_gpu_scan *h)
 {
 	const int ds = h->cfg.downsample;
-	return h->cfg.boxcar && ds >= 2 && ds <= 64 && h->cfg.bin_e >= 8 && h->cfg.bin_e <= 12 && h->n_blocks == 1 &&
-	       h->cfg.buf_len == 2 * h->N * ds && !h->dbg_no_fused_boxcar;
+	return h->cfg.boxcar && ds >= 2 && ds <= 64 && h->cfg.bin_e >= 8 && h->cfg.bin_e <= 12 && h->shape.n_blocks == 1 &&
+	       h->cfg.buf_len == 2 * h->shape.N * ds && !h->dbg_no_fused_boxcar;
 }
 
 /*
@@ -715,7 +753,7 @@ struct DecimScratch {
 	static size_t per_entry(const rtlsdr_gpu_scan *h)
 	{
 		size_t pairs = (size_t)h->cfg.buf_len / 2;
-		size_t b = (size_t)h->image_stride * 4 + 16 + 8;
+		size_t b = (size_t)h->shape.image_stride * 4 + 16 + 8;
 		if (halfband(h))
 			b += (pairs / 2) * 4 + (pairs / 4 + 4) * 4;
 		return b;
@@ -725,7 +763,7 @@ struct DecimScratch {
 	{
 		size_t pairs = (size_t)h->cfg.buf_len / 2;
 		img = (c16 *)p;
-		p += (size_t)n * h->image_stride * 4 + kStageBytes; /* a unit may read past the last image */
+		p += (size_t)n * h->shape.image_stride * 4 + kStageBytes; /* a unit may read past the last image */
 		a = b = nullptr;
 		if (halfband(h)) {
 			a = (c16 *)p;
@@ -743,7 +781,7 @@ struct DecimScratch {
 int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_offs, int n, const DecimScratch &sc)
 {
 	const int pairs = h->cfg.buf_len / 2;
-	const int img_count = (int)h->image_stride;
+	const int img_count = (int)h->shape.image_stride;
 	int rc;
 	if (h->cfg.boxcar && h->cfg.downsample > 1) {
 		DecimParams p;
@@ -753,9 +791,9 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 		p.pairs = pairs;
 		p.ds = h->cfg.downsample;
 		p.out = sc.img;
-		p.out_stride = h->image_stride;
+		p.out_stride = h->shape.image_stride;
 		p.out_count = img_count;
-		p.l_len = h->l_len;
+		p.l_len = h->shape.l_len;
 		p.sums = sc.sums;
 		CU(cudaMemsetAsync(sc.sums, 0, (size_t)n * 16, h->stream));
 		dim3 grid((img_count + 255) / 256, n);
@@ -785,24 +823,16 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 		const int *row = kCic9[passes];
 		p.f1 = row[0]; p.f2 = row[1]; p.f3 = row[2]; p.f4 = row[3]; p.f5 = row[4];
 		p.out = sc.img;
-		p.out_stride = h->image_stride;
-		p.l_len = h->l_len;
+		p.out_stride = h->shape.image_stride;
+		p.l_len = h->shape.l_len;
 		p.sums = sc.sums;
-		/* level-0 span of a tile: (tile + 9) * 2^P + 5 * (2^P - 1) + 9 samples at most */
-		int tile = std::min(256, std::max(8, (kChainCap0 >> passes) - 16));
-		tile = std::min(tile, M);
 		/* P <= 5: the register-streaming kernel computes final samples >= 16, the tile kernel only
 		 * the eased-in head [0, 16) of every read (RTLSDR_GPU_NO_HB_STREAM=1: tile kernel for all) */
 		const bool stream = passes <= kHbStreamMaxPasses && M >= 2 * kHbStreamHead && !h->dbg_no_hb_stream;
-		if (stream)
-			tile = kHbStreamHead;
-		p.tile = tile;
-		/* head tiles span (16 + 9) * 2^P + 5 * (2^P - 1) + 9 <= 964 level-0 samples: small buffers, many CTAs per SM */
-		p.cap0 = stream ? 1024 : kChainCap0;
-		const int smem = (p.cap0 + p.cap0 / 2 + 16) * 4;
+		const int smem = chain_tile(p, stream);
 		CU(cudaFuncSetAttribute(halfband_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
 		CU(cudaMemsetAsync(sc.sums, 0, (size_t)n * 16, h->stream));
-		dim3 grid(stream ? 1 : (M + tile - 1) / tile, n);
+		dim3 grid(stream ? 1 : (M + p.tile - 1) / p.tile, n);
 		/* With the streaming kernel the tile kernel only computes the eased-in heads (final samples 0..15 of
 		 * every read): small latency-bound CTAs that write other words than the streaming kernel and share
 		 * only the atomically updated DC sums -- they run beside it on a stream of their own instead of in
@@ -832,8 +862,8 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 			q.use_fir = p.use_fir;
 			q.f1 = p.f1; q.f2 = p.f2; q.f3 = p.f3; q.f4 = p.f4; q.f5 = p.f5;
 			q.out = sc.img;
-			q.out_stride = h->image_stride;
-			q.l_len = h->l_len;
+			q.out_stride = h->shape.image_stride;
+			q.l_len = h->shape.l_len;
 			q.sums = sc.sums;
 			/* span: as long as possible (16 warm-up samples per span are recomputed) while the grid
 			 * still fills at least half of the resident thread slots (640 per SM at 87 registers) */
@@ -884,7 +914,7 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 		f.in = cur;
 		f.in_stride = cur_stride;
 		f.out = sc.img;
-		f.out_stride = h->image_stride;
+		f.out_stride = h->shape.image_stride;
 		f.count = count;
 		f.use_fir = (h->cfg.comp_fir_size == 9 && passes <= 10) ? 1 : 0;
 		const int *row = kCic9[passes <= 10 ? passes : 0];
@@ -896,10 +926,10 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 		CU(cudaMemsetAsync(sc.sums, 0, (size_t)n * 16, h->stream));
 		DcSumParams d;
 		d.img = sc.img;
-		d.stride = h->image_stride;
-		d.l_len = h->l_len;
+		d.stride = h->shape.image_stride;
+		d.l_len = h->shape.l_len;
 		d.sums = sc.sums;
-		int nI = (h->l_len + 1) / 2;
+		int nI = (h->shape.l_len + 1) / 2;
 		dim3 grid_dc(std::max(1, std::min((nI + 1023) / 1024, 64)), n);
 		dc_sums_c16_kernel<<<grid_dc, 256, 0, h->stream>>>(d);
 		if ((rc = check_launch(h, "dc_sums_c16_kernel")))
@@ -909,7 +939,7 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 	f.sums = sc.sums;
 	f.ave = sc.ave;
 	f.n = n;
-	f.l_len = h->l_len;
+	f.l_len = h->shape.l_len;
 	dc_finalize_kernel<<<(2 * n + 255) / 256, 256, 0, h->stream>>>(f);
 	return check_launch(h, "dc_finalize_kernel");
 }
@@ -927,8 +957,8 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 	const int *d_hops = (const int *)(d_desc + lay.off_hops);
 	int rc = 0;
 	/* paths whose first kernel after a report is a transform kernel with a pdl_wait() keep the flag */
-	const bool pdl_path = h->path == PATH_SMALL_U8 || h->path == PATH_RMS ||
-			      (h->path == PATH_SMALL_DECIM && fused_boxcar_ok(h));
+	const bool pdl_path = h->shape.path == PATH_SMALL_U8 || h->shape.path == PATH_RMS ||
+			      (h->shape.path == PATH_SMALL_DECIM && fused_boxcar_ok(h));
 	if (!pdl_path || h->d_level)
 		h->last_was_epilogue = false;
 
@@ -946,7 +976,7 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 			return rc;
 	}
 
-	if (h->path == PATH_RMS) {
+	if (h->shape.path == PATH_RMS) {
 		RmsParams p;
 		p.base = base;
 		p.read_off = d_offs;
@@ -970,7 +1000,7 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 		return check_launch(h, "rms_kernel");
 	}
 
-	if (h->path == PATH_SMALL_U8) {
+	if (h->shape.path == PATH_SMALL_U8) {
 		SmallParams p;
 		memset(&p, 0, sizeof(p));
 		p.base = base;
@@ -980,7 +1010,7 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 		p.stagger_ns = h->dbg_stagger_ns;
 		p.avg = h->d_avg;
 		p.samples = h->d_smp64;
-		p.samples_per_read = h->samples_per_read;
+		p.samples_per_read = h->shape.samples_per_read;
 		p.tw = h->d_tw;
 		p.twc = h->d_twc;
 		p.win = h->d_win;
@@ -989,7 +1019,7 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 		return launch_small(h, p, false);
 	}
 
-	if (h->path == PATH_SMALL_DECIM && fused_boxcar_ok(h)) {
+	if (h->shape.path == PATH_SMALL_DECIM && fused_boxcar_ok(h)) {
 		FusedBoxcarParams p;
 		memset(&p, 0, sizeof(p));
 		p.base = base;
@@ -1006,7 +1036,7 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 		return launch_fused_boxcar(h, p);
 	}
 
-	if (h->path == PATH_SMALL_DECIM) {
+	if (h->shape.path == PATH_SMALL_DECIM) {
 		/* Entries are processed in chunks cut at segment boundaries.  Chunks alternate between
 		 * two auxiliary streams and two scratch halves, so the decimators of one chunk (HBM
 		 * bound) run while the transform of the previous one (issue bound) is still busy. */
@@ -1063,20 +1093,20 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 				memset(&p, 0, sizeof(p));
 				p.base = (const uint8_t *)sc.img;
 				p.read_off = nullptr; /* images are contiguous: entry e at (e - e0) * image bytes */
-				p.regular_stride = h->image_stride * 4;
+				p.regular_stride = h->shape.image_stride * 4;
 				p.entry_base = e0;
 				p.segs = d_segs + si;
 				p.n_segs = (int)(sj - si);
 				p.avg = h->d_avg;
 				p.samples = h->d_smp64;
-				p.samples_per_read = h->samples_per_read;
+				p.samples_per_read = h->shape.samples_per_read;
 				p.tw = h->d_tw;
 				p.twc = h->d_twc;
 				p.win = h->d_win;
 				p.dc_ave = sc.ave;
-				p.l_len = h->l_len;
-				p.n_blocks = h->n_blocks;
-				p.blocks_padded = h->blocks_padded;
+				p.l_len = h->shape.l_len;
+				p.n_blocks = h->shape.n_blocks;
+				p.blocks_padded = h->shape.blocks_padded;
 				p.tw0 = h->tw0;
 				rc = launch_small(h, p, true);
 			}
@@ -1128,7 +1158,7 @@ int process_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const std::vector<lon
 	if (rc)
 		return rc;
 	for (int i = 0; i < n; i++) {
-		h->samples[hops[i]] += h->samples_per_read;
+		h->samples[hops[i]] += h->shape.samples_per_read;
 		if (h->d_level)
 			h->level_bytes[hops[i]] += (uint64_t)h->cfg.buf_len;
 	}
@@ -1284,13 +1314,13 @@ int run_epilogue(rtlsdr_gpu_scan *h, int hop0, int nhops, double *db, long long 
 	p.avg_out = avg_out;
 	p.samples_out = samples_out;
 	p.bin_e = h->cfg.bin_e;
-	p.i1 = h->db_i1;
-	p.i2 = h->db_i2;
+	p.i1 = h->shape.db_i1;
+	p.i2 = h->shape.db_i2;
 	p.rate = h->cfg.rate;
 	p.hop0 = hop0;
 	p.iir = h->d_iir;
 	p.iir_alpha = h->cfg.iir_alpha;
-	const int span = std::max(h->db_count, avg_out ? h->N : 0);
+	const int span = std::max(h->shape.db_count, avg_out ? h->shape.N : 0);
 	dim3 grid((span + 255) / 256, nhops);
 	epilogue_kernel<<<grid, 256, 0, h->stream>>>(p);
 	h->last_was_epilogue = zero_after; /* nothing else follows it on the stream in the fused-zero case */
@@ -1300,7 +1330,7 @@ int run_epilogue(rtlsdr_gpu_scan *h, int hop0, int nhops, double *db, long long 
 /* bytes of `rows` CSV rows at their widest (csv_text.cuh) */
 size_t csv_bound(const rtlsdr_gpu_scan *h, int rows, size_t stamp_len)
 {
-	return (size_t)rows * (stamp_len + kCsvRowFixed + (size_t)kCsvValueMax * (size_t)h->db_count);
+	return (size_t)rows * (stamp_len + kCsvRowFixed + (size_t)kCsvValueMax * (size_t)h->shape.db_count);
 }
 
 /* rows [row_first, row_first + rows) of the column table, from dB rows and int32 counts in device memory, into
@@ -1323,7 +1353,7 @@ int run_csv(rtlsdr_gpu_scan *h, const char *stamp, size_t stamp_len, int row_fir
 	p.cols = h->d_csv_cols;
 	p.step = h->csv_step;
 	p.row_first = row_first;
-	p.db_count = h->db_count;
+	p.db_count = h->shape.db_count;
 	p.slots = h->d_csv_slots;
 	p.slot_bytes = (long long)slot;
 	p.lens = h->d_csv_lens;
@@ -1425,37 +1455,34 @@ int rtlsdr_gpu_scan_init(const rtlsdr_gpu_scan_cfg_t *cfg_in, rtlsdr_gpu_scan_t 
 	memset(&full, 0, sizeof(full));
 	memcpy(&full, cfg_in, cfg_in->struct_size); /* fields a shorter (older) struct lacks stay 0 */
 	const rtlsdr_gpu_scan_cfg_t *cfg = &full;
-	if (!(cfg->iir_alpha >= 0.0 && cfg->iir_alpha <= 1.0))
-		return RTLSDR_GPU_ERR_CONFIG;
-	if (cfg->tune_count <= 0 || cfg->tune_count > 3000 /* MAX_TUNES, rtl_power.c:113 */ ||
-	    cfg->bin_e < 0 || cfg->bin_e > 21 /* rtl_power.c:483 */ || cfg->downsample < 1 ||
-	    cfg->downsample_passes < 0 || cfg->downsample_passes > 20 || cfg->buf_len < 16 ||
-	    (cfg->buf_len & 15) || cfg->rate <= 0 || !(cfg->crop >= 0.0 && cfg->crop <= 1.0))
-		return RTLSDR_GPU_ERR_CONFIG;
-	const int N = 1 << cfg->bin_e;
-	const bool box = cfg->boxcar && cfg->downsample > 1;
-	const bool hb = !box && cfg->downsample_passes > 0;
-	if (hb && cfg->downsample != (1 << cfg->downsample_passes))
-		return RTLSDR_GPU_ERR_CONFIG;
-	if (hb && ((cfg->buf_len >> cfg->downsample_passes) < 24 || (cfg->buf_len & ((4 << cfg->downsample_passes) - 1))))
-		return RTLSDR_GPU_ERR_CONFIG;
-	if (!box && !hb && cfg->downsample != 1 && cfg->bin_e > 0) {
-		/* ds > 1 without a decimator: the reference would still divide lengths by ds
-		 * (rtl_power.c:692-695); the planner never produces this, reject it */
-		return RTLSDR_GPU_ERR_CONFIG;
+	ScanShape shape;
+	int rc = scan_shape(*cfg, &shape);
+	if (rc)
+		return rc;
+	const int L = cfg->bin_e, N = shape.N;
+
+	/* host tables: built, and the sine table checked, before any device work */
+	std::vector<int2> tw, twc, twb;
+	std::vector<uint16_t> win;
+	PassTw tw0 = {};
+	if (L > 0) {
+		std::vector<int16_t> sine((size_t)N * 3 / 4);
+		if (!cfg->sinewave)
+			host_sine_table(L, sine.data());
+		if ((rc = twiddles(cfg->sinewave ? cfg->sinewave : sine.data(), L, tw)))
+			return rc;
+		tw0 = first_stage_tw(tw, L);
+		twc = compact_tw(tw, L, shape.path == PATH_LARGE ? 8 : L);
+		if (shape.path == PATH_LARGE)
+			twb = round_b_tw(tw, L);
+		win = window16(cfg->window_coefs, N);
 	}
 
 	int ndev = 0;
-	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || cfg->device < 0 || cfg->device >= ndev) {
-		cudaGetLastError();
-		return RTLSDR_GPU_ERR_NO_DEVICE;
-	}
 	cudaDeviceProp prop;
-	if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess || prop.major != 10) {
-		cudaGetLastError();
-		return RTLSDR_GPU_ERR_NO_DEVICE;
-	}
-	if (cudaSetDevice(cfg->device) != cudaSuccess) {
+	if (cudaGetDeviceCount(&ndev) != cudaSuccess || cfg->device < 0 || cfg->device >= ndev ||
+	    cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess || prop.major != 10 ||
+	    cudaSetDevice(cfg->device) != cudaSuccess) {
 		cudaGetLastError();
 		return RTLSDR_GPU_ERR_NO_DEVICE;
 	}
@@ -1464,76 +1491,25 @@ int rtlsdr_gpu_scan_init(const rtlsdr_gpu_scan_cfg_t *cfg_in, rtlsdr_gpu_scan_t 
 	if (!h)
 		return RTLSDR_GPU_ERR_NOMEM;
 	h->cfg = *cfg;
-	if (const char *f = getenv("RTLSDR_GPU_BOXCAR_STREAM")) {
-		const int m = atoi(f);
-		if (m != 0 && m != 1 && m != 2 && m != 3 && m != 5) {
-			delete h;
-			return RTLSDR_GPU_ERR_CONFIG; /* not a kernel variant */
-		}
-		h->dbg_boxcar_mode = m;
+	if ((rc = read_debug_switches(h))) {
+		delete h;
+		return rc;
 	}
-	h->dbg_no_fused_boxcar = getenv("RTLSDR_GPU_NO_FUSED_BOXCAR") != nullptr;
-	if (const char *f = getenv("RTLSDR_GPU_STAGGER_NS"))
-		h->dbg_stagger_ns = atoi(f);
-	h->dbg_no_hb_stream = getenv("RTLSDR_GPU_NO_HB_STREAM") != nullptr;
-	if (const char *f = getenv("RTLSDR_GPU_LARGE_PIPE")) /* A/B switch: 0 = one-tile-per-CTA round B for N >= 2^17 */
-		h->dbg_large_pipe = atoi(f) != 0;
-	h->dbg_rms_warp = getenv("RTLSDR_GPU_RMS_WARP") != nullptr; /* 1-bin hops: warp-per-read kernel instead of CTA-per-read */
 	h->cfg.window_coefs = nullptr;
 	h->cfg.sinewave = nullptr;
-	h->N = N;
+	h->shape = shape;
+	h->tw0 = tw0;
 	h->num_sms = prop.multiProcessorCount;
 	h->samples.assign(cfg->tune_count, 0);
 
-	/* geometry of one read (rtl_power.c:692-695, 717) */
-	if (cfg->bin_e == 0) {
-		h->path = PATH_RMS;
-		h->samples_per_read = 1;
-	} else {
-		h->l_len = cfg->buf_len / cfg->downsample;
-		h->n_blocks = (h->l_len + 2 * N - 1) / (2 * N);
-		h->samples_per_read = h->n_blocks * cfg->downsample;
-		if (cfg->bin_e <= 12) {
-			if (!box && !hb) {
-				if (cfg->buf_len != kStageBytes) {
-					delete h;
-					return RTLSDR_GPU_ERR_CONFIG; /* planner gives 16384 whenever 2N <= 16384 (rtl_power.c:501-504) */
-				}
-				h->path = PATH_SMALL_U8;
-			} else {
-				h->path = PATH_SMALL_DECIM;
-				/* images of consecutive reads are contiguous; keep each 16-byte aligned */
-				h->blocks_padded = h->n_blocks;
-				while (((long long)h->blocks_padded * N) % 4)
-					h->blocks_padded++;
-				h->image_stride = (long long)h->blocks_padded * N;
-			}
-		} else {
-			h->path = PATH_LARGE;
-			if (h->n_blocks != 1 || (box || hb ? h->l_len != 2 * N : cfg->buf_len != 2 * N)) {
-				delete h;
-				return RTLSDR_GPU_ERR_CONFIG; /* 2N*ds >= 16384 always holds here, so one block per read */
-			}
-			h->image_stride = N;
-		}
-	}
-	/* what csv_dbm prints (rtl_power.c:741-748) */
-	h->db_i1 = 0 + (int)((double)N * cfg->crop * 0.5);
-	h->db_i2 = (N - 1) - (int)((double)N * cfg->crop * 0.5);
-	if (h->db_i2 < h->db_i1) {
-		delete h;
-		return RTLSDR_GPU_ERR_CONFIG;
-	}
-	h->db_count = h->db_i2 - h->db_i1 + 2;
-
-	int rc = RTLSDR_GPU_ERR_CUDA;
+	rc = RTLSDR_GPU_ERR_CUDA;
 	do {
 		if (cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking) != cudaSuccess)
 			break;
 		h->stream = h->own_stream;
 		const size_t avg_bytes = ((size_t)cfg->tune_count * N + (size_t)cfg->tune_count) * sizeof(long long);
 		if (cudaMalloc(&h->d_avg, avg_bytes) != cudaSuccess ||
-		    cudaMalloc(&h->d_db, (size_t)cfg->tune_count * h->db_count * sizeof(double)) != cudaSuccess ||
+		    cudaMalloc(&h->d_db, (size_t)cfg->tune_count * h->shape.db_count * sizeof(double)) != cudaSuccess ||
 		    cudaMalloc(&h->d_samples, (size_t)cfg->tune_count * sizeof(int)) != cudaSuccess ||
 		    cudaMallocHost(&h->h_samples_pinned, (size_t)cfg->tune_count * sizeof(int)) != cudaSuccess) {
 			rc = RTLSDR_GPU_ERR_NOMEM;
@@ -1541,127 +1517,28 @@ int rtlsdr_gpu_scan_init(const rtlsdr_gpu_scan_cfg_t *cfg_in, rtlsdr_gpu_scan_t 
 		}
 		h->d_smp64 = h->d_avg + (size_t)cfg->tune_count * N;
 		if (cfg->flags & RTLSDR_GPU_FLAG_ASYNC_REPORT) {
-			if (cudaMalloc(&h->d_avg_other, avg_bytes) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemsetAsync(h->d_avg_other, 0, avg_bytes, h->stream) != cudaSuccess ||
+			if (!alloc_fill(&h->d_avg_other, avg_bytes, 0, h->stream, &rc) ||
 			    cudaStreamCreateWithFlags(&h->report_stream, cudaStreamNonBlocking) != cudaSuccess ||
 			    cudaEventCreateWithFlags(&h->ev_scan, cudaEventDisableTiming) != cudaSuccess ||
 			    cudaEventCreateWithFlags(&h->ev_report[0], cudaEventDisableTiming) != cudaSuccess ||
 			    cudaEventCreateWithFlags(&h->ev_report[1], cudaEventDisableTiming) != cudaSuccess)
 				break;
 		}
-		if (cudaMalloc(&h->d_done, (size_t)cfg->tune_count * sizeof(unsigned)) != cudaSuccess) {
-			rc = RTLSDR_GPU_ERR_NOMEM;
+		if (!alloc_fill(&h->d_done, (size_t)cfg->tune_count * sizeof(unsigned), 0, h->stream, &rc) ||
+		    cudaMemsetAsync(h->d_avg, 0, avg_bytes, h->stream) != cudaSuccess)
 			break;
-		}
-		if (cudaMemsetAsync(h->d_done, 0, (size_t)cfg->tune_count * sizeof(unsigned), h->stream) != cudaSuccess)
+		/* smoothing state of the printed bins, NaN (all bits set) = no report yet */
+		const size_t iir_bytes = (size_t)cfg->tune_count * (size_t)(h->shape.db_count - 1) * sizeof(double);
+		if (cfg->iir_alpha > 0.0 && !alloc_fill(&h->d_iir, iir_bytes, 0xFF, h->stream, &rc))
 			break;
-		if (cudaMemsetAsync(h->d_avg, 0, avg_bytes, h->stream) != cudaSuccess)
-			break;
-		if (cfg->iir_alpha > 0.0) {
-			/* smoothing state of the printed bins, NaN (all bits set) = no report yet */
-			const size_t ib = (size_t)cfg->tune_count * (size_t)(h->db_count - 1) * sizeof(double);
-			if (cudaMalloc(&h->d_iir, ib) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemsetAsync(h->d_iir, 0xFF, ib, h->stream) != cudaSuccess)
-				break;
-		}
 		if (cfg->flags & RTLSDR_GPU_FLAG_LEVEL_STATS) {
-			const size_t lb = (size_t)cfg->tune_count * 2 * sizeof(unsigned long long);
-			if (cudaMalloc(&h->d_level, lb) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemsetAsync(h->d_level, 0, lb, h->stream) != cudaSuccess)
+			if (!alloc_fill(&h->d_level, (size_t)cfg->tune_count * 2 * sizeof(unsigned long long), 0, h->stream, &rc))
 				break;
 			h->level_bytes.assign(cfg->tune_count, 0);
 		}
-
-		if (cfg->bin_e > 0) {
-			/* twiddles: wr = Sinewave[j+N/4] >> 1, wi = (-Sinewave[j]) >> 1 (rtl_power.c:305-308) */
-			std::vector<int16_t> sine((size_t)N * 3 / 4 + 4, 0);
-			if (cfg->sinewave)
-				memcpy(sine.data(), cfg->sinewave, ((size_t)N * 3 / 4) * sizeof(int16_t));
-			else
-				host_sine_table(cfg->bin_e, sine.data());
-			const int half = std::max(N / 2, 1);
-			h->tw_host.resize(half);
-			for (int j = 0; j < half; j++) {
-				int16_t wr = (int16_t)(sine[j + N / 4] >> 1);
-				int16_t wi = (int16_t)((int16_t)(-sine[j]) >> 1);
-				h->tw_host[j] = make_int2(wr, wi);
-			}
-			/* the kernels special-case the angle-0 and quarter-turn groups of the first
-			 * four stages: (wr, 0) and (0, wi).  True for every table sine_table()
-			 * builds (Sinewave[0] = Sinewave[N/2] = 0); reject tables where it is not. */
-			if (h->tw_host[0].y != 0 || (N >= 4 && h->tw_host[N / 4].x != 0)) {
-				rc = RTLSDR_GPU_ERR_CONFIG;
-				break;
-			}
-			memset(&h->tw0, 0, sizeof(h->tw0));
-			for (int b = 0; b < 4 && b < cfg->bin_e; b++)
-				for (int g = 0; g < (1 << b); g++)
-					h->tw0.w[(1 << b) - 1 + g] = h->tw_host[(size_t)g << (cfg->bin_e - 1 - b)];
-			std::vector<uint16_t> win(N);
-			for (int i = 0; i < N; i++)
-				win[i] = (uint16_t)((cfg->window_coefs ? cfg->window_coefs[i] : 256) & 0xFFFF);
-			if (cudaMalloc(&h->d_tw, (size_t)half * sizeof(int2)) != cudaSuccess ||
-			    cudaMalloc(&h->d_win, (size_t)N * sizeof(uint16_t)) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemcpy(h->d_tw, h->tw_host.data(), (size_t)half * sizeof(int2), cudaMemcpyHostToDevice) != cudaSuccess ||
-			    cudaMemcpy(h->d_win, win.data(), (size_t)N * sizeof(uint16_t), cudaMemcpyHostToDevice) != cudaSuccess)
-				break;
-		}
-
-		if (cfg->bin_e > 4 && cfg->bin_e <= 12) {
-			/* compact table: stage s (4..L-1), group m at (1<<s)-16+m = tw[m << (L-1-s)] */
-			const int L = cfg->bin_e;
-			std::vector<int2> twc((size_t)N - 16);
-			for (int st = 4; st < L; st++)
-				for (int m = 0; m < (1 << st); m++)
-					twc[(size_t)(1 << st) - 16 + m] = h->tw_host[(size_t)m << (L - 1 - st)];
-			if (cudaMalloc(&h->d_twc, twc.size() * sizeof(int2)) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemcpy(h->d_twc, twc.data(), twc.size() * sizeof(int2), cudaMemcpyHostToDevice) != cudaSuccess)
-				break;
-		}
-		if (h->path == PATH_LARGE) {
-			/* round A's compact table: stage s (4..7), group m at (1<<s)-16+m = tw[m << (L-1-s)] */
-			std::vector<int2> twc(240);
-			for (int st = 4; st < 8; st++)
-				for (int m = 0; m < (1 << st); m++)
-					twc[(size_t)(1 << st) - 16 + m] = h->tw_host[(size_t)m << (cfg->bin_e - 1 - st)];
-			if (cudaMalloc(&h->d_twc, twc.size() * sizeof(int2)) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemcpy(h->d_twc, twc.data(), twc.size() * sizeof(int2), cudaMemcpyHostToDevice) != cudaSuccess)
-				break;
-		}
-		if (h->path == PATH_LARGE) {
-			/* twb[se][plow][ilow] = tw[((ilow << 8) | plow) << (L-9-se)], se = 4 .. min(8, L-8)-1 */
-			const int L = cfg->bin_e, lb = std::min(8, L - 8);
-			std::vector<int2> twb((size_t)256 * 240, make_int2(0, 0));
-			for (int se = 4; se < lb; se++)
-				for (int plow = 0; plow < 256; plow++)
-					for (int ilow = 0; ilow < (1 << se); ilow++)
-						twb[(size_t)256 * ((1 << se) - 16) + ((size_t)plow << se) + ilow] =
-							h->tw_host[((size_t)((ilow << 8) | plow)) << (L - 9 - se)];
-			if (cudaMalloc(&h->d_twb, twb.size() * sizeof(int2)) != cudaSuccess) {
-				rc = RTLSDR_GPU_ERR_NOMEM;
-				break;
-			}
-			if (cudaMemcpy(h->d_twb, twb.data(), twb.size() * sizeof(int2), cudaMemcpyHostToDevice) != cudaSuccess)
-				break;
-		}
+		if (!upload(&h->d_tw, tw, &rc) || !upload(&h->d_win, win, &rc) || !upload(&h->d_twc, twc, &rc) ||
+		    !upload(&h->d_twb, twb, &rc))
+			break;
 
 		/* staging ring */
 		size_t ring = cfg->ring_bytes ? cfg->ring_bytes : kDefaultRing;
@@ -1837,7 +1714,7 @@ static int submit_regular(rtlsdr_gpu_scan_t *h, int hop_first, int hop_count, in
 	if (rc)
 		return rc;
 	for (int k = 0; k < hop_count; k++) {
-		h->samples[hop_first + k] += h->samples_per_read * passes;
+		h->samples[hop_first + k] += h->shape.samples_per_read * passes;
 		if (h->d_level)
 			h->level_bytes[hop_first + k] += (uint64_t)h->cfg.buf_len * (uint64_t)passes;
 	}
@@ -2055,7 +1932,7 @@ int rtlsdr_gpu_scan_flag_wait(void *cuda_stream, const void *dev_flags, int coun
 
 int rtlsdr_gpu_scan_db_count(const rtlsdr_gpu_scan_t *h)
 {
-	return h ? h->db_count : RTLSDR_GPU_ERR_NULL;
+	return h ? h->shape.db_count : RTLSDR_GPU_ERR_NULL;
 }
 
 static int collect_range(rtlsdr_gpu_scan_t *h, int hop0, int nhops, int64_t *avg, int *samples, double *db)
@@ -2064,12 +1941,12 @@ static int collect_range(rtlsdr_gpu_scan_t *h, int hop0, int nhops, int64_t *avg
 	int rc = flush_ring(h);
 	if (rc)
 		return rc;
-	const size_t N = (size_t)h->N;
+	const size_t N = (size_t)h->shape.N;
 	if (db) {
 		if ((rc = run_epilogue(h, hop0, nhops, h->d_db, nullptr, nullptr)))
 			return rc;
-		CU(cudaMemcpyAsync(db, h->d_db, (size_t)nhops * h->db_count * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-		h->d2h += (uint64_t)nhops * h->db_count * sizeof(double);
+		CU(cudaMemcpyAsync(db, h->d_db, (size_t)nhops * h->shape.db_count * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+		h->d2h += (uint64_t)nhops * h->shape.db_count * sizeof(double);
 	}
 	if (avg) {
 		CU(cudaMemcpyAsync(avg, h->d_avg + (size_t)hop0 * N, (size_t)nhops * N * sizeof(long long),
@@ -2129,7 +2006,7 @@ int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *de
 	int rc = flush_ring(h);
 	if (rc)
 		return rc;
-	const size_t N = (size_t)h->N, tc = (size_t)h->cfg.tune_count;
+	const size_t N = (size_t)h->shape.N, tc = (size_t)h->cfg.tune_count;
 	/* one kernel writes dB rows, raw bins and sample counts straight into the
 	 * caller's buffers (e.g. the NCCL send buffer), one memset clears the state */
 	/* up to 8192 bins the last epilogue block of a hop also zeroes it (no memset launch) */
@@ -2245,7 +2122,7 @@ int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *t
 	/* the epilogue's dB rows and counts stay on the device: only the text crosses PCIe */
 	if ((rc = run_epilogue(h, 0, tc, h->d_db, nullptr, h->d_samples)))
 		return rc;
-	if ((rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_db, h->db_count, h->d_samples, h->d_csv_text, h->d_csv_len)))
+	if ((rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_db, h->shape.db_count, h->d_samples, h->d_csv_text, h->d_csv_len)))
 		return rc;
 	CU(cudaMemcpyAsync(h->h_csv_len, h->d_csv_len, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
 	CU(cudaStreamSynchronize(h->stream));
@@ -2255,7 +2132,7 @@ int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *t
 	CU(cudaMemcpyAsync(text, h->d_csv_text, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
 	h->d2h += (uint64_t)n + sizeof(long long);
 	/* read-and-zero, like csv_dbm (rtl_power.c:761-764) */
-	CU(cudaMemsetAsync(h->d_avg, 0, ((size_t)tc * h->N + (size_t)tc) * sizeof(long long), h->stream));
+	CU(cudaMemsetAsync(h->d_avg, 0, ((size_t)tc * h->shape.N + (size_t)tc) * sizeof(long long), h->stream));
 	if (h->d_level)
 		CU(cudaMemsetAsync(h->d_level, 0, (size_t)tc * 2 * sizeof(unsigned long long), h->stream));
 	CU(cudaStreamSynchronize(h->stream));
@@ -2276,7 +2153,7 @@ int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, i
 	if (((uintptr_t)dev_db & 7) || ((uintptr_t)dev_samples & 3) || ((uintptr_t)dev_len & 7))
 		return RTLSDR_GPU_ERR_ALIGN;
 	const size_t stamp_len = strlen(stamp);
-	if (stamp_len >= (size_t)kCsvStampMax || !h->d_csv_cols || db_stride < h->db_count)
+	if (stamp_len >= (size_t)kCsvStampMax || !h->d_csv_cols || db_stride < h->shape.db_count)
 		return RTLSDR_GPU_ERR_CONFIG;
 	if (rows < 1 || row_first < 0 || row_first > h->csv_rows - rows)
 		return RTLSDR_GPU_ERR_HOP;
@@ -2306,7 +2183,7 @@ int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, cons
 	p.ext_avg = (const uint8_t *)dev_avg;
 	p.ext_smp = (const uint8_t *)dev_samples;
 	p.stride = set_stride;
-	p.bins = (long long)h->cfg.tune_count * h->N;
+	p.bins = (long long)h->cfg.tune_count * h->shape.N;
 	p.hops = h->cfg.tune_count;
 	p.sets = sets;
 	p.peak = h->cfg.peak_hold ? 1 : 0;

@@ -5,6 +5,7 @@
  * oracle on a box without a GPU.  Built by tests/test_emu_kernels.py with
  *   g++ -std=c++20 -O2 -DSCAN_EMU -Itests/emu -Irtlsdr_b200/csrc -shared -fPIC
  */
+#include "scan_host.cuh"
 #include "scan_kernels.cuh"
 #include "scan_large.cuh"
 
@@ -51,22 +52,19 @@ void run_small(int L, const SmallParams &prm, int peak, int in16)
 	}
 }
 
-std::vector<int2> compact_tw(const int2 *tw, int L)
-{
-	std::vector<int2> twc((size_t)(L > 4 ? (1 << L) - 16 : 1));
-	for (int st = 4; st < L; st++)
-		for (int m = 0; m < (1 << st); m++)
-			twc[(size_t)(1 << st) - 16 + m] = tw[(size_t)m << (L - 1 - st)];
-	return twc;
-}
-
-void fill_tw0(PassTw &tw0, const int2 *tw, int L)
-{
-	memset(&tw0, 0, sizeof(tw0));
-	for (int b = 0; b < 4 && b < L; b++)
-		for (int g = 0; g < (1 << b); g++)
-			tw0.w[(1 << b) - 1 + g] = tw[(size_t)g << (L - 1 - b)];
-}
+/* the tables rtlsdr_gpu_scan_init() builds (scan_host.cuh), from the oracle's Sinewave[] and window_coefs[] */
+struct Tables {
+	std::vector<int2> tw, twc;
+	std::vector<uint16_t> win;
+	PassTw tw0;
+	Tables(const int16_t *sine, const int32_t *coefs, int L, int s_end)
+	{
+		twiddles(sine, L, tw); /* the oracle's sine_table() always passes the check */
+		tw0 = first_stage_tw(tw, L);
+		twc = compact_tw(tw, L, s_end);
+		win = window16(coefs, 1 << L);
+	}
+};
 
 } // namespace
 
@@ -74,8 +72,9 @@ extern "C" {
 
 /* u8 path: reads [n_reads][16384] sorted by hop, hop_of [n_reads]; `grid` CTAs share the working sets in equal runs */
 void emu_small_u8(int L, int peak, const uint8_t *reads, int n_reads, const int *hop_of, int grid,
-		  const int *tw /* [N/2][2] */, const uint16_t *win, long long *avg, long long *samples)
+		  const int16_t *sine, const int32_t *win, long long *avg, long long *samples)
 {
+	const Tables t(sine, win, L, L);
 	std::vector<long long> offs(n_reads);
 	for (int i = 0; i < n_reads; i++)
 		offs[i] = (long long)i * kStageBytes;
@@ -89,11 +88,10 @@ void emu_small_u8(int L, int peak, const uint8_t *reads, int n_reads, const int 
 	p.avg = avg;
 	p.samples = samples;
 	p.samples_per_read = kStageBytes / (2 << L); /* FFT blocks per read (ds = 1) */
-	p.tw = (const int2 *)tw;
-	std::vector<int2> twc = compact_tw(p.tw, L);
-	p.twc = twc.data();
-	p.win = win;
-	fill_tw0(p.tw0, p.tw, L);
+	p.tw = t.tw.data();
+	p.twc = t.twc.data();
+	p.win = t.win.data();
+	p.tw0 = t.tw0;
 	run_small(L, p, peak, 0);
 }
 
@@ -105,16 +103,17 @@ static int g_hb_span = 64;
 void emu_set_hb_span(int span) { g_hb_span = span; }
 
 void emu_small_decim(int L, int peak, const uint8_t *reads, int n_reads, int buf_len, int ds, int ds_p,
-		     int mode, const int *fir5, const int *segs, int n_segs, const int *tw,
-		     const uint16_t *win, long long *avg, uint32_t *image_out, long long *sums_out)
+		     int mode, const int *fir5, const int *segs, int n_segs, const int16_t *sine,
+		     const int32_t *win, long long *avg, uint32_t *image_out, long long *sums_out)
 {
-	const int N = 1 << L, pairs = buf_len / 2;
-	const int l_len = buf_len / ds;
-	const int n_blocks = (l_len + 2 * N - 1) / (2 * N);
-	int blocks_padded = n_blocks;
-	while (((long long)blocks_padded * N) % 4)
-		blocks_padded++;
-	const long long stride = (long long)blocks_padded * N;
+	const rtlsdr_gpu_scan_cfg_t cfg = { .tune_count = 1, .bin_e = L, .buf_len = buf_len, .downsample = ds,
+					    .downsample_passes = ds_p, .boxcar = mode == 0, .rate = 1 };
+	ScanShape shape;
+	if (scan_shape(cfg, &shape))
+		return; /* avg stays 0 */
+	const Tables t(sine, win, L, L);
+	const int pairs = buf_len / 2, l_len = shape.l_len;
+	const long long stride = shape.image_stride;
 	std::vector<long long> offs(n_reads);
 	for (int i = 0; i < n_reads; i++)
 		offs[i] = (long long)i * buf_len;
@@ -146,7 +145,7 @@ void emu_small_decim(int L, int peak, const uint8_t *reads, int n_reads, int buf
 		else
 			cuda_emu::launch(grid, dim3(256), 0, [&]() { boxcar_kernel<2>(d); });
 	} else if (ds_p <= 7) {
-		const int M = pairs >> ds_p, cap0 = 8192;
+		const int M = pairs >> ds_p;
 		HalfbandChainParams hp;
 		hp.base = reads;
 		hp.read_off = offs.data();
@@ -159,16 +158,9 @@ void emu_small_decim(int L, int peak, const uint8_t *reads, int n_reads, int buf
 		hp.out_stride = stride;
 		hp.l_len = l_len;
 		hp.sums = sums.data();
-		int tile = (cap0 >> ds_p) - 16;
-		if (tile > 256) tile = 256;
-		if (tile < 8) tile = 8;
-		if (tile > M) tile = M;
 		const bool stream = mode == 2 && ds_p <= kHbStreamMaxPasses; /* mode 2: streaming kernel + 16-sample head tiles */
-		if (stream)
-			tile = kHbStreamHead;
-		hp.tile = tile;
-		hp.cap0 = stream ? 1024 : cap0;
-		cuda_emu::launch(dim3(stream ? 1 : (M + tile - 1) / tile, n_reads), dim3(stream ? 64 : 256), (hp.cap0 + hp.cap0 / 2 + 16) * 4,
+		const int smem = chain_tile(hp, stream);
+		cuda_emu::launch(dim3(stream ? 1 : (M + hp.tile - 1) / hp.tile, n_reads), dim3(stream ? 64 : 256), smem,
 				 [&]() { halfband_chain_kernel(hp); });
 		if (stream) {
 			HalfbandStreamParams q;
@@ -253,8 +245,8 @@ void emu_small_decim(int L, int peak, const uint8_t *reads, int n_reads, int buf
 	p.avg = avg;
 	p.samples = smp.data();
 	p.samples_per_read = 1;
-	p.tw = (const int2 *)tw;
-	p.win = win;
+	p.tw = t.tw.data();
+	p.win = t.win.data();
 	std::vector<int> ave((size_t)n_reads * 2, 0);
 	DcFinalizeParams fz;
 	fz.sums = sums.data();
@@ -264,11 +256,10 @@ void emu_small_decim(int L, int peak, const uint8_t *reads, int n_reads, int buf
 	cuda_emu::launch(dim3((2 * n_reads + 255) / 256), dim3(256), 0, [&]() { dc_finalize_kernel(fz); });
 	p.dc_ave = ave.data();
 	p.l_len = l_len;
-	p.n_blocks = n_blocks;
-	p.blocks_padded = blocks_padded;
-	std::vector<int2> twc = compact_tw(p.tw, L);
-	p.twc = twc.data();
-	fill_tw0(p.tw0, p.tw, L);
+	p.n_blocks = shape.n_blocks;
+	p.blocks_padded = shape.blocks_padded;
+	p.twc = t.twc.data();
+	p.tw0 = t.tw0;
 	run_small(L, p, peak, 1);
 }
 
@@ -346,9 +337,10 @@ void emu_level_stats(const uint8_t *reads, int n_reads, int buf_len, const int *
 
 /* fused boxcar + transform kernel: reads [n_reads][2*N*ds] */
 void emu_fused_boxcar(int L, int peak, const uint8_t *reads, int n_reads, int ds, int slots, const int *segs,
-		      int n_segs, const int *tw, const uint16_t *win, long long *avg, long long *samples)
+		      int n_segs, const int16_t *sine, const int32_t *win, long long *avg, long long *samples)
 {
 	const int N = 1 << L;
+	const Tables t(sine, win, L, L);
 	std::vector<long long> offs(n_reads);
 	for (int i = 0; i < n_reads; i++)
 		offs[i] = (long long)i * 2 * N * ds;
@@ -362,10 +354,9 @@ void emu_fused_boxcar(int L, int peak, const uint8_t *reads, int n_reads, int ds
 	p.slots = slots;
 	p.avg = avg;
 	p.samples = samples;
-	std::vector<int2> twc = compact_tw((const int2 *)tw, L);
-	p.twc = twc.data();
-	p.win = win;
-	fill_tw0(p.tw0, (const int2 *)tw, L);
+	p.twc = t.twc.data();
+	p.win = t.win.data();
+	p.tw0 = t.tw0;
 #define FBS(LV, PK, NSV)                                                                              \
 	cuda_emu::launch(dim3(n_segs), dim3(kThreads), FusedSmem<LV>::bytes(ds, NSV),                 \
 			 [&]() { scan_boxcar_fused_kernel<LV, PK, NSV>(p); })
@@ -390,9 +381,10 @@ void emu_fused_boxcar(int L, int peak, const uint8_t *reads, int n_reads, int ds
 
 /* warp-specialised streaming variant of the same pipeline (producer / boxcar / transform roles) */
 void emu_stream_boxcar(int L, int peak, int mode, const uint8_t *reads, int n_reads, int ds, int slots, int grid, const int *segs,
-		       int n_segs, const int *tw, const uint16_t *win, long long *avg, long long *samples)
+		       int n_segs, const int16_t *sine, const int32_t *win, long long *avg, long long *samples)
 {
 	const int N = 1 << L;
+	const Tables t(sine, win, L, L);
 	std::vector<long long> offs(n_reads);
 	for (int i = 0; i < n_reads; i++)
 		offs[i] = (long long)i * 2 * N * ds;
@@ -406,10 +398,9 @@ void emu_stream_boxcar(int L, int peak, int mode, const uint8_t *reads, int n_re
 	p.slots = slots;
 	p.avg = avg;
 	p.samples = samples;
-	std::vector<int2> twc = compact_tw((const int2 *)tw, L);
-	p.twc = twc.data();
-	p.win = win;
-	fill_tw0(p.tw0, (const int2 *)tw, L);
+	p.twc = t.twc.data();
+	p.win = t.win.data();
+	p.tw0 = t.tw0;
 #define SBM(LV, PK, FG, BG)                                                                           \
 	cuda_emu::launch(dim3(grid), dim3(StreamShape<FG, BG>::threads), StreamSmem<LV, FG>::bytes(ds, slots), \
 			 [&]() { scan_boxcar_stream_kernel<LV, PK, FG, BG>(p); })

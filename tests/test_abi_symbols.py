@@ -105,3 +105,9 @@ def test_config_validation_happens_before_any_device_work(lib):
     assert init(downsample=0) == -2
     assert init(boxcar=0, downsample=8, downsample_passes=2) == -2   # ds must be 2^passes with -F
     assert init(boxcar=0, downsample=3, downsample_passes=0) == -2   # ds > 1 without a decimator
+    assert init(bin_e=10, buf_len=32768) == -2       # u8 path: the planner's 16384-byte reads only
+    assert init(bin_e=14, buf_len=16384) == -2       # large path: exactly one FFT block per read
+    assert init(bin_e=1, crop=1.0) == -2             # the crop leaves no bin printed
+    sine = rs.sine_table(10)
+    sine[0] = 1                                      # the kernels need Sinewave[0] = Sinewave[N/2] = 0
+    assert init(sinewave=sine.ctypes.data) == -2

@@ -26,20 +26,11 @@ def vp(a):
 def emu():
     srcs = [os.path.join(EMU_DIR, f) for f in ("emu_entry.cpp", "emu_large.inl", "cuda_emu.h")]
     srcs += [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(".cuh")]
+    srcs.append(os.path.join(ROOT, "include", "rtlsdr_gpu_scan.h"))  # scan_host.cuh reads the config struct
     if not os.path.exists(EMU_SO) or any(os.path.getmtime(s) > os.path.getmtime(EMU_SO) for s in srcs):
         subprocess.run(["g++", "-std=c++20", "-O2", "-DSCAN_EMU", "-I" + EMU_DIR, "-I" + CSRC, "-shared",
                         "-fPIC", "-pthread", "-o", EMU_SO, os.path.join(EMU_DIR, "emu_entry.cpp")], check=True)
     return ctypes.CDLL(EMU_SO)
-
-
-def twiddles(sine, bin_e):
-    """wr = Sinewave[j + N/4] >> 1, wi = (-Sinewave[j]) >> 1 (rtl_power.c:305-308)"""
-    n = 1 << bin_e
-    s = np.concatenate([sine.astype(np.int16), np.zeros(4, np.int16)])
-    j = np.arange(max(n // 2, 1))
-    wr = (s[j + n // 4] >> 1).astype(np.int32)
-    wi = ((-s[j]).astype(np.int16) >> 1).astype(np.int32)
-    return np.ascontiguousarray(np.stack([wr, wi], 1))
 
 
 def sort_by_hop(reads, hops, tune_count, split=2):
@@ -70,14 +61,13 @@ def test_small_u8_kernel(emu, port_oracle, bin_e):
         want, want_smp, _ = expected(port_oracle, plan, win, reads, hops)
         sreads, shops, _ = sort_by_hop(reads, hops, 2)
         shops = np.ascontiguousarray(shops, dtype=np.int32)
-        tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-        w16 = (win & 0xFFFF).astype(np.uint16)
+        sine = port_oracle.sine_table(bin_e)
         # the CTAs share the 6 reads in equal runs (cut at whole reads in so short a launch): 1 CTA, uneven
         # runs (4, 5 CTAs), one read per CTA, and more CTAs than reads
         for grid in ((1, 5) if bin_e < 12 else (1, 2, 4, 5, 6, 9)):
             avg = np.zeros((2, n), dtype=np.int64)
             smp = np.zeros(2, dtype=np.int64)
-            emu.emu_small_u8(bin_e, peak, vp(sreads), len(sreads), vp(shops), grid, vp(tw), vp(w16), vp(avg), vp(smp))
+            emu.emu_small_u8(bin_e, peak, vp(sreads), len(sreads), vp(shops), grid, vp(sine), vp(win), vp(avg), vp(smp))
             assert np.array_equal(avg, want), (bin_e, peak, grid)
             assert np.array_equal(smp, want_smp), (bin_e, peak, grid)
 
@@ -95,11 +85,10 @@ def test_small_u8_kernel_half_read_cuts(emu, port_oracle, bin_e, peak):
     want, want_smp, _ = expected(port_oracle, plan, win, reads, hops)
     sreads, shops, _ = sort_by_hop(reads, hops, 3)
     shops = np.ascontiguousarray(shops, dtype=np.int32)
-    tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-    w16 = (win & 0xFFFF).astype(np.uint16)
+    sine = port_oracle.sine_table(bin_e)
     avg = np.zeros((3, n), dtype=np.int64)
     smp = np.zeros(3, dtype=np.int64)
-    emu.emu_small_u8(bin_e, peak, vp(sreads), len(sreads), vp(shops), 2, vp(tw), vp(w16), vp(avg), vp(smp))
+    emu.emu_small_u8(bin_e, peak, vp(sreads), len(sreads), vp(shops), 2, vp(sine), vp(win), vp(avg), vp(smp))
     assert np.array_equal(avg, want)
     assert np.array_equal(smp, want_smp)
 
@@ -121,15 +110,14 @@ def test_decimating_kernels(emu, port_oracle, freq, window, fir, peak):
         reads, hops = make_reads(port_oracle.lib, plan, 2, mode, seed=3, param=param)
         want, _, _ = expected(port_oracle, plan, win, reads, hops)
         segs = np.array([(0, 0, len(reads), 0)], dtype=np.int32)
-        tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-        w16 = (win & 0xFFFF).astype(np.uint16)
+        sine = port_oracle.sine_table(bin_e)
         avg = np.zeros((1, n), dtype=np.int64)
         box = plan["boxcar"] and plan["downsample"] > 1
         fir5 = None
         if not box and plan["comp_fir_size"] == 9 and plan["downsample_passes"] <= 10:
             fir5 = np.array(list(port_oracle.lib.oracle_cic9(plan["downsample_passes"]).contents)[1:6], dtype=np.int32)
         emu.emu_small_decim(bin_e, peak, vp(reads), len(reads), plan["buf_len"], plan["downsample"],
-                            plan["downsample_passes"], 0 if box else 1, vp(fir5), vp(segs), 1, vp(tw), vp(w16),
+                            plan["downsample_passes"], 0 if box else 1, vp(fir5), vp(segs), 1, vp(sine), vp(win),
                             vp(avg), None, None)
         assert np.array_equal(avg, want), (freq, mode)
 
@@ -143,14 +131,13 @@ def test_large_kernels(emu, port_oracle, bin_e, peak):
     reads, hops = reads[:3], hops[:3]
     want, _, _ = expected(port_oracle, plan, win, reads, hops)
     sreads, shops, _ = sort_by_hop(reads, hops, 2)
-    tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-    w16 = (win & 0xFFFF).astype(np.uint16)
+    sine = port_oracle.sine_table(bin_e)
     avg = np.zeros((2, n), dtype=np.int64)
     # pipelined round B (the default for N >= 2^17) and the one-tile-per-CTA kernel it replaces (A/B switch)
     for pipe in (1, 0):
         avg[:] = 0
         emu.emu_set_large_pipe(pipe)
-        emu.emu_large(bin_e, peak, 0, vp(sreads), len(sreads), vp(shops.astype(np.int32)), vp(tw), vp(w16), None, vp(avg))
+        emu.emu_large(bin_e, peak, 0, vp(sreads), len(sreads), vp(shops.astype(np.int32)), vp(sine), vp(win), None, vp(avg))
         assert np.array_equal(avg, want), pipe
     emu.emu_set_large_pipe(1)
 
@@ -197,11 +184,10 @@ def test_decimating_small_n_multi_segment(emu, port_oracle, bin_e, ds):
     reads, hops = reads[:5], hops[:5]
     want, _, _ = expected(port_oracle, plan, win, reads, hops)
     sreads, shops, segs = sort_by_hop(reads, hops, 2, split=2)
-    tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-    w16 = (win & 0xFFFF).astype(np.uint16)
+    sine = port_oracle.sine_table(bin_e)
     avg = np.zeros((2, n), dtype=np.int64)
     emu.emu_small_decim(bin_e, plan["peak_hold"], vp(sreads), len(sreads), buf_len, ds, 0, 0, None, vp(segs),
-                        len(segs), vp(tw), vp(w16), vp(avg), None, None)
+                        len(segs), vp(sine), vp(win), vp(avg), None, None)
     assert np.array_equal(avg, want)
 
 
@@ -218,13 +204,12 @@ def test_fifth_order_chain_every_depth(emu, port_oracle, passes, fir):
     reads[1, 100:300] = 255
     want, _, _ = expected(port_oracle, plan, win, reads, hops)
     segs = np.array([(0, 0, 2, 0)], dtype=np.int32)
-    tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-    w16 = (win & 0xFFFF).astype(np.uint16)
+    sine = port_oracle.sine_table(bin_e)
     avg = np.zeros((1, n), dtype=np.int64)
     fir5 = None
     if fir == 9 and passes <= 10:
         fir5 = np.array(list(port_oracle.lib.oracle_cic9(passes).contents)[1:6], dtype=np.int32)
-    emu.emu_small_decim(bin_e, 0, vp(reads), 2, buf_len, ds, passes, 1, vp(fir5), vp(segs), 1, vp(tw), vp(w16),
+    emu.emu_small_decim(bin_e, 0, vp(reads), 2, buf_len, ds, passes, 1, vp(fir5), vp(segs), 1, vp(sine), vp(win),
                         vp(avg), None, None)
     assert np.array_equal(avg, want)
 
@@ -256,11 +241,10 @@ def test_fused_boxcar_kernel(emu, port_oracle, bin_e, ds, slots):
         reads[3, :] = 255
         want, want_smp, _ = expected(port_oracle, plan, win, reads, hops)
         sreads, _, segs = sort_by_hop(reads, hops, 2, split=2)
-        tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-        w16 = (win & 0xFFFF).astype(np.uint16)
+        sine = port_oracle.sine_table(bin_e)
         avg = np.zeros((2, n), dtype=np.int64)
         smp = np.zeros(2, dtype=np.int64)
-        emu.emu_fused_boxcar(bin_e, peak, vp(sreads), len(sreads), ds, slots, vp(segs), len(segs), vp(tw), vp(w16),
+        emu.emu_fused_boxcar(bin_e, peak, vp(sreads), len(sreads), ds, slots, vp(segs), len(segs), vp(sine), vp(win),
                              vp(avg), vp(smp))
         assert np.array_equal(avg, want), (bin_e, ds, peak)
         assert np.array_equal(smp, want_smp)
@@ -282,13 +266,12 @@ def test_stream_boxcar_kernel(emu, port_oracle, bin_e, ds, slots, grid, mode):
         reads[3, :] = 255
         want, want_smp, _ = expected(port_oracle, plan, win, reads, hops)
         sreads, _, segs = sort_by_hop(reads, hops, 2, split=2)
-        tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-        w16 = (win & 0xFFFF).astype(np.uint16)
+        sine = port_oracle.sine_table(bin_e)
         avg = np.zeros((2, n), dtype=np.int64)
         smp = np.zeros(2, dtype=np.int64)
         if mode in (1, 3):
             slots = max(4, slots & ~1)   # two boxcar groups: even ring, a slot always serves the same group
-        emu.emu_stream_boxcar(bin_e, peak, mode, vp(sreads), len(sreads), ds, slots, grid, vp(segs), len(segs), vp(tw), vp(w16),
+        emu.emu_stream_boxcar(bin_e, peak, mode, vp(sreads), len(sreads), ds, slots, grid, vp(segs), len(segs), vp(sine), vp(win),
                               vp(avg), vp(smp))
         assert np.array_equal(avg, want), (bin_e, ds, peak)
         assert np.array_equal(smp, want_smp)
@@ -310,13 +293,12 @@ def test_fifth_order_streaming_kernel(emu, port_oracle, passes, fir, span):
     reads[2, 5000:5100] = 255
     want, _, _ = expected(port_oracle, plan, win, reads, hops)
     segs = np.array([(0, 0, 3, 0)], dtype=np.int32)
-    tw = twiddles(port_oracle.sine_table(bin_e), bin_e)
-    w16 = (win & 0xFFFF).astype(np.uint16)
+    sine = port_oracle.sine_table(bin_e)
     avg = np.zeros((1, n), dtype=np.int64)
     fir5 = None
     if fir == 9:
         fir5 = np.array(list(port_oracle.lib.oracle_cic9(passes).contents)[1:6], dtype=np.int32)
     emu.emu_set_hb_span(span)
-    emu.emu_small_decim(bin_e, 0, vp(reads), 3, buf_len, ds, passes, 2, vp(fir5), vp(segs), 1, vp(tw), vp(w16),
+    emu.emu_small_decim(bin_e, 0, vp(reads), 3, buf_len, ds, passes, 2, vp(fir5), vp(segs), 1, vp(sine), vp(win),
                         vp(avg), None, None)
     assert np.array_equal(avg, want)
