@@ -86,6 +86,8 @@ static void print_usage(void)
 		"\t[-s avg|iir (default: avg; iir smooths the dB rows across reports)]\n"
 		"\t[-t workers (default: 1; hops -- or, with fewer hops than workers, sweeps -- are sharded over this many GPUs)]\n"
 		"\t[-R seed (visit the hops of every sweep in a random order)]\n"
+		"\t[-K sk_file (also write each bin's spectral kurtosis: rows like the power rows, %%.4f values,\n"
+		"\t\t~1 for noise, > 1 for intermittent signals, < 1 for steady carriers; not with -P)]\n"
 		"\tfilename (a '-' dumps samples to stdout, the default)\n");
 	exit(1);
 }
@@ -237,6 +239,45 @@ static int set_columns(rtlsdr_gpu_scan_t *gpu, const rp_plan_t *plan, int first,
 	return rc;
 }
 
+/* -K: one worker's report from rtlsdr_gpu_scan_collect_sk(): its power rows (rp_csv_row, the bytes
+ * rtlsdr_gpu_scan_collect_csv() would print) to `out`, and rows with the same prefix and the spectral
+ * kurtosis of the same columns (%.4f, nan where SK is undefined) to `skf` */
+static int write_sk_report(rtlsdr_gpu_scan_t *gpu, const rp_plan_t *plan, int first, int rows, const char *stamp,
+			   FILE *out, FILE *skf)
+{
+	const int dbc = rtlsdr_gpu_scan_db_count(gpu);
+	const size_t cap = 64 + 32 * (size_t)dbc;
+	int *smp = (int *)malloc(sizeof(int) * (size_t)rows);
+	double *db = (double *)malloc(sizeof(double) * (size_t)rows * dbc);
+	double *sk = (double *)malloc(sizeof(double) * (size_t)rows * dbc);
+	char *row = (char *)malloc(cap);
+	int rc = RTLSDR_GPU_ERR_NOMEM, i, k, low, high;
+	double step;
+	if (smp && db && sk && row)
+		rc = rtlsdr_gpu_scan_collect_sk(gpu, NULL, smp, db, NULL, sk);
+	for (i = 0; i < rows && !rc; i++) {
+		if (rp_csv_row(row, cap, plan, first + i, smp[i], db + (size_t)i * dbc, dbc) < 0) {
+			rc = RTLSDR_GPU_ERR_LENGTH;
+			break;
+		}
+		fprintf(out, "%s%s", stamp, row);
+		rp_csv_columns(plan, first + i, &low, &high, &step);
+		fprintf(skf, "%s%i, %i, %.2f, %i, ", stamp, low, high, step, smp[i]);
+		for (k = 0; k < dbc; k++) {
+			const double v = sk[(size_t)i * dbc + k];
+			if (isnan(v))
+				fputs(k + 1 < dbc ? "nan, " : "nan\n", skf);
+			else
+				fprintf(skf, k + 1 < dbc ? "%.4f, " : "%.4f\n", v);
+		}
+	}
+	free(smp);
+	free(db);
+	free(sk);
+	free(row);
+	return rc;
+}
+
 /* the device list of -t: RTLSDR_GPU_DEVICES=0,2,3 or RTLSDR_GPU_DEVICE, RTLSDR_GPU_DEVICE + 1, ... */
 static int device_list(int workers, int *devices)
 {
@@ -256,7 +297,7 @@ static int device_list(int workers, int *devices)
 
 int main(int argc, char **argv)
 {
-	const char *range = NULL, *window = "rectangle", *filename = "-";
+	const char *range = NULL, *window = "rectangle", *filename = "-", *sk_filename = NULL;
 	const char *fixed_stamp = getenv("RTL_POWER_TIMESTAMP");
 	int opt, interval = 10, single = 0, peak_hold = 0, boxcar = 1, comp_fir_size = 0;
 	int passes_per_report = env_int("RTL_POWER_PASSES", 0), passes = 0, rc = 0, hop, w;
@@ -278,11 +319,11 @@ int main(int argc, char **argv)
 	int *order;
 	char *text, stamp[80];
 	size_t text_cap = 0, text_len = 0;
-	FILE *out;
+	FILE *out, *skf = NULL;
 	struct sigaction sa;
 
 	memset(&ws, 0, sizeof(ws));
-	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POhTD:R:")) != -1) {
+	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POhTD:R:K:")) != -1) {
 		switch (opt) {
 		case 'f': range = optarg; break;
 		case 'i': interval = (int)round(rp_atoft(optarg)); break;
@@ -294,6 +335,7 @@ int main(int argc, char **argv)
 		case 'P': peak_hold = 1; break;
 		case 's': smooth_iir = strcmp("iir", optarg) == 0; break; /* avg | iir, rtl_power.c:820-825 */
 		case 't': want_workers = atoi(optarg); break;             /* rtl_power.c:844-846 */
+		case 'K': sk_filename = optarg; break;
 		case 'R': shuffle = 1; shuffle_state = 0x9E3779B97F4A7C15ULL ^ (uint64_t)strtoull(optarg, NULL, 0); break;
 		case 'd': case 'g': case 'p': case 'O': case 'T': case 'D':
 			break; /* device housekeeping: no dongle behind the synthetic source */
@@ -380,6 +422,17 @@ int main(int argc, char **argv)
 		ws.count = want_workers;
 	/* fewer hops than workers (single-hop scans): shard the sweeps, not the hops */
 	ws.by_pass = ws.count > plan->tune_count;
+	if (sk_filename && ws.by_pass) {
+		fprintf(stderr, "-K: the spectral kurtosis needs all reads of a hop on one worker (fewer hops than workers).\n");
+		return 1;
+	}
+	if (sk_filename) {
+		skf = fopen(sk_filename, "wb");
+		if (!skf) {
+			fprintf(stderr, "Failed to open %s\n", sk_filename);
+			return 1;
+		}
+	}
 	for (w = 0; w <= ws.count; w++) {
 		const int base = plan->tune_count / ws.count, extra = plan->tune_count % ws.count;
 		ws.first[w] = ws.by_pass ? (w < ws.count ? 0 : plan->tune_count) : w * base + (w < extra ? w : extra);
@@ -396,7 +449,7 @@ int main(int argc, char **argv)
 	cfg.rate = plan->rate;
 	cfg.crop = plan->crop;
 	cfg.window_coefs = window_coefs;
-	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS;
+	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS | (skf ? RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS : 0u);
 	if (smooth_iir) {
 		const char *a = getenv("RTL_POWER_IIR_ALPHA");
 		cfg.iir_alpha = (a && *a) ? atof(a) : 0.25;
@@ -480,7 +533,13 @@ int main(int argc, char **argv)
 				fprintf(stderr, "merging the workers' accumulators: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
 					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[0]));
 		}
-		for (w = 0; w < ws.count && !rc && !ws.by_pass; w++) {
+		for (w = 0; w < ws.count && !rc && !ws.by_pass && skf; w++) {
+			rc = write_sk_report(ws.gpu[w], plan, ws.first[w], ws.first[w + 1] - ws.first[w], stamp, out, skf);
+			if (rc)
+				fprintf(stderr, "rtlsdr_gpu_scan_collect_sk: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
+					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
+		}
+		for (w = 0; w < ws.count && !rc && !ws.by_pass && !skf; w++) {
 			rc = rtlsdr_gpu_scan_collect_csv(ws.gpu[w], stamp, text, text_cap, &text_len);
 			if (rc)
 				fprintf(stderr, "rtlsdr_gpu_scan_collect_csv: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
@@ -489,6 +548,8 @@ int main(int argc, char **argv)
 				fwrite(text, 1, text_len, out);
 		}
 		fflush(out);
+		if (skf)
+			fflush(skf);
 		if (rc)
 			break;
 		while (time(NULL) >= next_tick)
@@ -505,6 +566,8 @@ int main(int argc, char **argv)
 		fprintf(stderr, "\nLibrary error %d, exiting...\n", rc);
 	if (out != stdout)
 		fclose(out);
+	if (skf)
+		fclose(skf);
 	for (w = 0; w < ws.count; w++)
 		rtlsdr_gpu_scan_close(ws.gpu[w]);
 	rtlsdr_close(dev);

@@ -119,6 +119,16 @@ typedef struct rtlsdr_gpu_scan_cfg {
  * short read replaces its first len bytes, the rest is the hop's previous read.  Costs one extra host copy per
  * submit; without the flag a short len is RTLSDR_GPU_ERR_LENGTH. */
 #define RTLSDR_GPU_FLAG_SHORT_READS 4u
+/* cfg.flags: spectral kurtosis per bin (Nita & Gary 2010), which tells stationary noise (SK ~ 1) from
+ * intermittent interference (SK > 1) and steady carriers (SK < 1) in bins whose averaged power looks the same.
+ * Per hop and bin the handle also accumulates S2 = sum pw^2, pw = re^2 + im^2 being the per-block value the
+ * power bins (S1) sum, exactly as an unsigned 128-bit value; rtlsdr_gpu_scan_collect_sk() reports it with
+ *   SK = (M+1)/(M-1) * (M * S2 / S1^2 - 1),   M = samples / downsample (FFT blocks of the interval),
+ * evaluated in IEEE doubles in exactly this order without contraction (rtlsdr_b200/csrc/sk.cuh), a quiet NaN
+ * when M < 2 or S1 = 0.  Not with peak_hold, bin_e = 0 (rms) or RTLSDR_GPU_FLAG_ASYNC_REPORT
+ * (RTLSDR_GPU_ERR_CONFIG at init); on such a handle merge_device() and collect_device() return
+ * RTLSDR_GPU_ERR_CONFIG (they do not carry S2).  Every other collect also zeroes S2. */
+#define RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS 8u
 
 /* ---- lifecycle --------------------------------------------------------- */
 
@@ -210,6 +220,14 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_collect(rtlsdr_gpu_scan_t *h, int hop, int64_
 /* All hops at once: avg [tune_count << bin_e], samples [tune_count],
  * db [tune_count * db_count]; any may be NULL.  Zeroes every hop. */
 RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_all(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples, double *db);
+
+/* collect_all() plus the spectral-kurtosis report of a RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS handle (any pointer may
+ * be NULL): s2 [tune_count << bin_e][2] the raw 128-bit sums of pw^2 as (lo, hi) words in natural FFT order like
+ * `avg`, sk [tune_count * db_count] the SK row of every hop in the dB row's layout -- bin 0 takes bin 1's
+ * moments (csv_dbm's DC nuke), half swap, crop, duplicate of bin i2 -- so SK columns line up with dB columns
+ * (never smoothed by iir_alpha).  Zeroes every hop.  RTLSDR_GPU_ERR_CONFIG on a handle without the flag. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_sk(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples, double *db,
+		uint64_t *s2, double *sk);
 
 /* Same, into device buffers (for the per-interval NCCL gather); asynchronous
  * on the handle's stream, no host synchronisation. */

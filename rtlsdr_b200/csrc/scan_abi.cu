@@ -80,6 +80,8 @@ struct rtlsdr_gpu_scan {
 	int cur_acc = 0;
 	unsigned *d_done = nullptr;     /* [tune_count] epilogue tickets (fused read-and-zero) */
 	unsigned long long *d_level = nullptr; /* [tune_count][2] soft-AGC byte counts (optional) */
+	unsigned long long *d_s2 = nullptr;    /* RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS: [tune_count * N][2] sum pw^2 (lo, hi) */
+	double *d_sk = nullptr;                /* [tune_count][db_count] SK rows of collect_sk() */
 	std::vector<uint64_t> level_bytes;
 	int2 *d_tw = nullptr;
 	int2 *d_twc = nullptr;          /* small path: per-stage compact twiddles (shared-memory image); large path: round A's */
@@ -530,9 +532,34 @@ int launch_small_t(rtlsdr_gpu_scan *h, const SmallParams &prm)
 	return check_launch(h, "scan_small_kernel");
 }
 
+/* RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS: no programmatic dependent launch (an SK handle's reports end with a memset,
+ * never with the epilogue), and the u8 grid is one resident wave at the kernel's own occupancy */
+template <int L, bool IN16>
+int launch_small_sk_t(rtlsdr_gpu_scan *h, const SmallParams &prm)
+{
+	auto kern = scan_small_sk_kernel<L, IN16>;
+	const int smem = SmallSmem<L>::bytes;
+	static int per_sm[64] = { 0 };
+	int resident = h->cfg.device < 64 ? per_sm[h->cfg.device] : 0;
+	if (!resident) {
+		CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+		CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, kThreads, smem));
+		resident = std::max(resident, 1);
+		if (h->cfg.device < 64)
+			per_sm[h->cfg.device] = resident;
+	}
+	const int grid = IN16 ? std::min(prm.n_segs, h->num_sms * 8)
+			      : (int)std::min<long long>(2ll * prm.n_entries, (long long)h->num_sms * resident);
+	kern<<<grid, kThreads, smem, h->stream>>>(prm, h->d_s2);
+	h->last_was_epilogue = false;
+	return check_launch(h, "scan_small_sk_kernel");
+}
+
 template <int L>
 int launch_small_l(rtlsdr_gpu_scan *h, const SmallParams &prm, bool in16)
 {
+	if (h->d_s2)
+		return in16 ? launch_small_sk_t<L, true>(h, prm) : launch_small_sk_t<L, false>(h, prm);
 	if (h->cfg.peak_hold)
 		return in16 ? launch_small_t<L, true, true>(h, prm) : launch_small_t<L, true, false>(h, prm);
 	return in16 ? launch_small_t<L, false, true>(h, prm) : launch_small_t<L, false, false>(h, prm);
@@ -728,11 +755,12 @@ int launch_fused_boxcar(rtlsdr_gpu_scan *h, const FusedBoxcarParams &prm)
 	}
 }
 
-/* narrow boxcar scans whose every read is exactly one FFT block: one fused kernel */
+/* narrow boxcar scans whose every read is exactly one FFT block: one fused kernel (without sum |X|^4: an SK handle
+ * takes the staged boxcar and scan_small_sk_kernel) */
 bool fused_boxcar_ok(const rtlsdr_gpu_scan *h)
 {
 	const int ds = h->cfg.downsample;
-	return h->cfg.boxcar && ds >= 2 && ds <= 64 && h->cfg.bin_e >= 8 && h->cfg.bin_e <= 12 && h->shape.n_blocks == 1 &&
+	return !h->d_s2 && h->cfg.boxcar && ds >= 2 && ds <= 64 && h->cfg.bin_e >= 8 && h->cfg.bin_e <= 12 && h->shape.n_blocks == 1 &&
 	       h->cfg.buf_len == 2 * h->shape.N * ds && !h->dbg_no_fused_boxcar;
 }
 
@@ -1230,6 +1258,8 @@ void free_all(rtlsdr_gpu_scan *h)
 			cudaEventDestroy(h->ev_report[i]);
 	cudaFree(h->d_tw);
 	cudaFree(h->d_level);
+	cudaFree(h->d_s2);
+	cudaFree(h->d_sk);
 	cudaFree(h->d_done);
 	cudaFree(h->d_twb);
 	cudaFree(h->d_twc);
@@ -1531,6 +1561,11 @@ int rtlsdr_gpu_scan_init(const rtlsdr_gpu_scan_cfg_t *cfg_in, rtlsdr_gpu_scan_t 
 		const size_t iir_bytes = (size_t)cfg->tune_count * (size_t)(h->shape.db_count - 1) * sizeof(double);
 		if (cfg->iir_alpha > 0.0 && !alloc_fill(&h->d_iir, iir_bytes, 0xFF, h->stream, &rc))
 			break;
+		if (cfg->flags & RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS) {
+			if (!alloc_fill(&h->d_s2, (size_t)cfg->tune_count * N * 2 * sizeof(unsigned long long), 0, h->stream, &rc) ||
+			    !alloc_fill(&h->d_sk, (size_t)cfg->tune_count * h->shape.db_count * sizeof(double), 0, h->stream, &rc))
+				break;
+		}
 		if (cfg->flags & RTLSDR_GPU_FLAG_LEVEL_STATS) {
 			if (!alloc_fill(&h->d_level, (size_t)cfg->tune_count * 2 * sizeof(unsigned long long), 0, h->stream, &rc))
 				break;
@@ -1969,6 +2004,8 @@ static int collect_range(rtlsdr_gpu_scan_t *h, int hop0, int nhops, int64_t *avg
 	}
 	if (h->d_level)
 		CU(cudaMemsetAsync(h->d_level + 2 * (size_t)hop0, 0, (size_t)nhops * 2 * sizeof(unsigned long long), h->stream));
+	if (h->d_s2)
+		CU(cudaMemsetAsync(h->d_s2 + 2 * (size_t)hop0 * N, 0, (size_t)nhops * N * 2 * sizeof(unsigned long long), h->stream));
 	CU(cudaStreamSynchronize(h->stream));
 	for (int i = 0; i < nhops; i++) {
 		if (samples)
@@ -1998,10 +2035,52 @@ int rtlsdr_gpu_scan_collect_all(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples
 	return collect_range(h, 0, h->cfg.tune_count, avg, samples, db);
 }
 
+int rtlsdr_gpu_scan_collect_sk(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples, double *db, uint64_t *s2, double *sk)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc = flush_ring(h);
+	if (rc)
+		return rc;
+	const int tc = h->cfg.tune_count, dbc = h->shape.db_count;
+	const size_t N = (size_t)h->shape.N;
+	h->last_was_epilogue = false;
+	if (sk) {
+		/* reads S1 and the sample counters: on the handle's stream in front of collect_range()'s epilogue and
+		 * read-and-zero memsets */
+		SkReportParams p;
+		p.avg = h->d_avg;
+		p.samples = h->d_smp64;
+		p.s2 = h->d_s2;
+		p.sk = h->d_sk;
+		p.bin_e = h->cfg.bin_e;
+		p.i1 = h->shape.db_i1;
+		p.i2 = h->shape.db_i2;
+		p.downsample = h->cfg.downsample;
+		p.hop0 = 0;
+		sk_report_kernel<<<dim3((dbc + 255) / 256, tc), 256, 0, h->stream>>>(p);
+		if ((rc = check_launch(h, "sk_report_kernel")))
+			return rc;
+		CU(cudaMemcpyAsync(sk, h->d_sk, (size_t)tc * dbc * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+		h->d2h += (uint64_t)tc * dbc * sizeof(double);
+	}
+	if (s2) {
+		CU(cudaMemcpyAsync(s2, h->d_s2, (size_t)tc * N * 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+		h->d2h += (uint64_t)tc * N * 2 * sizeof(uint64_t);
+	}
+	/* dB rows, raw copies, and the read-and-zero of S1, the counters and S2 */
+	return collect_range(h, 0, tc, avg, samples, db);
+}
+
 int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples, void *dev_db)
 {
 	if (!h)
 		return RTLSDR_GPU_ERR_NULL;
+	if (h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG; /* the device report carries no S2 */
 	CU(cudaSetDevice(h->cfg.device));
 	int rc = flush_ring(h);
 	if (rc)
@@ -2135,6 +2214,8 @@ int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *t
 	CU(cudaMemsetAsync(h->d_avg, 0, ((size_t)tc * h->shape.N + (size_t)tc) * sizeof(long long), h->stream));
 	if (h->d_level)
 		CU(cudaMemsetAsync(h->d_level, 0, (size_t)tc * 2 * sizeof(unsigned long long), h->stream));
+	if (h->d_s2)
+		CU(cudaMemsetAsync(h->d_s2, 0, (size_t)tc * h->shape.N * 2 * sizeof(unsigned long long), h->stream));
 	CU(cudaStreamSynchronize(h->stream));
 	std::fill(h->samples.begin(), h->samples.end(), 0);
 	if (h->d_level)
@@ -2173,6 +2254,8 @@ int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, cons
 		return RTLSDR_GPU_ERR_CONFIG;
 	if (((uintptr_t)dev_avg & 7) || ((uintptr_t)dev_samples & 3) || (set_stride & 7))
 		return RTLSDR_GPU_ERR_ALIGN;
+	if (h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG; /* the external sets carry no S2 */
 	CU(cudaSetDevice(h->cfg.device));
 	int rc = flush_ring(h);
 	if (rc)

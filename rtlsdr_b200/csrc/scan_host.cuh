@@ -29,6 +29,10 @@ inline int scan_shape(const rtlsdr_gpu_scan_cfg_t &cfg, ScanShape *out)
 	    cfg.downsample_passes < 0 || cfg.downsample_passes > 20 || cfg.buf_len < 16 ||
 	    (cfg.buf_len & 15) || cfg.rate <= 0 || !(cfg.crop >= 0.0 && cfg.crop <= 1.0))
 		return RTLSDR_GPU_ERR_CONFIG;
+	/* spectral kurtosis needs sums (not maxima) of FFT powers, and its report is synchronous */
+	if ((cfg.flags & RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS) &&
+	    (cfg.peak_hold || cfg.bin_e == 0 || (cfg.flags & RTLSDR_GPU_FLAG_ASYNC_REPORT)))
+		return RTLSDR_GPU_ERR_CONFIG;
 	const int N = 1 << cfg.bin_e;
 	const bool box = cfg.boxcar && cfg.downsample > 1;
 	const bool hb = !box && cfg.downsample_passes > 0;

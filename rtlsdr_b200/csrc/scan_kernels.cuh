@@ -31,6 +31,7 @@
  */
 #pragma once
 #include "scan_compat.cuh"
+#include "sk.cuh"
 
 /* Micro-variants of the transform kernel, all measured on B200 (profiles/r02d_small_kernel_ab.txt, config 5):
  * window coefficients in registers +0.4 %, IDP.4A front end +0.8 %, packed "b" operands after a transpose +0.5 %,
@@ -593,6 +594,54 @@ SCAN_DEV void flush_bins(unsigned long long (&acc)[kPts], long long *out, unsign
 	}
 }
 
+/* ---- spectral kurtosis: sum |X|^4 beside the power sums (sk.cuh) ----------- */
+
+SCAN_DEV void sk_zero(unsigned long long (&lo)[kPts], unsigned (&hi)[kPts])
+{
+#pragma unroll
+	for (int r = 0; r < kPts; ++r) {
+		lo[r] = 0ull;
+		hi[r] = 0u;
+	}
+}
+
+/* accumulate_power<false> plus pw^2 into the 128-bit partial (lo, hi) */
+SCAN_DEV void accumulate_power_sk(unsigned long long &acc, unsigned long long &lo, unsigned &hi, int re, int im)
+{
+	const unsigned pw = (unsigned)(re * re) + (unsigned)(im * im);
+	acc += pw;
+	sk_accumulate(lo, hi, pw);
+}
+
+/* flush_bins<L, false> for the S2 partials: out = the hop's [N][2] words; `bins` = 2N x u64 of idle shared memory */
+template <int L>
+SCAN_DEV void flush_s2(const unsigned long long (&lo)[kPts], const unsigned (&hi)[kPts], unsigned long long *out,
+		       unsigned long long *bins, int t)
+{
+	constexpr int N = 1 << L;
+	if constexpr (L == 12) {
+#pragma unroll
+		for (int r = 0; r < kPts; ++r) {
+			const int bin = last_pos<L>(t, r) & (N - 1);
+			sk_atomic_add(out + 2 * bin, lo[r], hi[r]);
+		}
+	} else {
+		__syncthreads();
+		for (int i = t; i < 2 * N; i += kThreads)
+			bins[i] = 0ull;
+		__syncthreads();
+#pragma unroll
+		for (int r = 0; r < kPts; ++r) {
+			const int bin = last_pos<L>(t, r) & (N - 1);
+			sk_atomic_add(bins + 2 * bin, lo[r], hi[r]);
+		}
+		__syncthreads();
+		for (int i = t; i < N; i += kThreads)
+			sk_atomic_add(out + 2 * i, bins[2 * i], bins[2 * i + 1]);
+		__syncthreads();
+	}
+}
+
 /*
  * u8 reads (IN16 = false): the launch's hop-sorted reads are cut into gridDim.x contiguous runs of equal
  * length, counted in 4096-sample working sets (half reads), so every CTA does the same amount of work whatever
@@ -605,230 +654,23 @@ template <int L, bool PEAK, bool IN16>
 __global__ void __launch_bounds__(kThreads, 2)
 scan_small_kernel(const SCAN_GRID_CONSTANT SmallParams prm)
 {
-	SCAN_DYN_SMEM(smem);
-	typedef SmallSmem<L> SM;
-	constexpr int N = 1 << L;
-	uint8_t *stage = smem + SM::off_stage;
-	c16 *xch = (c16 *)(smem + SM::off_xch);
-	int2 *tws = (int2 *)(smem + SM::off_tw);
-	uint16_t *wins = (uint16_t *)(smem + SM::off_win);
-	int *red = (int *)(smem + SM::off_red); /* [8 warps][2] */
+	constexpr bool SK = false;
+	[[maybe_unused]] unsigned long long *const s2 = nullptr;
+#include "scan_small_body.inl"
+}
 
-	const int t = threadIdx.x;
-	load_tables<L>(tws, wins, prm.twc, prm.win, t, kThreads); /* overlapped with the first read's prefetch */
-
-	TwSmall<L> tw;
-	tw.tws = tws;
-	tw.tw0 = &prm.tw0;
-
-	/* sample index (inside its FFT block) that feeds position (16t + r), minus
-	 * the r-dependent part: n = blkbase + (brev4(r) << (L-4)) + trev   (L >= 4) */
-	int blkbase = 0, t0;
-	const int trev = front_thread_map<L>(t, t0);
-	if constexpr (L >= 4)
-		blkbase = (t >> (L - 4)) << L;
-
-	int flip = 0;
-
-	if constexpr (!IN16) {
-		/* runs are cut at half reads only when a CTA has several reads to amortise the read it shares with
-		 * its neighbour (both stage it and sum its DC term); short launches are cut at whole reads */
-		const long long total_ws = 2ll * prm.n_entries;
-		long long ws_lo, ws_hi;
-		if (total_ws >= 8ll * gridDim.x) {
-			ws_lo = total_ws * blockIdx.x / gridDim.x;
-			ws_hi = total_ws * (blockIdx.x + 1) / gridDim.x;
-		} else {
-			ws_lo = 2 * ((long long)prm.n_entries * blockIdx.x / gridDim.x);
-			ws_hi = 2 * ((long long)prm.n_entries * (blockIdx.x + 1) / gridDim.x);
-		}
-		if (ws_lo >= ws_hi)
-			return;
-#ifndef SCAN_EMU
-		/* The two CTAs of an SM start in lockstep (same phase of every working set: both in the front end, both at
-		 * a barrier ...) and only drift into complementary phases after many working sets; delaying the second
-		 * half of the grid (CTA b and b + gridDim/2 share an SM under round-robin placement) by about half a
-		 * working set de-phases them from the start.  Only worth it for short launches. */
-		if (prm.stagger_ns > 0 && blockIdx.x >= gridDim.x / 2)
-			__nanosleep((unsigned)prm.stagger_ns);
-#endif
-		const int e_lo = (int)(ws_lo >> 1), e_hi = (int)((ws_hi + 1) >> 1); /* reads [e_lo, e_hi) are touched */
-
-		unsigned long long acc[kPts];
-#pragma unroll
-		for (int r = 0; r < kPts; ++r)
-			acc[r] = 0ull;
-		int hop = prm.hop_of[e_lo], hop_ws = 0;
-		bool waited = false;
-
-		{
-			const uint8_t *src = prm.base + prm.read_off[e_lo];
-#pragma unroll
-			for (int i = 0; i < kStageBytes / (kThreads * 16); ++i)
-				cp_async16(stage + (i * kThreads + t) * 16, src + (i * kThreads + t) * 16);
-			cp_async_commit();
-		}
-		constexpr bool kWinRegsOn = RSCAN_WIN_REGS && L == 12;
-		unsigned wreg[kWinRegs];
-		if constexpr (kWinRegsOn) {
-			cp_async_wait_all(); /* the tables have landed too (same thread's copies are not enough: barrier) */
-			__syncthreads();
-			load_window_regs<L>(wreg, wins, t, trev, blkbase);
-		}
-		for (int e = e_lo; e < e_hi; ++e) {
-			const int u = e - e_lo;
-			cp_async_wait_all();
-			__syncthreads(); /* slot u&1 landed; slot (u+1)&1 no longer read */
-			int next_hop = -1;
-			if (e + 1 < e_hi) {
-				const uint8_t *src = prm.base + prm.read_off[e + 1];
-				uint8_t *dst = stage + ((u + 1) & 1) * kStageBytes;
-#pragma unroll
-				for (int i = 0; i < kStageBytes / (kThreads * 16); ++i)
-					cp_async16(dst + (i * kThreads + t) * 16, src + (i * kThreads + t) * 16);
-				cp_async_commit();
-				next_hop = prm.hop_of[e + 1];
-			}
-			const uint8_t *st = stage + (u & 1) * kStageBytes;
-			int kI, kQ;
-			u8_read_dc(st, red, t, kI, kQ);
-
-			/* this CTA's working sets of the read: both, except at the two ends of its run */
-			const int ws0 = (2ll * e < ws_lo) ? 1 : 0, ws1 = (2ll * e + 2 > ws_hi) ? 1 : 2;
-#pragma unroll 1
-			for (int ws = ws0; ws < ws1; ++ws) {
-				X2 x[kPts];
-				front_u8<L, kWinRegsOn>(x, st, ws, kI, kQ, wins, t, trev, blkbase, wreg);
-				engine_fft_db<L>(x, xch, flip, t, tw, BlockBar(), t0);
-				/* ---- |X|^2 (rtl_power.c:636-640, 708-716) ---- */
-#pragma unroll
-				for (int r = 0; r < kPts; ++r)
-					accumulate_power<PEAK>(acc[r], x[r].re >> 16, x[r].im >> 16);
-			}
-			hop_ws += ws1 - ws0;
-
-			if (next_hop != hop) {
-				/* everything above only read this launch's inputs; the accumulators may still be in use
-				 * by the report epilogue of the previous interval (programmatic dependent launch) */
-				if (!waited)
-					pdl_wait();
-				waited = true;
-				if (t == 0) /* tunes[hop].samples += ds per FFT block (rtl_power.c:717) */
-					atomicAdd((unsigned long long *)(prm.samples + hop),
-						  (unsigned long long)((long long)hop_ws * (prm.samples_per_read / 2)));
-				/* N < 4096: the transpose buffers are idle here and serve as the shared bin array */
-				flush_bins<L, PEAK>(acc, prm.avg + ((long long)hop << L), (unsigned long long *)xch, t);
-#pragma unroll
-				for (int r = 0; r < kPts; ++r)
-					acc[r] = 0ull;
-				hop = next_hop;
-				hop_ws = 0;
-			}
-		}
-	} else {
-	for (int seg = blockIdx.x; seg < prm.n_segs; seg += gridDim.x) {
-		const int4 sg = prm.segs[seg];
-		const int hop = sg.x, first = sg.y;
-		/* the segment's images form one contiguous run of blocks, cut into 4096-sample units */
-		const int seg_blocks = sg.z * prm.blocks_padded;
-		const int units = (int)(((long long)seg_blocks * N + kWS - 1) / kWS);
-
-		unsigned long long acc[kPts];
-#pragma unroll
-		for (int r = 0; r < kPts; ++r)
-			acc[r] = 0ull;
-
-		/* prefetch unit 0 */
-		{
-			const uint8_t *src = prm.base + entry_offset(prm, first);
-#pragma unroll
-			for (int i = 0; i < kStageBytes / (kThreads * 16); ++i)
-				cp_async16(stage + (i * kThreads + t) * 16, src + (i * kThreads + t) * 16);
-			cp_async_commit();
-		}
-
-		for (int u = 0; u < units; ++u) {
-			cp_async_wait_all();
-			__syncthreads(); /* slot u&1 landed; slot (u+1)&1 no longer read */
-			if (u + 1 < units) {
-				const uint8_t *src = prm.base + entry_offset(prm, first) + (long long)(u + 1) * kStageBytes;
-				uint8_t *dst = stage + ((u + 1) & 1) * kStageBytes;
-#pragma unroll
-				for (int i = 0; i < kStageBytes / (kThreads * 16); ++i)
-					cp_async16(dst + (i * kThreads + t) * 16, src + (i * kThreads + t) * 16);
-				cp_async_commit();
-			}
-			const uint8_t *st = stage + (u & 1) * kStageBytes;
-
-			/* ---- DC term of the whole read (rtl_power.c:692-693) ---- */
-			int limI = kWS, limQ = kWS, kI, kQ;
-			/* working-set block b is block gb = u * (4096/N) + b of the segment */
-			if constexpr (L >= 4) {
-				const int gb = u * (kWS / N) + (t >> (L - 4));
-				const int rd = gb / prm.blocks_padded, bir = gb - rd * prm.blocks_padded;
-				const bool live = gb < seg_blocks && bir < prm.n_blocks;
-				const int e = first + (live ? rd : 0) - prm.entry_base;
-				kI = __ldg(prm.dc_ave + 2 * e);
-				kQ = __ldg(prm.dc_ave + 2 * e + 1);
-				/* remove_dc covers int16 indices < l_len of the read (rtl_power.c:692-693) */
-				limI = live ? ((prm.l_len + 1) >> 1) - bir * N : 0;
-				limQ = live ? (prm.l_len >> 1) - bir * N : 0;
-			} else {
-				kI = kQ = 0; /* per element below */
-			}
-
-			X2 x[kPts];
-			/* ---- remove DC, window, bit-reversed placement ---- */
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				int nblk, n; /* sample index inside its block / inside the working set */
-				front_index<L>(r, t, trev, blkbase, nblk, n);
-				const int wv = wins[nblk];
-				const c16 raw = ((const c16 *)st)[n];
-				int re = c16_re(raw), im = c16_im(raw);
-				if constexpr (L >= 4) {
-					if (nblk < limI)
-						re -= kI;
-					if (nblk < limQ)
-						im -= kQ;
-				} else {
-					/* several blocks per thread: look the read up per element */
-					const int gb = u * (kWS / N) + (n >> L);
-					const int rd = gb / prm.blocks_padded, bir = gb - rd * prm.blocks_padded;
-					if (gb < seg_blocks && bir < prm.n_blocks) {
-						const int e = first + rd - prm.entry_base;
-						const int k = bir * N + nblk;
-						if (2 * k < prm.l_len)
-							re -= __ldg(prm.dc_ave + 2 * e);
-						if (2 * k + 1 < prm.l_len)
-							im -= __ldg(prm.dc_ave + 2 * e + 1);
-					}
-				}
-				x[r].re = (re * wv) << 16;
-				x[r].im = (im * wv) << 16;
-			}
-
-			engine_fft_db<L>(x, xch, flip, t, tw, BlockBar(), t0);
-
-			/* ---- |X|^2 (rtl_power.c:636-640, 708-716) ---- */
-#pragma unroll
-			for (int r = 0; r < kPts; ++r) {
-				const int gb = u * (kWS / N) + (last_pos<L>(t, r) >> L);
-				bool ok = gb < seg_blocks;
-				if (prm.blocks_padded != prm.n_blocks)
-					ok = ok && (gb % prm.blocks_padded) < prm.n_blocks;
-				if (ok)
-					accumulate_power<PEAK>(acc[r], x[r].re >> 16, x[r].im >> 16);
-			}
-		}
-
-		pdl_wait();
-		if (t == 0)
-			atomicAdd((unsigned long long *)(prm.samples + hop), (unsigned long long)((long long)sg.z * prm.samples_per_read));
-		/* ---- flush this segment's sums (the staging area is idle: no prefetch is pending) ---- */
-		flush_bins<L, PEAK>(acc, prm.avg + ((long long)hop << L), (unsigned long long *)stage, t);
-	}
-	}
+/*
+ * RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS: the same kernel with sum |X|^4 (sk.cuh) accumulated beside the power sums, into
+ * s2 [tune_count << L][2] (lo, hi).  The 128-bit register partials take 48 more registers than scan_small_kernel's
+ * 2-CTA budget of 128 allows, so this variant is compiled for one CTA per SM (no spills) instead of a shared-memory
+ * S2 image: at N = 4096 the 48 KiB image would not leave room for a second CTA either.
+ */
+template <int L, bool IN16>
+__global__ void __launch_bounds__(kThreads, 1)
+scan_small_sk_kernel(const SCAN_GRID_CONSTANT SmallParams prm, unsigned long long *s2)
+{
+	constexpr bool SK = true, PEAK = false;
+#include "scan_small_body.inl"
 }
 
 /* ======================================================================== *

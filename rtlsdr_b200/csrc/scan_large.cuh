@@ -285,53 +285,20 @@ template <int LB, bool LAST, bool PEAK>
 __global__ void __launch_bounds__(kThreads, 2) /* (3 CTAs per SM at 80 registers: measured 103 vs 105 G samples/s) */
 large_round_b_kernel(const SCAN_GRID_CONSTANT LargeParams prm)
 {
-	SCAN_DYN_SMEM(smem);
-	c16 *stage = (c16 *)smem;
-	constexpr int ncols = kWS >> LB;
-	constexpr int tiles_per_u = 256 / ncols;
-	const int t = threadIdx.x, L = prm.L;
-	const int rel = blockIdx.y;
-	const long long N = 1ll << L;
-	const int U = blockIdx.x / tiles_per_u, plow0 = (blockIdx.x % tiles_per_u) * ncols;
-	c16 *data = prm.scratch + (long long)rel * N + ((long long)U << (8 + LB)) + plow0;
+	constexpr bool SK = false;
+	[[maybe_unused]] unsigned long long *const s2 = nullptr;
+#include "large_round_b_body.inl"
+}
 
-#pragma unroll
-	for (int k = 0; k < kPts; ++k) {
-		const int eidx = t + kThreads * k;
-		const int col = eidx % ncols, i = eidx / ncols;
-		stage[tile_idx((col << LB) | i)] = data[((long long)i << 8) + col];
-	}
-	__syncthreads();
-	X2 x[kPts];
-#pragma unroll
-	for (int r = 0; r < kPts; ++r)
-		x[r] = x_unpack(stage[tile_idx(pos<0>(t, r))]);
-
-	TwLargeB<LB> tw;
-	tw.tw = prm.tw;
-	tw.twb = prm.twb;
-	tw.plow0 = plow0;
-	tw.L = L;
-	engine_fft<LB>(x, stage, t, tw);
-
-	__syncthreads();
-#pragma unroll
-	for (int r = 0; r < kPts; ++r)
-		stage[tile_idx(last_pos<LB>(t, r))] = x_pack(x[r]);
-	__syncthreads();
-	long long *out = nullptr;
-	if constexpr (LAST)
-		out = prm.avg + ((long long)prm.hop_of[prm.entry_base + rel] << L) + plow0;
-#pragma unroll
-	for (int k = 0; k < kPts; ++k) {
-		const int eidx = t + kThreads * k;
-		const int col = eidx % ncols, i = eidx / ncols;
-		const c16 x = stage[tile_idx((col << LB) | i)];
-		if constexpr (LAST)
-			accumulate_bin(out + ((long long)i << 8) + col, x, PEAK);
-		else
-			data[((long long)i << 8) + col] = x;
-	}
+/* RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS, N <= 2^16: the last round B with pw^2 added to s2 [tune_count << L][2] beside
+ * each |X|^2 (sk.cuh) */
+template <int LB>
+__global__ void __launch_bounds__(kThreads, 2)
+large_round_b_sk_kernel(const SCAN_GRID_CONSTANT LargeParams prm, unsigned long long *s2)
+{
+	constexpr bool SK = true, LAST = true;
+	[[maybe_unused]] constexpr bool PEAK = false;
+#include "large_round_b_body.inl"
 }
 
 /*
@@ -504,101 +471,19 @@ template <int LC, bool PEAK, int VEC>
 __global__ void __launch_bounds__(kThreads)
 large_round_c_kernel(const SCAN_GRID_CONSTANT LargeParams prm)
 {
-	constexpr int R = 1 << LC;
-	constexpr bool kHoist = LC <= 3; /* twiddles depend on the position only: keep them in registers */
-	const int L = prm.L;
-	const int plow = (blockIdx.x * kThreads + threadIdx.x) * VEC; /* 0 .. 65535 */
-	const long long N = 1ll << L;
-	int2 wreg[kHoist ? (R - 1) * VEC : 1];
-	if constexpr (kHoist) {
-#pragma unroll
-		for (int se = 0; se < LC; ++se)
-#pragma unroll
-			for (int g = 0; g < (1 << se); ++g)
-#pragma unroll
-				for (int j = 0; j < VEC; ++j) {
-					const long long m = ((long long)g << 16) | (plow + j);
-					wreg[((1 << se) - 1 + g) * VEC + j] = __ldg(prm.tw + (m << (L - 17 - se)));
-				}
-	}
-	unsigned long long acc[R * VEC];
-#pragma unroll
-	for (int r = 0; r < R * VEC; ++r)
-		acc[r] = 0ull;
-	int cur_hop = -1;
-	pdl_wait(); /* the twiddles above did not depend on round B */
-	const int rel0 = blockIdx.y * prm.c_reads;
-	const int rel1 = (rel0 + prm.c_reads < prm.n_entries) ? rel0 + prm.c_reads : prm.n_entries;
-	c16 nxt[R * VEC];
-	auto fetch = [&](int rel) {
-		const c16 *data = prm.scratch + (long long)rel * N + plow;
-#pragma unroll
-		for (int r = 0; r < R; ++r) {
-			if constexpr (VEC == 4) {
-				const uint4 q = *(const uint4 *)(data + ((long long)r << 16));
-				nxt[4 * r] = q.x, nxt[4 * r + 1] = q.y, nxt[4 * r + 2] = q.z, nxt[4 * r + 3] = q.w;
-			} else if constexpr (VEC == 2) {
-				const uint2 q = *(const uint2 *)(data + ((long long)r << 16));
-				nxt[2 * r] = q.x, nxt[2 * r + 1] = q.y;
-			} else {
-				nxt[r] = data[(long long)r << 16];
-			}
-		}
-	};
-	if (rel0 < rel1)
-		fetch(rel0);
-	for (int rel = rel0; rel <= rel1; ++rel) {
-		const int hop = (rel < rel1) ? prm.hop_of[prm.entry_base + rel] : -1;
-		if (hop != cur_hop) {
-			if (cur_hop >= 0) {
-				long long *out = prm.avg + ((long long)cur_hop << L) + plow;
-#pragma unroll
-				for (int r = 0; r < R; ++r)
-#pragma unroll
-					for (int j = 0; j < VEC; ++j) {
-						if (PEAK)
-							atomicMax(out + ((long long)r << 16) + j, (long long)acc[r * VEC + j]);
-						else
-							atomicAdd((unsigned long long *)(out + ((long long)r << 16) + j), acc[r * VEC + j]);
-						acc[r * VEC + j] = 0ull;
-					}
-			}
-			cur_hop = hop;
-		}
-		if (rel == rel1)
-			break;
-		c16 v[R * VEC];
-#pragma unroll
-		for (int r = 0; r < R * VEC; ++r)
-			v[r] = nxt[r];
-		if (rel + 1 < rel1)
-			fetch(rel + 1);
-#pragma unroll
-		for (int se = 0; se < LC; ++se) {
-#pragma unroll
-			for (int r = 0; r < R; ++r) {
-				if ((r & (1 << se)) == 0) {
-					const int g = r & ((1 << se) - 1);
-#pragma unroll
-					for (int j = 0; j < VEC; ++j) {
-						int2 w;
-						if constexpr (kHoist) {
-							w = wreg[((1 << se) - 1 + g) * VEC + j];
-						} else {
-							const long long m = ((long long)g << 16) | (plow + j);
-							w = __ldg(prm.tw + (m << (L - 17 - se)));
-						}
-						butterfly(v[r * VEC + j], v[(r | (1 << se)) * VEC + j], w.x, w.y);
-					}
-				}
-			}
-		}
-#pragma unroll
-		for (int r = 0; r < R * VEC; ++r) {
-			const int re = c16_re(v[r]), im = c16_im(v[r]);
-			accumulate_power<PEAK>(acc[r], re, im);
-		}
-	}
+	constexpr bool SK = false;
+	[[maybe_unused]] unsigned long long *const s2 = nullptr;
+#include "large_round_c_body.inl"
+}
+
+/* RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS, N >= 2^17: round C with 128-bit sum |X|^4 register partials beside the power
+ * sums, flushed into s2 [tune_count << L][2] at the same hop changes */
+template <int LC, int VEC>
+__global__ void __launch_bounds__(kThreads)
+large_round_c_sk_kernel(const SCAN_GRID_CONSTANT LargeParams prm, unsigned long long *s2)
+{
+	constexpr bool SK = true, PEAK = false;
+#include "large_round_c_body.inl"
 }
 
 /* positions per thread of round C for 2^LC strided points: 16-byte loads while the accumulators fit */

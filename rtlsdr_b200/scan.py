@@ -56,6 +56,7 @@ def load_library():
     L.rtlsdr_gpu_scan_collect.argtypes = [vp, i, vp, vp, vp]
     L.rtlsdr_gpu_scan_collect_all.argtypes = [vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_collect_device.argtypes = [vp, vp, vp, vp]
+    L.rtlsdr_gpu_scan_collect_sk.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_merge_device.argtypes = [vp, vp, vp, i, i64]
     L.rtlsdr_gpu_scan_set_csv_columns.argtypes = [vp, i, vp, vp, ctypes.c_double]
     L.rtlsdr_gpu_scan_csv_capacity.argtypes = [vp, i, ctypes.c_size_t]
@@ -159,7 +160,7 @@ class GpuScan:
     def __init__(self, tune_count, bin_e, buf_len, downsample=1, downsample_passes=0, boxcar=1,
                  comp_fir_size=0, peak_hold=0, rate=2400000, crop=0.0, window_coefs=None,
                  sinewave=None, device=0, ring_bytes=0, level_stats=False, iir_alpha=0.0, async_report=False,
-                 short_reads=False):
+                 short_reads=False, spectral_kurtosis=False):
         self.lib = load_library()
         self.tune_count, self.bin_e, self.buf_len = tune_count, bin_e, buf_len
         self.n = 1 << bin_e
@@ -179,8 +180,9 @@ class GpuScan:
             self._s = np.ascontiguousarray(sinewave, dtype=np.int16)
             cfg.sinewave = self._s.ctypes.data
         cfg.ring_bytes = ring_bytes
-        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS
-        cfg.flags = (1 if level_stats else 0) | (2 if async_report else 0) | (4 if short_reads else 0)
+        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS / _SPECTRAL_KURTOSIS
+        cfg.flags = ((1 if level_stats else 0) | (2 if async_report else 0) | (4 if short_reads else 0)
+                     | (8 if spectral_kurtosis else 0))
         cfg.iir_alpha = iir_alpha            # -s iir smoothing of the dB rows across reports (0 = off)
         self.h = ctypes.c_void_p()
         rc = self.lib.rtlsdr_gpu_scan_init(ctypes.byref(cfg), ctypes.byref(self.h))
@@ -248,6 +250,19 @@ class GpuScan:
         self._check(self.lib.rtlsdr_gpu_scan_collect_all(self.h, avg.ctypes.data, smp.ctypes.data,
                                                          db.ctypes.data if db is not None else None), "collect_all")
         return avg, smp, db
+
+    def collect_sk(self):
+        """collect_all() plus the spectral-kurtosis report (spectral_kurtosis=True handles):
+        (avg int64 [tc, N], samples int32 [tc], db float64 [tc, db_count],
+         s2 uint64 [tc, N, 2] the 128-bit sums of |X|^4 as (lo, hi), sk float64 [tc, db_count] in the dB row's layout)"""
+        avg = np.zeros((self.tune_count, self.n), dtype=np.int64)
+        smp = np.zeros(self.tune_count, dtype=np.int32)
+        db = np.zeros((self.tune_count, self.db_count), dtype=np.float64)
+        s2 = np.zeros((self.tune_count, self.n, 2), dtype=np.uint64)
+        sk = np.zeros((self.tune_count, self.db_count), dtype=np.float64)
+        self._check(self.lib.rtlsdr_gpu_scan_collect_sk(self.h, avg.ctypes.data, smp.ctypes.data, db.ctypes.data,
+                                                        s2.ctypes.data, sk.ctypes.data), "collect_sk")
+        return avg, smp, db, s2, sk
 
     def collect_device(self, dev_avg=None, dev_samples=None, dev_db=None):
         self._check(self.lib.rtlsdr_gpu_scan_collect_device(self.h, dev_avg, dev_samples, dev_db), "collect_device")
