@@ -239,45 +239,6 @@ static int set_columns(rtlsdr_gpu_scan_t *gpu, const rp_plan_t *plan, int first,
 	return rc;
 }
 
-/* -K: one worker's report from rtlsdr_gpu_scan_collect_sk(): its power rows (rp_csv_row, the bytes
- * rtlsdr_gpu_scan_collect_csv() would print) to `out`, and rows with the same prefix and the spectral
- * kurtosis of the same columns (%.4f, nan where SK is undefined) to `skf` */
-static int write_sk_report(rtlsdr_gpu_scan_t *gpu, const rp_plan_t *plan, int first, int rows, const char *stamp,
-			   FILE *out, FILE *skf)
-{
-	const int dbc = rtlsdr_gpu_scan_db_count(gpu);
-	const size_t cap = 64 + 32 * (size_t)dbc;
-	int *smp = (int *)malloc(sizeof(int) * (size_t)rows);
-	double *db = (double *)malloc(sizeof(double) * (size_t)rows * dbc);
-	double *sk = (double *)malloc(sizeof(double) * (size_t)rows * dbc);
-	char *row = (char *)malloc(cap);
-	int rc = RTLSDR_GPU_ERR_NOMEM, i, k, low, high;
-	double step;
-	if (smp && db && sk && row)
-		rc = rtlsdr_gpu_scan_collect_sk(gpu, NULL, smp, db, NULL, sk);
-	for (i = 0; i < rows && !rc; i++) {
-		if (rp_csv_row(row, cap, plan, first + i, smp[i], db + (size_t)i * dbc, dbc) < 0) {
-			rc = RTLSDR_GPU_ERR_LENGTH;
-			break;
-		}
-		fprintf(out, "%s%s", stamp, row);
-		rp_csv_columns(plan, first + i, &low, &high, &step);
-		fprintf(skf, "%s%i, %i, %.2f, %i, ", stamp, low, high, step, smp[i]);
-		for (k = 0; k < dbc; k++) {
-			const double v = sk[(size_t)i * dbc + k];
-			if (isnan(v))
-				fputs(k + 1 < dbc ? "nan, " : "nan\n", skf);
-			else
-				fprintf(skf, k + 1 < dbc ? "%.4f, " : "%.4f\n", v);
-		}
-	}
-	free(smp);
-	free(db);
-	free(sk);
-	free(row);
-	return rc;
-}
-
 /* the device list of -t: RTLSDR_GPU_DEVICES=0,2,3 or RTLSDR_GPU_DEVICE, RTLSDR_GPU_DEVICE + 1, ... */
 static int device_list(int workers, int *devices)
 {
@@ -317,8 +278,8 @@ int main(int argc, char **argv)
 	int32_t *window_coefs = NULL;
 	uint8_t *buf8, *replay = NULL;
 	int *order;
-	char *text, stamp[80];
-	size_t text_cap = 0, text_len = 0;
+	char *text, *sk_text = NULL, stamp[80];
+	size_t text_cap = 0, text_len = 0, sk_cap = 0, sk_len = 0;
 	FILE *out, *skf = NULL;
 	struct sigaction sa;
 
@@ -467,6 +428,8 @@ int main(int argc, char **argv)
 		/* text buffer for the longest stamp this program prints */
 		if ((size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > text_cap)
 			text_cap = (size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1);
+		if (skf && (size_t)rtlsdr_gpu_scan_sk_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > sk_cap)
+			sk_cap = (size_t)rtlsdr_gpu_scan_sk_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1);
 	}
 	if (ws.count > 1 && ws.by_pass)
 		fprintf(stderr, "GPU workers: %d (all %d hops each, every %d-th sweep; accumulators merged per report)\n",
@@ -487,8 +450,10 @@ int main(int argc, char **argv)
 	buf8 = (uint8_t *)malloc((size_t)plan->buf_len);
 	/* report landing area: pinned, so every worker's device-to-host copy is plain DMA */
 	text = (char *)rtlsdr_gpu_scan_host_alloc(text_cap);
+	if (skf)
+		sk_text = (char *)rtlsdr_gpu_scan_host_alloc(sk_cap);
 	order = (int *)malloc(sizeof(int) * (size_t)plan->tune_count);
-	if (!buf8 || !text || !order) {
+	if (!buf8 || !text || (skf && !sk_text) || !order) {
 		fprintf(stderr, "Out of memory.\n");
 		return 1;
 	}
@@ -533,19 +498,19 @@ int main(int argc, char **argv)
 				fprintf(stderr, "merging the workers' accumulators: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
 					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[0]));
 		}
-		for (w = 0; w < ws.count && !rc && !ws.by_pass && skf; w++) {
-			rc = write_sk_report(ws.gpu[w], plan, ws.first[w], ws.first[w + 1] - ws.first[w], stamp, out, skf);
-			if (rc)
-				fprintf(stderr, "rtlsdr_gpu_scan_collect_sk: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
-					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
-		}
-		for (w = 0; w < ws.count && !rc && !ws.by_pass && !skf; w++) {
-			rc = rtlsdr_gpu_scan_collect_csv(ws.gpu[w], stamp, text, text_cap, &text_len);
-			if (rc)
-				fprintf(stderr, "rtlsdr_gpu_scan_collect_csv: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
-					rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
-			else
+		/* -K: the SK rows are formatted beside the power rows, with the same read-and-zero */
+		for (w = 0; w < ws.count && !rc && !ws.by_pass; w++) {
+			rc = skf ? rtlsdr_gpu_scan_collect_sk_csv(ws.gpu[w], stamp, text, text_cap, &text_len, sk_text, sk_cap,
+								  &sk_len)
+				 : rtlsdr_gpu_scan_collect_csv(ws.gpu[w], stamp, text, text_cap, &text_len);
+			if (rc) {
+				fprintf(stderr, "%s: %s (%s)\n", skf ? "rtlsdr_gpu_scan_collect_sk_csv" : "rtlsdr_gpu_scan_collect_csv",
+					rtlsdr_gpu_scan_strerror(rc), rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
+			} else {
 				fwrite(text, 1, text_len, out);
+				if (skf)
+					fwrite(sk_text, 1, sk_len, skf);
+			}
 		}
 		fflush(out);
 		if (skf)
@@ -573,6 +538,7 @@ int main(int argc, char **argv)
 	rtlsdr_close(dev);
 	free(buf8);
 	rtlsdr_gpu_scan_host_free(text);
+	rtlsdr_gpu_scan_host_free(sk_text);
 	rtlsdr_gpu_scan_host_free(parts);
 	free(order);
 	free(window_coefs);

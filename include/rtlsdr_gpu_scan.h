@@ -127,7 +127,8 @@ typedef struct rtlsdr_gpu_scan_cfg {
  * evaluated in IEEE doubles in exactly this order without contraction (rtlsdr_b200/csrc/sk.cuh), a quiet NaN
  * when M < 2 or S1 = 0.  Not with peak_hold, bin_e = 0 (rms) or RTLSDR_GPU_FLAG_ASYNC_REPORT
  * (RTLSDR_GPU_ERR_CONFIG at init); on such a handle merge_device() and collect_device() return
- * RTLSDR_GPU_ERR_CONFIG (they do not carry S2).  Every other collect also zeroes S2. */
+ * RTLSDR_GPU_ERR_CONFIG (they do not carry S2): use collect_sk_device() and merge_sk_device(), which do, and
+ * collect_sk_csv() / format_sk_csv_device() for the SK rows' text.  Every other collect also zeroes S2. */
 #define RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS 8u
 
 /* ---- lifecycle --------------------------------------------------------- */
@@ -233,6 +234,14 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_sk(rtlsdr_gpu_scan_t *h, int64_t *avg
  * on the handle's stream, no host synchronisation. */
 RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples, void *dev_db);
 
+/* collect_device() for a RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS handle: the same three outputs plus S2 (dev_s2, u64
+ * [tune_count << bin_e][2] (lo, hi), 8-byte aligned) and the SK rows (dev_sk, double [tune_count][db_count]) as
+ * collect_sk() writes them; any pointer may be NULL.  Read-and-zero of S1, the counts and S2.  Asynchronous on the
+ * handle's stream, no host synchronisation; destinations may be peer-mapped memory of another GPU.
+ * RTLSDR_GPU_ERR_CONFIG on a handle without the flag. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_sk_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples,
+		void *dev_db, void *dev_s2, void *dev_sk);
+
 /*
  * Reads of the SAME hops processed by several handles (e.g. one per GPU, each fed a share of the reads of a
  * single-hop scan): fold `sets` external accumulator sets into this handle's.  Set s is what
@@ -247,6 +256,14 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *de
  */
 RTLSDR_GPU_API int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, const void *dev_samples,
 		int sets, int64_t set_stride);
+
+/* merge_device() for a RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS handle: set s also has its S2 (what collect_sk_device()
+ * wrote, u64 [tune_count << bin_e][2], 8-byte aligned) at dev_s2 + s * set_stride.  S1 and the counts are added like
+ * merge_device() does, S2 as an exact unsigned 128-bit sum (a carry out of the low word goes into the high word), so
+ * a following collect_sk() / collect_sk_csv() returns bit-identical bins, S2 and SK rows to ONE handle that had seen
+ * all the reads.  Same argument and alignment checks as merge_device(); RTLSDR_GPU_ERR_CONFIG without the flag. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_merge_sk_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, const void *dev_samples,
+		const void *dev_s2, int sets, int64_t set_stride);
 
 /*
  * Soft-AGC statistics of hop `hop` since its last collect (needs RTLSDR_GPU_FLAG_LEVEL_STATS):
@@ -299,6 +316,27 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char 
 RTLSDR_GPU_API int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first,
 		int rows, const void *dev_db, int64_t db_stride, const void *dev_samples, void *dev_text, size_t cap,
 		void *dev_len);
+
+/*
+ * The spectral-kurtosis rows of a RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS handle (RTLSDR_GPU_ERR_CONFIG without the flag):
+ * per row the power row's prefix "<stamp>low, high, step, samples, ", then the SK values as printf("%.4f"), joined
+ * by ", " and ended by "\n"; a NaN of either sign (SK undefined) prints "nan".  SK <= M + 1 < 2^31 + 1, so a value
+ * takes at most 15 characters ("2147483649.0000"); a wider one met in a caller's buffer is an error, never text.
+ */
+/* Bytes of `rows` SK rows at their widest: rows * (stamp_len + 56 + 17 * db_count); negative = error. */
+RTLSDR_GPU_API int64_t rtlsdr_gpu_scan_sk_csv_capacity(const rtlsdr_gpu_scan_t *h, int rows, size_t stamp_len);
+/* format_csv_device() for SK rows: row r's values at dev_sk + r * sk_stride doubles (the layout collect_sk_device()
+ * writes), its count at dev_samples[r]; cap >= sk_csv_capacity(rows), *dev_len = -1 for a value outside the
+ * formatter's domain.  Asynchronous on the handle's stream. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_format_sk_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first,
+		int rows, const void *dev_sk, int64_t sk_stride, const void *dev_samples, void *dev_text, size_t cap,
+		void *dev_len);
+/* collect_csv() plus the SK rows: the power rows' text to `text` (*len bytes, cap >= csv_capacity(tune_count)) and
+ * the SK rows' text to `sk_text` (*sk_len bytes, sk_cap >= sk_csv_capacity(tune_count)), with the same read-and-zero
+ * of S1, the counts and S2; only the text crosses PCIe.  On any error the accumulators are left as they were.  Blocks
+ * until both texts are in host memory. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_sk_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap,
+		size_t *len, char *sk_text, size_t sk_cap, size_t *sk_len);
 
 /* ---- multi-GPU report hand-off ----------------------------------------- */
 

@@ -20,7 +20,16 @@
  * kCsvValueMax * db_count bytes; anything wider can only come from a caller's
  * own buffer and is reported as an error instead of printed.
  *
- * Two kernels: csv_rows_kernel formats row r into slot r of a scratch area
+ * %.4f (the spectral-kurtosis rows) needs M * 10^4, which does not fit 64 bits: with k = -E the integer part is
+ * M >> k, and the fraction F = M mod 2^k gives the four decimals D = F * 10^4 >> k, computed exactly in 128 bits
+ * (__umul64hi on the device, unsigned __int128 in the emulator build) and rounded half to even against the
+ * remainder like %.2f (Q = integer * 10^4 + D has D's parity); a carry to D = 10^4 moves into the integer part.
+ * k > 67 means |v| * 10^4 < 2^-1, D = 0.  Sign bit kept (-0.0000), inf with the sign, and every NaN prints "nan"
+ * (the SK rows' format, not glibc's "-nan").  Domain: finite |v| < 2^53, plus inf and NaN.  An SK value is at
+ * most M + 1 < 2^31 + 1 (Cauchy-Schwarz: M * S2 >= S1^2), so an SK row accepts value text of at most 15
+ * characters ("2147483649.0000") and is bounded like a dB row with kCsvSkValueMax per value.
+ *
+ * Three kernels: csv_rows_kernel (dB) or csv_sk_rows_kernel (SK) formats row r into slot r of a scratch area
  * (one CTA per row, a block-wide scan places the variable-width values), then
  * csv_pack_kernel moves every slot to its place in the contiguous text (each
  * CTA sums the lengths of the rows before it) and the last CTA stores the
@@ -38,6 +47,7 @@ namespace rscan {
 constexpr int kCsvStampMax = 128; /* stamp bytes carried in the kernel parameters (length < this) */
 constexpr int kCsvRowFixed = 56;  /* "low, high, step, samples, " at their widest (54) and the newline, rounded up */
 constexpr int kCsvValueMax = 9;   /* "-999.99, " */
+constexpr int kCsvSkValueMax = 17; /* "2147483649.0000, ": SK <= M + 1 (Cauchy-Schwarz) and M < 2^31 */
 constexpr int kCsvThreads = 256;
 constexpr double kCsvStepLimit = 2147483648.0; /* step column: 0 <= step < 2^31 */
 
@@ -120,6 +130,86 @@ SCAN_DEV int csv_fmt_f2(double v, char *out)
 	return n;
 }
 
+/* the high word of the 128-bit product a * b */
+SCAN_DEV unsigned long long csv_mul_hi(unsigned long long a, unsigned long long b)
+{
+#ifdef SCAN_EMU
+	return (unsigned long long)(((unsigned __int128)a * b) >> 64);
+#else
+	return __umul64hi(a, b);
+#endif
+}
+
+/* printf("%.4f", v) into out (at most 22 bytes), except that a NaN of either sign prints "nan"; returns the length,
+ * or -1 for a finite |v| >= 2^53 */
+SCAN_DEV int csv_fmt_f4(double v, char *out)
+{
+	const unsigned long long b = csv_bits(v);
+	const int neg = (int)(b >> 63), e = (int)((b >> 52) & 0x7FF);
+	const unsigned long long frac = b & ((1ull << 52) - 1);
+	int n = 0;
+	if (e == 0x7FF && frac) {
+		out[0] = 'n';
+		out[1] = 'a';
+		out[2] = 'n';
+		return 3;
+	}
+	if (neg)
+		out[n++] = '-';
+	if (e == 0x7FF) {
+		out[n++] = 'i';
+		out[n++] = 'n';
+		out[n++] = 'f';
+		return n;
+	}
+	const unsigned long long M = e ? (frac | (1ull << 52)) : frac;
+	const int E = (e ? e : 1) - 1075;
+	unsigned long long I = 0, D = 0; /* integer part, four decimals */
+	if (E > 0) {                     /* |v| >= 2^53 */
+		return -1;
+	} else if (E == 0) {
+		I = M;
+	} else if (-E <= 67) {           /* else |v| * 10^4 < 2^66 / 2^68: rounds to 0 */
+		const int k = -E;
+		I = k < 64 ? M >> k : 0;
+		const unsigned long long F = k < 64 ? M & ((1ull << k) - 1) : M;
+		/* (nh:nl) = F * 10^4 < 2^67; D = that >> k, rounded half to even against the remainder (rh:rl) */
+		const unsigned long long nl = F * 10000ull, nh = csv_mul_hi(F, 10000ull);
+		unsigned long long rl, rh, hl, hh;
+		if (k < 64) {
+			D = (nl >> k) | (nh << (64 - k));
+			rl = nl & ((1ull << k) - 1);
+			rh = 0;
+			hl = 1ull << (k - 1);
+			hh = 0;
+		} else {
+			D = nh >> (k - 64);
+			rl = nl;
+			rh = nh & ((1ull << (k - 64)) - 1);
+			hl = k == 64 ? 1ull << 63 : 0ull;
+			hh = k == 64 ? 0ull : 1ull << (k - 65);
+		}
+		const bool above = rh > hh || (rh == hh && rl > hl), tie = rh == hh && rl == hl;
+		if (above || (tie && (D & 1)))
+			D++;
+		if (D == 10000) {
+			I++;
+			D = 0;
+		}
+	}
+	char tmp[24];
+	char *end = tmp + sizeof(tmp);
+	for (int i = 0; i < 4; i++) {
+		*--end = (char)('0' + (int)(D % 10));
+		D /= 10;
+	}
+	*--end = '.';
+	char *s = csv_digits_rev(I, end);
+	for (char *p = s; p < tmp + sizeof(tmp); p++)
+		out[n++] = *p;
+	return n;
+}
+
 struct CsvRowParams {
 	const double *db;      /* row r's values at db + r * db_stride */
 	long long db_stride;   /* doubles */
@@ -139,68 +229,22 @@ struct CsvRowParams {
 __global__ void __launch_bounds__(kCsvThreads)
 csv_rows_kernel(const SCAN_GRID_CONSTANT CsvRowParams prm)
 {
-	__shared__ int scan[kCsvThreads];
-	__shared__ int bad;
-	const int row = blockIdx.x, t = threadIdx.x;
-	char *out = prm.slots + (long long)row * prm.slot_bytes;
-	const double *db = prm.db + (long long)row * prm.db_stride;
-	for (int i = t; i < prm.stamp_len; i += kCsvThreads)
-		out[i] = prm.stamp[i];
-	long long pos = prm.stamp_len;
-	if (t == 0) {
-		/* "%i, %i, %.2f, %i, " (rtl_power.c:739-746) */
-		const int2 c = prm.cols[prm.row_first + row];
-		char *p = out + pos;
-		int n = csv_fmt_i(c.x, p);
-		p[n++] = ',';
-		p[n++] = ' ';
-		n += csv_fmt_i(c.y, p + n);
-		p[n++] = ',';
-		p[n++] = ' ';
-		n += csv_fmt_f2(prm.step, p + n); /* 0 <= step < 2^31, checked on the host */
-		p[n++] = ',';
-		p[n++] = ' ';
-		n += csv_fmt_i(prm.samples[row], p + n);
-		p[n++] = ',';
-		p[n++] = ' ';
-		scan[0] = n;
-		bad = 0;
-	}
-	__syncthreads();
-	pos += scan[0];
-	for (int base = 0; base < prm.db_count; base += kCsvThreads) {
-		const int k = base + t;
-		char txt[24];
-		int w = 0;
-		if (k < prm.db_count) {
-			w = csv_fmt_f2(db[k], txt);
-			if (w < 0 || w > kCsvValueMax - 2) {
-				bad = 1;
-				w = 0;
-			} else if (k + 1 < prm.db_count) {
-				txt[w++] = ',';
-				txt[w++] = ' ';
-			} else {
-				txt[w++] = '\n';
-			}
-		}
-		__syncthreads(); /* scan[0] has been read */
-		scan[t] = w;
-		__syncthreads();
-		for (int d = 1; d < kCsvThreads; d <<= 1) { /* inclusive Hillis-Steele scan of the widths */
-			const int add = t >= d ? scan[t - d] : 0;
-			__syncthreads();
-			scan[t] += add;
-			__syncthreads();
-		}
-		char *p = out + pos + scan[t] - w;
-		for (int i = 0; i < w; i++)
-			p[i] = txt[i];
-		pos += scan[kCsvThreads - 1];
-	}
-	__syncthreads();
-	if (t == 0)
-		prm.lens[row] = bad ? -1 : (int)pos;
+#define CSV_FMT_VALUE(v, out) csv_fmt_f2(v, out)
+#define CSV_VALUE_WIDTH (kCsvValueMax - 2)
+#include "csv_rows_body.inl"
+#undef CSV_FMT_VALUE
+#undef CSV_VALUE_WIDTH
+}
+
+/* the SK rows: the same prefix, prm.db holds SK values printed as %.4f ("nan" for any NaN) */
+__global__ void __launch_bounds__(kCsvThreads)
+csv_sk_rows_kernel(const SCAN_GRID_CONSTANT CsvRowParams prm)
+{
+#define CSV_FMT_VALUE(v, out) csv_fmt_f4(v, out)
+#define CSV_VALUE_WIDTH (kCsvSkValueMax - 2)
+#include "csv_rows_body.inl"
+#undef CSV_FMT_VALUE
+#undef CSV_VALUE_WIDTH
 }
 
 struct CsvPackParams {

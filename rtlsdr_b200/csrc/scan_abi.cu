@@ -1357,18 +1357,20 @@ int run_epilogue(rtlsdr_gpu_scan *h, int hop0, int nhops, double *db, long long 
 	return check_launch(h, "epilogue_kernel");
 }
 
-/* bytes of `rows` CSV rows at their widest (csv_text.cuh) */
-size_t csv_bound(const rtlsdr_gpu_scan *h, int rows, size_t stamp_len)
+/* bytes of `rows` CSV rows at their widest (csv_text.cuh): dB rows, or SK rows with sk */
+size_t csv_bound(const rtlsdr_gpu_scan *h, int rows, size_t stamp_len, bool sk = false)
 {
-	return (size_t)rows * (stamp_len + kCsvRowFixed + (size_t)kCsvValueMax * (size_t)h->shape.db_count);
+	const size_t value_max = sk ? kCsvSkValueMax : kCsvValueMax;
+	return (size_t)rows * (stamp_len + kCsvRowFixed + value_max * (size_t)h->shape.db_count);
 }
 
-/* rows [row_first, row_first + rows) of the column table, from dB rows and int32 counts in device memory, into
- * `text` (csv_bound() bytes) and `len` (-1 = a value outside the formatter's domain), on the handle's stream */
+/* rows [row_first, row_first + rows) of the column table, from dB rows (SK rows with sk) and int32 counts in device
+ * memory, into `text` (csv_bound() bytes) and `len` (-1 = a value outside the formatter's domain), on the handle's
+ * stream */
 int run_csv(rtlsdr_gpu_scan *h, const char *stamp, size_t stamp_len, int row_first, int rows, const double *db,
-	    long long db_stride, const int *samples, char *text, long long *len)
+	    long long db_stride, const int *samples, char *text, long long *len, bool sk = false)
 {
-	const size_t slot = csv_bound(h, 1, stamp_len), need = slot * (size_t)rows;
+	const size_t slot = csv_bound(h, 1, stamp_len, sk), need = slot * (size_t)rows;
 	if (need > h->csv_slot_bytes) {
 		cudaFree(h->d_csv_slots);
 		h->d_csv_slots = nullptr;
@@ -1390,8 +1392,11 @@ int run_csv(rtlsdr_gpu_scan *h, const char *stamp, size_t stamp_len, int row_fir
 	p.stamp_len = (int)stamp_len;
 	memcpy(p.stamp, stamp, stamp_len);
 	h->last_was_epilogue = false;
-	csv_rows_kernel<<<rows, kCsvThreads, 0, h->stream>>>(p);
-	if (int rc = check_launch(h, "csv_rows_kernel"))
+	if (sk)
+		csv_sk_rows_kernel<<<rows, kCsvThreads, 0, h->stream>>>(p);
+	else
+		csv_rows_kernel<<<rows, kCsvThreads, 0, h->stream>>>(p);
+	if (int rc = check_launch(h, sk ? "csv_sk_rows_kernel" : "csv_rows_kernel"))
 		return rc;
 	CsvPackParams q;
 	q.slots = h->d_csv_slots;
@@ -1401,6 +1406,25 @@ int run_csv(rtlsdr_gpu_scan *h, const char *stamp, size_t stamp_len, int row_fir
 	q.len = len;
 	csv_pack_kernel<<<rows, kCsvThreads, 0, h->stream>>>(q);
 	return check_launch(h, "csv_pack_kernel");
+}
+
+/* the SK rows of every hop into `sk` ([tune_count][db_count]; may be peer memory).  Reads S1, the sample counters
+ * and S2, so it goes on the handle's stream in front of the epilogue and the memsets that zero them. */
+int run_sk_report(rtlsdr_gpu_scan *h, double *sk)
+{
+	SkReportParams p;
+	p.avg = h->d_avg;
+	p.samples = h->d_smp64;
+	p.s2 = h->d_s2;
+	p.sk = sk;
+	p.bin_e = h->cfg.bin_e;
+	p.i1 = h->shape.db_i1;
+	p.i2 = h->shape.db_i2;
+	p.downsample = h->cfg.downsample;
+	p.hop0 = 0;
+	h->last_was_epilogue = false;
+	sk_report_kernel<<<dim3((h->shape.db_count + 255) / 256, h->cfg.tune_count), 256, 0, h->stream>>>(p);
+	return check_launch(h, "sk_report_kernel");
 }
 
 } // namespace
@@ -2049,20 +2073,8 @@ int rtlsdr_gpu_scan_collect_sk(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples,
 	const size_t N = (size_t)h->shape.N;
 	h->last_was_epilogue = false;
 	if (sk) {
-		/* reads S1 and the sample counters: on the handle's stream in front of collect_range()'s epilogue and
-		 * read-and-zero memsets */
-		SkReportParams p;
-		p.avg = h->d_avg;
-		p.samples = h->d_smp64;
-		p.s2 = h->d_s2;
-		p.sk = h->d_sk;
-		p.bin_e = h->cfg.bin_e;
-		p.i1 = h->shape.db_i1;
-		p.i2 = h->shape.db_i2;
-		p.downsample = h->cfg.downsample;
-		p.hop0 = 0;
-		sk_report_kernel<<<dim3((dbc + 255) / 256, tc), 256, 0, h->stream>>>(p);
-		if ((rc = check_launch(h, "sk_report_kernel")))
+		/* in front of collect_range()'s epilogue and read-and-zero memsets */
+		if ((rc = run_sk_report(h, h->d_sk)))
 			return rc;
 		CU(cudaMemcpyAsync(sk, h->d_sk, (size_t)tc * dbc * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
 		h->d2h += (uint64_t)tc * dbc * sizeof(double);
@@ -2073,6 +2085,29 @@ int rtlsdr_gpu_scan_collect_sk(rtlsdr_gpu_scan_t *h, int64_t *avg, int *samples,
 	}
 	/* dB rows, raw copies, and the read-and-zero of S1, the counters and S2 */
 	return collect_range(h, 0, tc, avg, samples, db);
+}
+
+/* collect_device()'s report on the handle's stream: the epilogue into the caller's buffers, then the read-and-zero
+ * (fused into the epilogue up to 8192 bins) */
+static int report_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples, void *dev_db)
+{
+	const size_t N = (size_t)h->shape.N, tc = (size_t)h->cfg.tune_count;
+	const bool fused_zero = N <= 8192;
+	int rc;
+	if ((rc = run_epilogue(h, 0, (int)tc, (double *)dev_db, (long long *)dev_avg, (int *)dev_samples, fused_zero)))
+		return rc;
+	if (!fused_zero) {
+		h->last_was_epilogue = false;
+		CU(cudaMemsetAsync(h->d_avg, 0, (tc * N + tc) * sizeof(long long), h->stream));
+	}
+	if (h->d_level) {
+		h->last_was_epilogue = false;
+		CU(cudaMemsetAsync(h->d_level, 0, tc * 2 * sizeof(unsigned long long), h->stream));
+		std::fill(h->level_bytes.begin(), h->level_bytes.end(), 0);
+	}
+	std::fill(h->samples.begin(), h->samples.end(), 0);
+	h->samples_on_device = false;
+	return 0;
 }
 
 int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples, void *dev_db)
@@ -2117,19 +2152,30 @@ int rtlsdr_gpu_scan_collect_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *de
 		h->samples_on_device = false;
 		return 0;
 	}
-	if ((rc = run_epilogue(h, 0, (int)tc, (double *)dev_db, (long long *)dev_avg, (int *)dev_samples, fused_zero)))
+	return report_device(h, dev_avg, dev_samples, dev_db);
+}
+
+int rtlsdr_gpu_scan_collect_sk_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void *dev_samples, void *dev_db,
+				      void *dev_s2, void *dev_sk)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc = flush_ring(h);
+	if (rc)
 		return rc;
-	if (!fused_zero) {
-		h->last_was_epilogue = false;
-		CU(cudaMemsetAsync(h->d_avg, 0, (tc * N + tc) * sizeof(long long), h->stream));
-	}
-	if (h->d_level) {
-		h->last_was_epilogue = false;
-		CU(cudaMemsetAsync(h->d_level, 0, tc * 2 * sizeof(unsigned long long), h->stream));
-		std::fill(h->level_bytes.begin(), h->level_bytes.end(), 0);
-	}
-	std::fill(h->samples.begin(), h->samples.end(), 0);
-	h->samples_on_device = false;
+	const size_t s2_bytes = (size_t)h->cfg.tune_count * h->shape.N * 2 * sizeof(unsigned long long);
+	/* S1, the counters and S2 are read here, in front of the epilogue's fused zeroing and the memsets */
+	if (dev_sk && (rc = run_sk_report(h, (double *)dev_sk)))
+		return rc;
+	if (dev_s2)
+		CU(cudaMemcpyAsync(dev_s2, h->d_s2, s2_bytes, cudaMemcpyDefault, h->stream));
+	if ((rc = report_device(h, dev_avg, dev_samples, dev_db)))
+		return rc;
+	h->last_was_epilogue = false;
+	CU(cudaMemsetAsync(h->d_s2, 0, s2_bytes, h->stream));
 	return 0;
 }
 
@@ -2172,44 +2218,62 @@ int64_t rtlsdr_gpu_scan_csv_capacity(const rtlsdr_gpu_scan_t *h, int rows, size_
 	return (int64_t)csv_bound(h, rows, stamp_len);
 }
 
-int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len)
+int64_t rtlsdr_gpu_scan_sk_csv_capacity(const rtlsdr_gpu_scan_t *h, int rows, size_t stamp_len)
 {
-	if (!h || !stamp || !text || !len)
+	if (!h)
 		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_s2 || rows < 0 || stamp_len >= (size_t)kCsvStampMax)
+		return RTLSDR_GPU_ERR_CONFIG;
+	return (int64_t)csv_bound(h, rows, stamp_len, true);
+}
+
+/* collect_csv(), and with sk_text also the SK rows (collect_sk_csv()) */
+static int collect_text(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len, char *sk_text,
+			size_t sk_cap, size_t *sk_len)
+{
 	const size_t stamp_len = strlen(stamp);
 	const int tc = h->cfg.tune_count;
 	if (stamp_len >= (size_t)kCsvStampMax || h->csv_rows < tc)
 		return RTLSDR_GPU_ERR_CONFIG;
-	const size_t bound = csv_bound(h, tc, stamp_len);
-	if (cap < bound)
+	const size_t bound = csv_bound(h, tc, stamp_len), sk_bound = sk_text ? csv_bound(h, tc, stamp_len, true) : 0;
+	if (cap < bound || sk_cap < sk_bound)
 		return RTLSDR_GPU_ERR_LENGTH;
 	CU(cudaSetDevice(h->cfg.device));
 	int rc = flush_ring(h);
 	if (rc)
 		return rc;
-	if (!h->d_csv_len) {
-		CU(cudaMalloc(&h->d_csv_len, sizeof(long long)));
-		CU(cudaMallocHost(&h->h_csv_len, sizeof(long long)));
+	if (!h->d_csv_len) { /* [0] the power text's length, [1] the SK text's */
+		CU(cudaMalloc(&h->d_csv_len, 2 * sizeof(long long)));
+		CU(cudaMallocHost(&h->h_csv_len, 2 * sizeof(long long)));
 	}
-	if (bound > h->csv_text_bytes) {
+	if (bound + sk_bound > h->csv_text_bytes) {
 		cudaFree(h->d_csv_text);
 		h->d_csv_text = nullptr;
 		h->csv_text_bytes = 0;
-		CU(cudaMalloc(&h->d_csv_text, bound));
-		h->csv_text_bytes = bound;
+		CU(cudaMalloc(&h->d_csv_text, bound + sk_bound));
+		h->csv_text_bytes = bound + sk_bound;
 	}
+	/* in front of the epilogue: reads S1, the counters and S2 */
+	if (sk_text && (rc = run_sk_report(h, h->d_sk)))
+		return rc;
 	/* the epilogue's dB rows and counts stay on the device: only the text crosses PCIe */
 	if ((rc = run_epilogue(h, 0, tc, h->d_db, nullptr, h->d_samples)))
 		return rc;
 	if ((rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_db, h->shape.db_count, h->d_samples, h->d_csv_text, h->d_csv_len)))
 		return rc;
-	CU(cudaMemcpyAsync(h->h_csv_len, h->d_csv_len, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+	if (sk_text && (rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_sk, h->shape.db_count, h->d_samples,
+				      h->d_csv_text + bound, h->d_csv_len + 1, true)))
+		return rc;
+	const int nlen = sk_text ? 2 : 1;
+	CU(cudaMemcpyAsync(h->h_csv_len, h->d_csv_len, nlen * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
 	CU(cudaStreamSynchronize(h->stream));
-	const long long n = *h->h_csv_len;
-	if (n < 0 || (size_t)n > bound)
-		return RTLSDR_GPU_ERR_CONFIG; /* cannot happen for the epilogue's values; the accumulators are kept */
+	const long long n = h->h_csv_len[0], m = sk_text ? h->h_csv_len[1] : 0;
+	if (n < 0 || (size_t)n > bound || m < 0 || (size_t)m > sk_bound)
+		return RTLSDR_GPU_ERR_CONFIG; /* cannot happen for the report's values; the accumulators are kept */
 	CU(cudaMemcpyAsync(text, h->d_csv_text, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
-	h->d2h += (uint64_t)n + sizeof(long long);
+	if (sk_text)
+		CU(cudaMemcpyAsync(sk_text, h->d_csv_text + bound, (size_t)m, cudaMemcpyDeviceToHost, h->stream));
+	h->d2h += (uint64_t)n + (uint64_t)m + nlen * sizeof(long long);
 	/* read-and-zero, like csv_dbm (rtl_power.c:761-764) */
 	CU(cudaMemsetAsync(h->d_avg, 0, ((size_t)tc * h->shape.N + (size_t)tc) * sizeof(long long), h->stream));
 	if (h->d_level)
@@ -2222,27 +2286,60 @@ int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *t
 		std::fill(h->level_bytes.begin(), h->level_bytes.end(), 0);
 	h->samples_on_device = false;
 	*len = (size_t)n;
+	if (sk_len)
+		*sk_len = (size_t)m;
 	return 0;
 }
 
-int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first, int rows,
-				      const void *dev_db, int64_t db_stride, const void *dev_samples, void *dev_text,
-				      size_t cap, void *dev_len)
+int rtlsdr_gpu_scan_collect_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len)
+{
+	if (!h || !stamp || !text || !len)
+		return RTLSDR_GPU_ERR_NULL;
+	return collect_text(h, stamp, text, cap, len, nullptr, 0, nullptr);
+}
+
+int rtlsdr_gpu_scan_collect_sk_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len,
+				   char *sk_text, size_t sk_cap, size_t *sk_len)
+{
+	if (!h || !stamp || !text || !len || !sk_text || !sk_len)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	return collect_text(h, stamp, text, cap, len, sk_text, sk_cap, sk_len);
+}
+
+/* format_csv_device(), or with sk format_sk_csv_device() */
+static int format_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first, int rows, const void *dev_db,
+			 int64_t db_stride, const void *dev_samples, void *dev_text, size_t cap, void *dev_len, bool sk)
 {
 	if (!h || !stamp || !dev_db || !dev_samples || !dev_text || !dev_len)
 		return RTLSDR_GPU_ERR_NULL;
 	if (((uintptr_t)dev_db & 7) || ((uintptr_t)dev_samples & 3) || ((uintptr_t)dev_len & 7))
 		return RTLSDR_GPU_ERR_ALIGN;
 	const size_t stamp_len = strlen(stamp);
-	if (stamp_len >= (size_t)kCsvStampMax || !h->d_csv_cols || db_stride < h->shape.db_count)
+	if (stamp_len >= (size_t)kCsvStampMax || !h->d_csv_cols || db_stride < h->shape.db_count || (sk && !h->d_s2))
 		return RTLSDR_GPU_ERR_CONFIG;
 	if (rows < 1 || row_first < 0 || row_first > h->csv_rows - rows)
 		return RTLSDR_GPU_ERR_HOP;
-	if (cap < csv_bound(h, rows, stamp_len))
+	if (cap < csv_bound(h, rows, stamp_len, sk))
 		return RTLSDR_GPU_ERR_LENGTH;
 	CU(cudaSetDevice(h->cfg.device));
 	return run_csv(h, stamp, stamp_len, row_first, rows, (const double *)dev_db, (long long)db_stride,
-		       (const int *)dev_samples, (char *)dev_text, (long long *)dev_len);
+		       (const int *)dev_samples, (char *)dev_text, (long long *)dev_len, sk);
+}
+
+int rtlsdr_gpu_scan_format_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first, int rows,
+				      const void *dev_db, int64_t db_stride, const void *dev_samples, void *dev_text,
+				      size_t cap, void *dev_len)
+{
+	return format_device(h, stamp, row_first, rows, dev_db, db_stride, dev_samples, dev_text, cap, dev_len, false);
+}
+
+int rtlsdr_gpu_scan_format_sk_csv_device(rtlsdr_gpu_scan_t *h, const char *stamp, int row_first, int rows,
+					 const void *dev_sk, int64_t sk_stride, const void *dev_samples, void *dev_text,
+					 size_t cap, void *dev_len)
+{
+	return format_device(h, stamp, row_first, rows, dev_sk, sk_stride, dev_samples, dev_text, cap, dev_len, true);
 }
 
 int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, const void *dev_samples, int sets,
@@ -2275,6 +2372,39 @@ int rtlsdr_gpu_scan_merge_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, cons
 	merge_sets_kernel<<<std::max(grid, 1), 256, 0, h->stream>>>(p);
 	h->samples_on_device = true; /* the host mirror of tunes[i].samples no longer knows the totals */
 	return check_launch(h, "merge_sets_kernel");
+}
+
+int rtlsdr_gpu_scan_merge_sk_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, const void *dev_samples,
+				    const void *dev_s2, int sets, int64_t set_stride)
+{
+	if (!h || !dev_avg || !dev_samples || !dev_s2)
+		return RTLSDR_GPU_ERR_NULL;
+	if (sets <= 0 || (sets > 1 && set_stride <= 0))
+		return RTLSDR_GPU_ERR_CONFIG;
+	if (((uintptr_t)dev_avg & 7) || ((uintptr_t)dev_samples & 3) || ((uintptr_t)dev_s2 & 7) || (set_stride & 7))
+		return RTLSDR_GPU_ERR_ALIGN;
+	if (!h->d_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc = flush_ring(h);
+	if (rc)
+		return rc;
+	MergeSkParams p;
+	p.avg = h->d_avg;
+	p.samples = h->d_smp64;
+	p.s2 = h->d_s2;
+	p.ext_avg = (const uint8_t *)dev_avg;
+	p.ext_smp = (const uint8_t *)dev_samples;
+	p.ext_s2 = (const uint8_t *)dev_s2;
+	p.stride = set_stride;
+	p.bins = (long long)h->cfg.tune_count * h->shape.N;
+	p.hops = h->cfg.tune_count;
+	p.sets = sets;
+	const int grid = (int)std::min<long long>((p.bins + 255) / 256, (long long)h->num_sms * 8);
+	h->last_was_epilogue = false;
+	merge_sk_sets_kernel<<<std::max(grid, 1), 256, 0, h->stream>>>(p);
+	h->samples_on_device = true; /* the host mirror of tunes[i].samples no longer knows the totals */
+	return check_launch(h, "merge_sk_sets_kernel");
 }
 
 int rtlsdr_gpu_scan_level_stats(rtlsdr_gpu_scan_t *h, int hop, uint64_t *overload, uint64_t *high_level, uint64_t *bytes)

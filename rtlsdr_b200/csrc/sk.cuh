@@ -150,4 +150,48 @@ sk_report_kernel(const SCAN_GRID_CONSTANT SkReportParams prm)
 		sk_from_moments(prm.avg[b], prm.s2[2 * b], prm.s2[2 * b + 1], prm.samples[hop] / prm.downsample);
 }
 
+/* Reads of the same hops on several SK handles (rtlsdr_gpu_scan_merge_sk_device): `sets` external sets -- S1 int64
+ * [bins], int32 counts [hops] and S2 (lo, hi) u64 [bins][2] at ext_* + s * stride -- are added into this handle's
+ * accumulators.  S2 is added as an unsigned 128-bit value (a wrap of the low word carries into the high word), so the
+ * merged sums do not depend on how the reads were grouped.  No peak hold on an SK handle. */
+struct MergeSkParams {
+	long long *avg;                     /* [bins] */
+	long long *samples;                 /* [hops] */
+	unsigned long long *s2;             /* [bins][2] */
+	const uint8_t *ext_avg;
+	const uint8_t *ext_smp;
+	const uint8_t *ext_s2;
+	long long stride;
+	long long bins;
+	int hops;
+	int sets;
+};
+
+__global__ void __launch_bounds__(256)
+merge_sk_sets_kernel(const SCAN_GRID_CONSTANT MergeSkParams prm)
+{
+	const long long step = (long long)gridDim.x * blockDim.x;
+	const long long first = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+	for (long long i = first; i < prm.bins; i += step) {
+		long long v = prm.avg[i];
+		unsigned long long lo = prm.s2[2 * i], hi = prm.s2[2 * i + 1];
+		for (int s = 0; s < prm.sets; ++s) {
+			v += ((const long long *)(prm.ext_avg + s * prm.stride))[i];
+			const unsigned long long *e = (const unsigned long long *)(prm.ext_s2 + s * prm.stride) + 2 * i;
+			const unsigned long long el = e[0];
+			lo += el;
+			hi += e[1] + (lo < el ? 1ull : 0ull);
+		}
+		prm.avg[i] = v;
+		prm.s2[2 * i] = lo;
+		prm.s2[2 * i + 1] = hi;
+	}
+	for (long long i = first; i < prm.hops; i += step) {
+		long long v = prm.samples[i];
+		for (int s = 0; s < prm.sets; ++s)
+			v += ((const int *)(prm.ext_smp + s * prm.stride))[i];
+		prm.samples[i] = v;
+	}
+}
+
 } // namespace rscan

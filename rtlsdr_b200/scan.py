@@ -58,6 +58,14 @@ def load_library():
     L.rtlsdr_gpu_scan_collect_device.argtypes = [vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_collect_sk.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rtlsdr_gpu_scan_merge_device.argtypes = [vp, vp, vp, i, i64]
+    L.rtlsdr_gpu_scan_collect_sk_device.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.rtlsdr_gpu_scan_merge_sk_device.argtypes = [vp, vp, vp, vp, i, i64]
+    L.rtlsdr_gpu_scan_sk_csv_capacity.argtypes = [vp, i, ctypes.c_size_t]
+    L.rtlsdr_gpu_scan_sk_csv_capacity.restype = i64
+    L.rtlsdr_gpu_scan_format_sk_csv_device.argtypes = [vp, ctypes.c_char_p, i, i, vp, i64, vp, vp, ctypes.c_size_t, vp]
+    L.rtlsdr_gpu_scan_collect_sk_csv.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t,
+                                                 ctypes.POINTER(ctypes.c_size_t), vp, ctypes.c_size_t,
+                                                 ctypes.POINTER(ctypes.c_size_t)]
     L.rtlsdr_gpu_scan_set_csv_columns.argtypes = [vp, i, vp, vp, ctypes.c_double]
     L.rtlsdr_gpu_scan_csv_capacity.argtypes = [vp, i, ctypes.c_size_t]
     L.rtlsdr_gpu_scan_csv_capacity.restype = i64
@@ -272,6 +280,18 @@ class GpuScan:
         `set_stride` bytes apart; may be peer memory) into this handle's: sums, or maxima under peak hold"""
         self._check(self.lib.rtlsdr_gpu_scan_merge_device(self.h, dev_avg, dev_samples, sets, set_stride), "merge_device")
 
+    def collect_sk_device(self, dev_avg=None, dev_samples=None, dev_db=None, dev_s2=None, dev_sk=None):
+        """collect_device() plus S2 (uint64 [tc, N, 2]) and the SK rows (float64 [tc, db_count]) of a
+        spectral_kurtosis=True handle; any address may be None; async on the handle's stream"""
+        self._check(self.lib.rtlsdr_gpu_scan_collect_sk_device(self.h, dev_avg, dev_samples, dev_db, dev_s2, dev_sk),
+                    "collect_sk_device")
+
+    def merge_sk_device(self, dev_avg, dev_samples, dev_s2, sets=1, set_stride=0):
+        """merge_device() plus S2 (what collect_sk_device wrote, `set_stride` bytes apart like the other two),
+        added as exact 128-bit sums"""
+        self._check(self.lib.rtlsdr_gpu_scan_merge_sk_device(self.h, dev_avg, dev_samples, dev_s2, sets, set_stride),
+                    "merge_sk_device")
+
     def set_csv_columns(self, low, high, step):
         """row table of the CSV formatter: row r prints low[r], high[r], step (Plan.csv_columns())"""
         lo = np.ascontiguousarray(low, dtype=np.int32)
@@ -296,6 +316,33 @@ class GpuScan:
         self._check(self.lib.rtlsdr_gpu_scan_collect_csv(self.h, s, out.ctypes.data, out.nbytes, ctypes.byref(n)),
                     "collect_csv")
         return out[: n.value].tobytes()
+
+    def sk_csv_capacity(self, rows, stamp_len):
+        """bytes `rows` spectral-kurtosis rows with a stamp of `stamp_len` bytes can take at most"""
+        n = self.lib.rtlsdr_gpu_scan_sk_csv_capacity(self.h, rows, stamp_len)
+        self._check(n if n < 0 else 0, "sk_csv_capacity")
+        return n
+
+    def collect_sk_csv(self, stamp, out=None, sk_out=None):
+        """collect_csv() plus the spectral-kurtosis rows: (power rows' text, SK rows' text) as bytes, formatted on
+        the GPU; out / sk_out: optional writable uint8 buffers"""
+        s = stamp.encode() if isinstance(stamp, str) else bytes(stamp)
+        if out is None:
+            out = np.empty(max(1, self.csv_capacity(self.tune_count, len(s))), dtype=np.uint8)
+        if sk_out is None:
+            sk_out = np.empty(max(1, self.sk_csv_capacity(self.tune_count, len(s))), dtype=np.uint8)
+        n, m = ctypes.c_size_t(0), ctypes.c_size_t(0)
+        self._check(self.lib.rtlsdr_gpu_scan_collect_sk_csv(self.h, s, out.ctypes.data, out.nbytes, ctypes.byref(n),
+                                                            sk_out.ctypes.data, sk_out.nbytes, ctypes.byref(m)),
+                    "collect_sk_csv")
+        return out[: n.value].tobytes(), sk_out[: m.value].tobytes()
+
+    def format_sk_csv_device(self, stamp, row_first, rows, dev_sk, sk_stride, dev_samples, dev_text, cap, dev_len):
+        """format_csv_device() for the SK rows of a collect_sk_device() report (sk_stride doubles apart)"""
+        s = stamp.encode() if isinstance(stamp, str) else bytes(stamp)
+        self._check(self.lib.rtlsdr_gpu_scan_format_sk_csv_device(self.h, s, row_first, rows, dev_sk, sk_stride,
+                                                                  dev_samples, dev_text, cap, dev_len),
+                    "format_sk_csv_device")
 
     def format_csv_device(self, stamp, row_first, rows, dev_db, db_stride, dev_samples, dev_text, cap, dev_len):
         """rows [row_first, row_first + rows) of a collect_device() report (dB rows db_stride doubles apart,

@@ -99,19 +99,24 @@ class IntervalReport:
     avg: np.ndarray       # [tune_count, N] int64, natural FFT order
     db: np.ndarray        # [tune_count, db_count] float64
     samples: np.ndarray   # [tune_count] int32
+    s2: Optional[np.ndarray] = None   # sk: [tune_count, N, 2] uint64 (lo, hi) sums of |X|^4
+    sk: Optional[np.ndarray] = None   # sk: [tune_count, db_count] float64 SK rows
 
 
 class SpectrumGather:
     """One rank's side of the per-interval exchange.
 
     A report buffer is `words` int64 words: [avg hmax*N | db hmax*db_count (bit patterns) |
-    samples hmax x int32, padded to 8 bytes], hmax = the largest shard.  Use per interval j
+    samples hmax x int32, padded to 8 bytes], hmax = the largest shard; with sk=True (spectral-kurtosis handles)
+    followed by [S2 hmax*N*2 (lo, hi) | SK rows hmax*db_count], at word offsets s2_at and sk_at.  Use per interval j
     (k = j % SLOTS):
         before_collect(k, stream); collect_device(*pointers(k)); publish(k, stream)
+        (sk: collect_sk_device(*pointers(k), *sk_pointers(k)))
         ... later, rank 0: fetch(k)  (needs publish(..., to_host=True))
     """
 
-    def __init__(self, tune_count, n_bins, db_count, world, rank, device, mode=None, sizes=None, replicated=False):
+    def __init__(self, tune_count, n_bins, db_count, world, rank, device, mode=None, sizes=None, replicated=False,
+                 sk=False):
         self.tune_count, self.n, self.db_count = tune_count, n_bins, db_count
         self.world, self.rank = world, rank
         self.device = torch.device(device)
@@ -123,6 +128,12 @@ class SpectrumGather:
         self.hmax = max(1, max(len(r) for r in self.ranges))
         self.smp_words = (self.hmax + 1) // 2
         self.words = self.hmax * (n_bins + db_count) + self.smp_words
+        self.sk = sk
+        self.s2_at = self.sk_at = None
+        if sk:
+            self.s2_at = self.words
+            self.sk_at = self.s2_at + self.hmax * n_bins * 2
+            self.words = self.sk_at + self.hmax * db_count
         self.my_hops = self.ranges[rank]
         self.peer = None
         # peer mode: int32 flags behind the report buffers of the symmetric allocation:
@@ -218,9 +229,21 @@ class SpectrumGather:
         p_smp = p_db + self.hmax * self.db_count * 8
         return base, p_smp, p_db
 
+    def sk_pointers(self, k=0):
+        """sk: device addresses of S2 and the SK rows for rtlsdr_gpu_scan_collect_sk_device() of report buffer k,
+        behind pointers(k)'s sections of the same slot"""
+        return self.sk_sections(self.pointers(k)[0])
+
+    def sk_sections(self, slot_base):
+        """sk: (address of S2, address of the SK rows) of the slot starting at `slot_base`; slots are words * 8
+        bytes apart, so merge_sk_device() walks the S2 of consecutive slots with that stride"""
+        assert self.sk
+        return slot_base + self.s2_at * 8, slot_base + self.sk_at * 8
+
     def views(self, k=0):
         """(avg [h, N] int64, db [h, db_count] float64, samples [h] int32) views of the LOCAL send buffer k
-        sized for this rank's hop count (host mode / tests fill these instead of a GPU epilogue)"""
+        sized for this rank's hop count (host mode / tests fill these instead of a GPU epilogue); with sk also
+        (s2 [h, N, 2] uint64, sk [h, db_count] float64)"""
         h = len(self.my_hops)
         s = self.send[k]
         a = s[: self.hmax * self.n].view(self.hmax, self.n)[:h]
@@ -228,7 +251,11 @@ class SpectrumGather:
         d = s[o: o + self.hmax * self.db_count].view(torch.float64).view(self.hmax, self.db_count)[:h]
         o += self.hmax * self.db_count
         c = s[o: o + self.smp_words].view(torch.int32)[:h]
-        return a, d, c
+        if not self.sk:
+            return a, d, c
+        s2 = s[self.s2_at: self.sk_at].view(torch.uint64).view(self.hmax, self.n, 2)[:h]
+        sk = s[self.sk_at: self.words].view(torch.float64).view(self.hmax, self.db_count)[:h]
+        return a, d, c, s2, sk
 
     def _flag_addr(self, owner, index):
         """device address (as seen from this rank) of int32 flag `index` in rank `owner`'s symmetric buffer"""
@@ -362,6 +389,10 @@ class SpectrumGather:
         p_db = base + self.hmax * self.n * 8
         return p_db, p_db + self.hmax * self.db_count * 8
 
+    def slot_sk(self, k, r):
+        """rank 0, sk: (device address of S2, of the SK rows) of rank r's slot in the private copy of buffer k"""
+        return self.sk_sections(self.dev_copy[k].data_ptr() + r * self.words * 8)
+
     def release_copy(self, k, stream):
         """rank 0, replicated mode: everything enqueued so far on `stream` (the merge) is the last reader of the
         private copy of buffer k; the exchange two intervals later waits for it before overwriting the copy"""
@@ -374,6 +405,8 @@ class SpectrumGather:
         avg = np.zeros((self.tune_count, self.n), dtype=np.int64)
         db = np.zeros((self.tune_count, self.db_count), dtype=np.float64)
         smp = np.zeros(self.tune_count, dtype=np.int32)
+        s2 = np.zeros((self.tune_count, self.n, 2), dtype=np.uint64) if self.sk else None
+        sk = np.zeros((self.tune_count, self.db_count), dtype=np.float64) if self.sk else None
         for r in range(self.world):
             hops = self.ranges[r]
             h = len(hops)
@@ -386,7 +419,11 @@ class SpectrumGather:
                 self.hmax, self.db_count)[:h]
             o += self.hmax * self.db_count
             smp[hops.start: hops.stop] = b[o: o + self.smp_words].view(np.int32)[:h]
-        return IntervalReport(avg, db, smp)
+            if self.sk:
+                s2[hops.start: hops.stop] = b[self.s2_at: self.sk_at].view(np.uint64).reshape(self.hmax, self.n, 2)[:h]
+                sk[hops.start: hops.stop] = b[self.sk_at: self.words].view(np.float64).reshape(
+                    self.hmax, self.db_count)[:h]
+        return IntervalReport(avg, db, smp, s2, sk)
 
     def describe(self):
         return {"peer": "every rank's report epilogue stores its int64 bins + dB + counts straight into rank 0's "

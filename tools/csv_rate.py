@@ -13,6 +13,11 @@ format_csv_device on a collect_device report), CUDA events over repeated launche
 on its own stream at the same time (the alternative to formatting behind the exchange on the handle's stream).
 --sweep-main times `sweep_main -f 24M:1766M:1k --sweeps 64 --intervals 8` end to end (and the same command from
 --baseline-tree, e.g. a checkout of the parent commit with its library built).
+--sk measures the spectral-kurtosis rows instead, on two spectral_kurtosis=True handles fed the same reads:
+  host  collect_sk() then the power rows through rp_csv_row() and the SK rows through Python's "%.4f" (the bytes
+        rtl_power_gpu -K printed with host printf before collect_sk_csv; Python's formatter stands in for printf)
+  gpu   collect_sk_csv(): both texts formatted on the GPU, only text to the host
+and with --sweep-main times the sweep_main command above with and without `--sk FILE`, alternated.
 Records the GPU name and power limit beside the numbers.  Needs a CUDA device: there is no CPU fallback."""
 import argparse
 import json
@@ -136,10 +141,58 @@ def run_config(torch, rs, cfg, reps):
     return res
 
 
-def time_sweep_main(tree, reps):
+def run_sk_config(torch, rs, cfg, reps):
+    import math
+    from rtlsdr_b200.planner import plan_scan, synth_cube
+    rng_, crop, fir, sweeps = CONFIGS[cfg]
+    plan = plan_scan(rng_, crop, fir)
+    pd = plan.as_dict()
+    pd["peak_hold"] = 0
+    tc, b, n = pd["tune_count"], pd["buf_len"], 1 << pd["bin_e"]
+    w = rs.window_coefs("hamming", n)
+    host_g = rs.GpuScan.from_plan(pd, window_coefs=w, spectral_kurtosis=True)
+    gpu_g = rs.GpuScan.from_plan(pd, window_coefs=w, spectral_kurtosis=True)
+    gpu_g.set_csv_columns(*plan.csv_columns())
+    low, high, step = plan.csv_columns()
+    pin = rs.PinnedBuffer(sweeps * tc * b)
+    synth_cube(pin.ptr, 0, 1, 0, tc, 0, tc, 0, sweeps, b)
+    cube = torch.from_numpy(pin.array).cuda()
+    out = np.empty(gpu_g.csv_capacity(tc, len(STAMP)), dtype=np.uint8)
+    sk_out = np.empty(gpu_g.sk_csv_capacity(tc, len(STAMP)), dtype=np.uint8)
+    host_ms, gpu_ms, same = [], [], True
+    for _ in range(reps + 1):                       # the first round warms up both paths
+        feed(torch, pd, (host_g, gpu_g), sweeps, cube)
+        host_g.sync()
+        gpu_g.sync()
+        t0 = time.perf_counter()
+        _, smp, db, _, sk = host_g.collect_sk()
+        text_h = "".join(STAMP + plan.csv_row(h, int(smp[h]), db[h]) for h in range(tc)).encode()
+        sk_h = "".join("%s%i, %i, %.2f, %i, " % (STAMP, low[h], high[h], step, smp[h])
+                       + ", ".join("nan" if math.isnan(v) else "%.4f" % v for v in sk[h].tolist()) + "\n"
+                       for h in range(tc)).encode()
+        t1 = time.perf_counter()
+        text_g, sk_g = gpu_g.collect_sk_csv(STAMP, out=out, sk_out=sk_out)
+        t2 = time.perf_counter()
+        same &= text_h == text_g and sk_h == sk_g
+        host_ms.append((t1 - t0) * 1e3)
+        gpu_ms.append((t2 - t1) * 1e3)
+    host_ms, gpu_ms = host_ms[1:], gpu_ms[1:]
+    values = tc * gpu_g.db_count
+    res = dict(config=cfg, range=rng_, hops=tc, bins=n, sweeps=sweeps, values_per_text=values,
+               text_bytes=len(text_g), sk_text_bytes=len(sk_g), identical_bytes=bool(same),
+               host_ms=[round(x, 2) for x in host_ms], gpu_ms=[round(x, 3) for x in gpu_ms],
+               host_ms_median=round(float(np.median(host_ms)), 2), gpu_ms_median=round(float(np.median(gpu_ms)), 3),
+               speedup=round(float(np.median(host_ms) / np.median(gpu_ms)), 1))
+    for g in (host_g, gpu_g):
+        g.close()
+    pin.free()
+    return res
+
+
+def time_sweep_main(tree, reps, extra=()):
     out, env = [], dict(os.environ, PYTHONPATH=tree, PYTHONDONTWRITEBYTECODE="1")
     cmd = [sys.executable, "-m", "rtlsdr_b200.sweep_main", "-f", "24M:1766M:1k", "--sweeps", "64",
-           "--intervals", "8", "-o", os.devnull]
+           "--intervals", "8", "-o", os.devnull] + list(extra)
     for _ in range(reps):
         t0 = time.perf_counter()
         subprocess.run(cmd, cwd=tree, env=env, check=True, capture_output=True)
@@ -152,12 +205,25 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--sweep-main", action="store_true")
     ap.add_argument("--baseline-tree", default=None)
+    ap.add_argument("--sk", action="store_true", help="the spectral-kurtosis rows (see above)")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("csv_rate: no CUDA device")
     import rtlsdr_b200.scan as rs
     rs.load_library()
+    if args.sk:
+        import tempfile
+        res = dict(gpu=gpu_info(), sk_configs=[run_sk_config(torch, rs, c, args.reps) for c in (3, 5)])
+        if args.sweep_main:
+            sm = dict(without_sk_s=[], with_sk_s=[])
+            with tempfile.TemporaryDirectory() as tmp:
+                for _ in range(3):
+                    sm["without_sk_s"] += time_sweep_main(ROOT, 1)
+                    sm["with_sk_s"] += time_sweep_main(ROOT, 1, ["--sk", os.path.join(tmp, "sk.csv")])
+            res["sweep_main_24M_1766M_1k_64x8"] = sm
+        print(json.dumps(res, indent=1))
+        return
     res = dict(gpu=gpu_info(), configs=[run_config(torch, rs, c, args.reps) for c in (3, 5)])
     if args.sweep_main:
         # alternate the two trees so that drift on a shared host hits both alike
