@@ -83,6 +83,7 @@ static void print_usage(void)
 		"\t[-c crop_percent (default: 0%%)]\n"
 		"\t[-F fir_size (default: disabled)] (0 or 9; switches boxcar off)\n"
 		"\t[-P enables peak hold (default: off)]\n"
+		"\t[-G fix_fft with 8 guard bits: the transform rounds 2^8 below the reference's LSB (default: off)]\n"
 		"\t[-s avg|iir (default: avg; iir smooths the dB rows across reports)]\n"
 		"\t[-t workers (default: 1; hops -- or, with fewer hops than workers, sweeps -- are sharded over this many GPUs)]\n"
 		"\t[-R seed (visit the hops of every sweep in a random order)]\n"
@@ -261,6 +262,7 @@ int main(int argc, char **argv)
 	const char *range = NULL, *window = "rectangle", *filename = "-", *sk_filename = NULL;
 	const char *fixed_stamp = getenv("RTL_POWER_TIMESTAMP");
 	int opt, interval = 10, single = 0, peak_hold = 0, boxcar = 1, comp_fir_size = 0;
+	int guard_bits = 0;
 	int passes_per_report = env_int("RTL_POWER_PASSES", 0), passes = 0, rc = 0, hop, w;
 	int max_reports = env_int("RTL_POWER_REPORTS", 0), reports = 0;
 	int want_workers = 1, smooth_iir = 0, shuffle = 0, devices[MAX_WORKERS];
@@ -284,7 +286,7 @@ int main(int argc, char **argv)
 	struct sigaction sa;
 
 	memset(&ws, 0, sizeof(ws));
-	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POhTD:R:K:")) != -1) {
+	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POGhTD:R:K:")) != -1) {
 		switch (opt) {
 		case 'f': range = optarg; break;
 		case 'i': interval = (int)round(rp_atoft(optarg)); break;
@@ -294,6 +296,7 @@ int main(int argc, char **argv)
 		case 'F': boxcar = 0; comp_fir_size = atoi(optarg); break;
 		case '1': single = 1; break;
 		case 'P': peak_hold = 1; break;
+		case 'G': guard_bits = 1; break;                         /* RTLSDR_GPU_FLAG_GUARD_BITS */
 		case 's': smooth_iir = strcmp("iir", optarg) == 0; break; /* avg | iir, rtl_power.c:820-825 */
 		case 't': want_workers = atoi(optarg); break;             /* rtl_power.c:844-846 */
 		case 'K': sk_filename = optarg; break;
@@ -410,7 +413,8 @@ int main(int argc, char **argv)
 	cfg.rate = plan->rate;
 	cfg.crop = plan->crop;
 	cfg.window_coefs = window_coefs;
-	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS | (skf ? RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS : 0u);
+	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS | (skf ? RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS : 0u) |
+		    (guard_bits ? RTLSDR_GPU_FLAG_GUARD_BITS : 0u);
 	if (smooth_iir) {
 		const char *a = getenv("RTL_POWER_IIR_ALPHA");
 		cfg.iir_alpha = (a && *a) ? atof(a) : 0.25;

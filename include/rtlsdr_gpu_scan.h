@@ -130,6 +130,21 @@ typedef struct rtlsdr_gpu_scan_cfg {
  * RTLSDR_GPU_ERR_CONFIG (they do not carry S2): use collect_sk_device() and merge_sk_device(), which do, and
  * collect_sk_csv() / format_sk_csv_device() for the SK rows' text.  Every other collect also zeroes S2. */
 #define RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS 8u
+/* cfg.flags: fix_fft with 8 fractional guard bits.  The reference's transform halves and rounds to int16 at each of
+ * its log2 N stages, so its output is X/N in whole LSBs with rounding noise from every stage, which sets the noise
+ * floor of fine-resolution scans.  With this flag the front end is unchanged (u8 - 127, decimators, remove_dc, the
+ * wrapping int16 window multiply give x), the data enters the transform as v = x << 8 in int32, and every stage keeps
+ * fix_fft's bit reversal, halved Q15 twiddles, halving and FIX_MPY rounding R(p) = (p + 2^14) >> 15, applied to the
+ * exact product: t = (R(wr br) - R(wi bi), R(wr bi) + R(wi br)), q = a >> 1, a' = q + t, b' = q - t.  Every value
+ * stays below 2^24, so int32 never wraps.  Per block and bin pw = (re^2 + im^2 + 2^7) >> 8 < 2^40 (exact): the bins
+ * add it (peak_hold keeps the maximum) and SK adds pw^2 < 2^80 to S2, so the int64 bins are exact for at least 2^23
+ * FFT blocks per interval and hop (the reference's int16 path allows 2^32).  The bins therefore carry 2^8 times the
+ * reference's power scale; the dB rows take v = (double)avg * 2^-8 (exact), then the reference's v /= rate,
+ * v /= samples, 10*log10(v), so a strong tone reads the same dB with and without the flag while the lowest non-zero
+ * value drops by about 24 dB (dB values lie in (-211, 190), still within the CSV formatter's 7 characters).  SK is
+ * scale-invariant: its rows have the same meaning.  Combines with every other flag and option; RTLSDR_GPU_ERR_CONFIG
+ * at init with bin_e = 0 (the rms path has no transform). */
+#define RTLSDR_GPU_FLAG_GUARD_BITS 16u
 
 /* ---- lifecycle --------------------------------------------------------- */
 

@@ -16,6 +16,7 @@
 #include "scan_host.cuh"
 #include "scan_kernels.cuh"
 #include "scan_large.cuh"
+#include "scan_guard.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -972,6 +973,111 @@ int run_decimators(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_o
 	return check_launch(h, "dc_finalize_kernel");
 }
 
+/* RTLSDR_GPU_FLAG_GUARD_BITS (scan_guard.cuh): entries [0, n_reads), `chunk` at a time.  The front end's constants
+ * come from the existing kernels -- dc_sums_u8_kernel for u8 reads, run_decimators() for decimated images -- then
+ * guard_fft_a_kernel, and for N > 4096 guard_fft_b_kernel.  Scratch per chunk:
+ *   [N > 4096: transform chunk x N int2][sums chunk x 2 int64][tickets chunk x 8 B][consts chunk x int2][decimation] */
+template <int MODE>
+int guard_launch(rtlsdr_gpu_scan *h, const GuardParams &p, bool in16, int items)
+{
+	const int grid_a = std::max(1, std::min(items, h->num_sms * 8));
+	if (in16)
+		guard_fft_a_kernel<true, MODE><<<grid_a, kThreads, 0, h->stream>>>(p);
+	else
+		guard_fft_a_kernel<false, MODE><<<grid_a, kThreads, 0, h->stream>>>(p);
+	if (int rc = check_launch(h, "guard_fft_a_kernel"))
+		return rc;
+	if (p.L <= 12)
+		return 0;
+	guard_fft_b_kernel<MODE><<<dim3(1u << (p.L - 12), p.b_groups), kThreads, 0, h->stream>>>(p);
+	return check_launch(h, "guard_fft_b_kernel");
+}
+
+int guard_process(rtlsdr_gpu_scan *h, const uint8_t *base, const long long *d_offs, const int *d_hops, int n_reads)
+{
+	const int L = h->cfg.bin_e;
+	const size_t N = (size_t)1 << L;
+	const bool decim = (h->cfg.boxcar && h->cfg.downsample > 1) || h->cfg.downsample_passes > 0;
+	const size_t data = L > 12 ? N * 8 : 0;
+	const size_t per = data + 32 + (decim ? DecimScratch::per_entry(h) : 0);
+	const size_t extra = decim ? DecimScratch::slack() + 512 : 512;
+	/* (the DC and decimator kernels take one grid row per read: at most 65535) */
+	const int chunk_max = (int)std::max<size_t>(1, std::min<size_t>(65535, kScratchBudget / per));
+	const long long span = L <= 12 ? (long long)h->shape.n_blocks * (long long)N : (long long)N;
+	const int wpr = (int)((span + kWS - 1) / kWS);
+	h->last_was_epilogue = false;
+	int rc;
+	for (int e0 = 0; e0 < n_reads; e0 += chunk_max) {
+		const int cnt = std::min(chunk_max, n_reads - e0);
+		if ((rc = ensure_scratch(h, per * (size_t)cnt + extra)))
+			return rc;
+		uint8_t *sp = h->d_scratch;
+		int2 *xf = (int2 *)sp;
+		sp += (size_t)cnt * data;
+		long long *sums = (long long *)sp;
+		sp += (size_t)cnt * 16;
+		unsigned *tickets = (unsigned *)sp;
+		sp += (size_t)cnt * 8;
+		int2 *consts = (int2 *)sp;
+		sp += (size_t)cnt * 8;
+
+		GuardParams p;
+		memset(&p, 0, sizeof(p));
+		p.entry_base = e0;
+		p.n_entries = cnt;
+		p.hop_of = d_hops;
+		p.n_blocks = h->shape.n_blocks;
+		p.L = L;
+		p.tw = h->d_tw;
+		p.win = h->d_win;
+		p.scratch = xf;
+		p.avg = h->d_avg;
+		p.samples = h->d_smp64;
+		p.samples_per_read = h->shape.samples_per_read;
+		p.s2 = h->d_s2;
+		/* round B: about four CTAs per SM in all */
+		p.b_groups = L > 12 ? std::max(1, std::min(cnt, (4 * h->num_sms + (1 << (L - 12)) - 1) >> (L - 12))) : 1;
+		if (!decim) {
+			CU(cudaMemsetAsync(sums, 0, (size_t)cnt * 24, h->stream));
+			DcSumU8Params d;
+			d.base = base;
+			d.read_off = d_offs;
+			d.entry_base = e0;
+			d.buf_len = h->cfg.buf_len;
+			d.sums = sums;
+			d.tickets = tickets;
+			d.consts = consts;
+			const unsigned per_read =
+				(unsigned)std::max<size_t>(1, std::min<size_t>(32, (size_t)h->cfg.buf_len / (256 * 16 * 8)));
+			dc_sums_u8_kernel<<<dim3(per_read, (unsigned)cnt), 256, 0, h->stream>>>(d);
+			if ((rc = check_launch(h, "dc_sums_u8_kernel")))
+				return rc;
+			p.base = base;
+			p.read_off = d_offs;
+			p.dc_u8 = consts;
+		} else {
+			DecimScratch sc(h, cnt, (uint8_t *)(((uintptr_t)sp + 255) & ~(uintptr_t)255));
+			if ((rc = run_decimators(h, base, d_offs + e0, cnt, sc)))
+				return rc;
+			p.base = (const uint8_t *)sc.img;
+			p.regular_stride = h->shape.image_stride * 4;
+			p.dc_ave = sc.ave;
+			p.l_len = h->shape.l_len;
+			p.blocks_padded = h->shape.blocks_padded;
+		}
+		const int items = (int)std::min<long long>((long long)cnt * wpr, 1ll << 30);
+		if (h->d_s2)
+			rc = guard_launch<GUARD_SK>(h, p, decim, items);
+		else if (h->cfg.peak_hold)
+			rc = guard_launch<GUARD_PEAK>(h, p, decim, items);
+		else
+			rc = guard_launch<GUARD_SUM>(h, p, decim, items);
+		if (rc)
+			return rc;
+	}
+	return 0;
+}
+
 /*
  * Process one batch of reads already on the device.  `d_desc` holds the
  * descriptor blob (sorted read offsets, segments, hop per read).
@@ -1026,6 +1132,11 @@ int launch_batch(rtlsdr_gpu_scan *h, const uint8_t *base, const uint8_t *d_desc,
 		if ((rc = launch_after_epilogue(h, rms_kernel, blocks, 256, 0, p)))
 			return rc;
 		return check_launch(h, "rms_kernel");
+	}
+
+	if (h->cfg.flags & RTLSDR_GPU_FLAG_GUARD_BITS) {
+		TimedScope ts(h);
+		return guard_process(h, base, d_offs, d_hops, n_reads);
 	}
 
 	if (h->shape.path == PATH_SMALL_U8) {
@@ -1352,7 +1463,10 @@ int run_epilogue(rtlsdr_gpu_scan *h, int hop0, int nhops, double *db, long long 
 	p.iir_alpha = h->cfg.iir_alpha;
 	const int span = std::max(h->shape.db_count, avg_out ? h->shape.N : 0);
 	dim3 grid((span + 255) / 256, nhops);
-	epilogue_kernel<<<grid, 256, 0, h->stream>>>(p);
+	if (h->cfg.flags & RTLSDR_GPU_FLAG_GUARD_BITS)
+		epilogue_guard_kernel<<<grid, 256, 0, h->stream>>>(p);
+	else
+		epilogue_kernel<<<grid, 256, 0, h->stream>>>(p);
 	h->last_was_epilogue = zero_after; /* nothing else follows it on the stream in the fused-zero case */
 	return check_launch(h, "epilogue_kernel");
 }

@@ -2385,75 +2385,30 @@ struct EpilogueParams {
 	double iir_alpha;
 };
 
+/* the bin as the dB chain's first double: (double)avg, times 2^-8 (exact) for guard-bit bins */
+template <bool GUARD>
+SCAN_DEV double epilogue_value(long long v)
+{
+	if constexpr (GUARD)
+		return __dmul_rn((double)v, 0x1p-8);
+	else
+		return (double)v;
+}
+
 /* one launch per report: dB row, raw-bin copy and sample count of every hop */
 __global__ void __launch_bounds__(256)
 epilogue_kernel(const SCAN_GRID_CONSTANT EpilogueParams prm)
 {
-	pdl_launch_dependents(); /* the next interval's transform may start; it waits before its flush */
-	const int hop = prm.hop0 + blockIdx.y;
-	const int n = 1 << prm.bin_e;
-	const int count = prm.i2 - prm.i1 + 2;
-	const int k = blockIdx.x * blockDim.x + threadIdx.x;
-	const long long *a = prm.avg + ((long long)hop << prm.bin_e);
-	if (prm.avg_out && k < n)
-		prm.avg_out[((long long)blockIdx.y << prm.bin_e) + k] = a[k];
-	if (prm.samples_out && k == 0)
-		prm.samples_out[blockIdx.y] = (int)prm.samples[hop];
-	if (k < count && prm.db) {
-	const int i = (k < count - 1) ? prm.i1 + k : prm.i2;
-	long long v;
-	if (prm.bin_e > 0) {
-		const int j = (i + n / 2) & (n - 1); /* undo the half swap */
-		v = a[j == 0 ? 1 : j];               /* avg[0] = avg[1] */
-	} else {
-		v = a[0];
-	}
-	const double rate = (double)prm.rate, smp = (double)(int)prm.samples[hop];
-	double d;
-	if (k < count - 1)
-		d = __ddiv_rn(__ddiv_rn((double)v, rate), smp);
-	else
-		d = __ddiv_rn((double)v, __dmul_rn(rate, smp));
-	if (!prm.iir) {
-		prm.db[(long long)blockIdx.y * count + k] = 10 * log10(d);
-	} else if (k < count - 1) {
-		/* -s iir (parsed, never implemented by the reference, rtl_power.c:820-825 and its TODO list :29-36):
-		 * exponential smoothing ACROSS reports of the linear value csv_dbm takes the logarithm of,
-		 *   s = d for a bin's first report, s += alpha * (d - s) afterwards (reports without samples skip it);
-		 * the duplicated last column (rtl_power.c:755-760) prints the same smoothed bin again */
-		double *st = prm.iir + (long long)hop * (count - 1) + k;
-		double sm = *st;
-		if (smp != 0.0) {
-			sm = (sm != sm) ? d : __dadd_rn(sm, __dmul_rn(prm.iir_alpha, __dadd_rn(d, -sm)));
-			*st = sm;
-		} else {
-			sm = d;
-		}
-		const double o = 10 * log10(sm);
-		prm.db[(long long)blockIdx.y * count + k] = o;
-		if (k == count - 2)
-			prm.db[(long long)blockIdx.y * count + k + 1] = o;
-	}
-	}
-	/* read-and-zero (rtl_power.c:761-764): the last block of a hop to finish clears its
-	 * bins and sample counter, so no separate memset has to follow the report */
-	if (prm.done) {
-		__shared__ unsigned ticket;
-		__threadfence();
-		__syncthreads();
-		if (threadIdx.x == 0)
-			ticket = atomicAdd(prm.done + hop, 1u);
-		__syncthreads();
-		if (ticket == gridDim.x - 1) {
-			long long *z = prm.avg_rw + ((long long)hop << prm.bin_e);
-			for (int j = threadIdx.x; j < n; j += blockDim.x)
-				z[j] = 0;
-			if (threadIdx.x == 0) {
-				prm.samples_rw[hop] = 0;
-				prm.done[hop] = 0;
-			}
-		}
-	}
+	constexpr bool GUARD = false;
+#include "epilogue_body.inl"
+}
+
+/* the same for a RTLSDR_GPU_FLAG_GUARD_BITS handle */
+__global__ void __launch_bounds__(256)
+epilogue_guard_kernel(const SCAN_GRID_CONSTANT EpilogueParams prm)
+{
+	constexpr bool GUARD = true;
+#include "epilogue_body.inl"
 }
 
 /* ======================================================================== *

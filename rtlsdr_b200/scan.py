@@ -168,7 +168,7 @@ class GpuScan:
     def __init__(self, tune_count, bin_e, buf_len, downsample=1, downsample_passes=0, boxcar=1,
                  comp_fir_size=0, peak_hold=0, rate=2400000, crop=0.0, window_coefs=None,
                  sinewave=None, device=0, ring_bytes=0, level_stats=False, iir_alpha=0.0, async_report=False,
-                 short_reads=False, spectral_kurtosis=False):
+                 short_reads=False, spectral_kurtosis=False, guard_bits=False):
         self.lib = load_library()
         self.tune_count, self.bin_e, self.buf_len = tune_count, bin_e, buf_len
         self.n = 1 << bin_e
@@ -188,9 +188,9 @@ class GpuScan:
             self._s = np.ascontiguousarray(sinewave, dtype=np.int16)
             cfg.sinewave = self._s.ctypes.data
         cfg.ring_bytes = ring_bytes
-        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS / _SPECTRAL_KURTOSIS
+        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS / _SPECTRAL_KURTOSIS / _GUARD_BITS
         cfg.flags = ((1 if level_stats else 0) | (2 if async_report else 0) | (4 if short_reads else 0)
-                     | (8 if spectral_kurtosis else 0))
+                     | (8 if spectral_kurtosis else 0) | (16 if guard_bits else 0))
         cfg.iir_alpha = iir_alpha            # -s iir smoothing of the dB rows across reports (0 = off)
         self.h = ctypes.c_void_p()
         rc = self.lib.rtlsdr_gpu_scan_init(ctypes.byref(cfg), ctypes.byref(self.h))

@@ -56,6 +56,9 @@ def main(argv=None):
     ap.add_argument("--device", type=int, default=None, help="CUDA device of this rank (default: LOCAL_RANK)")
     ap.add_argument("--sk", dest="sk_out", default=None, metavar="FILE",
                     help="also write each bin's spectral kurtosis to FILE (rows like the power rows, %%.4f values)")
+    ap.add_argument("--guard-bits", action="store_true",
+                    help="fix_fft with 8 fractional guard bits (RTLSDR_GPU_FLAG_GUARD_BITS): the transform rounds "
+                         "2^8 below the reference's LSB, so fine-resolution rows show the signal's noise floor")
     ap.add_argument("-o", dest="out", default="-")
     args = ap.parse_args(argv)
     if args.sk_out is not None and args.peak:
@@ -88,6 +91,8 @@ def main(argv=None):
     sk = args.sk_out is not None
     if sk and pd["bin_e"] == 0:
         raise SystemExit("sweep_main: --sk needs FFT bins; this scan's hops are 1-bin (rms) power readings")
+    if args.guard_bits and pd["bin_e"] == 0:
+        raise SystemExit("sweep_main: --guard-bits needs FFT bins; this scan's hops are 1-bin (rms) power readings")
     tc, b, n = pd["tune_count"], pd["buf_len"], 1 << pd["bin_e"]
     mine = shard_hops(tc, world, rank)
     mode = ["xorshift", "counter", "const", "biased", "tone"].index(args.synth)
@@ -98,7 +103,8 @@ def main(argv=None):
     g = None
     if len(mine):
         window = rs.window_coefs(args.window, n) if pd["bin_e"] else None
-        g = rs.GpuScan.from_plan(pd, window_coefs=window, device=local, hops=list(mine), spectral_kurtosis=sk)
+        g = rs.GpuScan.from_plan(pd, window_coefs=window, device=local, hops=list(mine), spectral_kurtosis=sk,
+                                 guard_bits=args.guard_bits)
     db_count = g.db_count if g else plan.db_count
     gather = SpectrumGather(tc, n, db_count, world, rank, torch.device("cuda", local),
                             mode=("host" if args.backend == "gloo" and world > 1 else None), sk=sk)
@@ -231,7 +237,8 @@ def _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch
     sweeps = shard_hops(args.sweeps, world, rank)            # the same balanced split, over sweeps
     window = rs.window_coefs(args.window, n) if pd["bin_e"] else None
     sk = args.sk_out is not None
-    g = rs.GpuScan.from_plan(pd, window_coefs=window, device=local, spectral_kurtosis=sk)
+    g = rs.GpuScan.from_plan(pd, window_coefs=window, device=local, spectral_kurtosis=sk,
+                             guard_bits=args.guard_bits)
     gather = SpectrumGather(tc, n, g.db_count, world, rank, torch.device("cuda", local),
                             mode=("host" if args.backend == "gloo" and world > 1 else None), replicated=True, sk=sk)
     if rank == 0 and world > 1:
