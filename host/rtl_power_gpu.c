@@ -89,6 +89,12 @@ static void print_usage(void)
 		"\t[-R seed (visit the hops of every sweep in a random order)]\n"
 		"\t[-K sk_file (also write each bin's spectral kurtosis: rows like the power rows, %%.4f values,\n"
 		"\t\t~1 for noise, > 1 for intermittent signals, < 1 for steady carriers; not with -P)]\n"
+		"\t[-X excised_file (spectral-kurtosis RFI excision: every sub-integration of a bin whose SK lies outside\n"
+		"\t\tthe thresholds is left out of that bin's average; rows like the power rows, the folded samples as count;\n"
+		"\t\tnot with -P, 1-bin hops or more workers than hops)]\n"
+		"\t[-Y flag_file (with -X: the flagged fraction of every bin's sub-integrations, %%.4f values)]\n"
+		"\t[-M sweeps (with -X: sweeps per sub-integration; default: the fewest giving every hop 64 FFT blocks)]\n"
+		"\t[-k low[:high] (with -X: thresholds 1 - low*sigma and 1 + high*sigma, default 3:3; inf never flags)]\n"
 		"\tfilename (a '-' dumps samples to stdout, the default)\n");
 	exit(1);
 }
@@ -260,6 +266,9 @@ static int device_list(int workers, int *devices)
 int main(int argc, char **argv)
 {
 	const char *range = NULL, *window = "rectangle", *filename = "-", *sk_filename = NULL;
+	const char *x_filename = NULL, *y_filename = NULL;
+	int excise_sweeps = 0, since_fold = 0;
+	double k_low = 3.0, k_high = 3.0;
 	const char *fixed_stamp = getenv("RTL_POWER_TIMESTAMP");
 	int opt, interval = 10, single = 0, peak_hold = 0, boxcar = 1, comp_fir_size = 0;
 	int guard_bits = 0;
@@ -280,13 +289,13 @@ int main(int argc, char **argv)
 	int32_t *window_coefs = NULL;
 	uint8_t *buf8, *replay = NULL;
 	int *order;
-	char *text, *sk_text = NULL, stamp[80];
-	size_t text_cap = 0, text_len = 0, sk_cap = 0, sk_len = 0;
-	FILE *out, *skf = NULL;
+	char *text, *sk_text = NULL, *x_text = NULL, *y_text = NULL, stamp[80];
+	size_t text_cap = 0, text_len = 0, sk_cap = 0, sk_len = 0, x_len = 0, y_len = 0;
+	FILE *out, *skf = NULL, *xf = NULL, *yf = NULL;
 	struct sigaction sa;
 
 	memset(&ws, 0, sizeof(ws));
-	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POGhTD:R:K:")) != -1) {
+	while ((opt = getopt(argc, argv, "f:i:s:t:d:g:p:e:w:c:F:1POGhTD:R:K:X:Y:M:k:")) != -1) {
 		switch (opt) {
 		case 'f': range = optarg; break;
 		case 'i': interval = (int)round(rp_atoft(optarg)); break;
@@ -300,6 +309,15 @@ int main(int argc, char **argv)
 		case 's': smooth_iir = strcmp("iir", optarg) == 0; break; /* avg | iir, rtl_power.c:820-825 */
 		case 't': want_workers = atoi(optarg); break;             /* rtl_power.c:844-846 */
 		case 'K': sk_filename = optarg; break;
+		case 'X': x_filename = optarg; break;                   /* RTLSDR_GPU_FLAG_SK_EXCISION */
+		case 'Y': y_filename = optarg; break;
+		case 'M': excise_sweeps = atoi(optarg); break;
+		case 'k': {
+			char *end;
+			k_low = strtod(optarg, &end);
+			k_high = *end == ':' ? strtod(end + 1, NULL) : k_low;
+			break;
+		}
 		case 'R': shuffle = 1; shuffle_state = 0x9E3779B97F4A7C15ULL ^ (uint64_t)strtoull(optarg, NULL, 0); break;
 		case 'd': case 'g': case 'p': case 'O': case 'T': case 'D':
 			break; /* device housekeeping: no dongle behind the synthetic source */
@@ -390,6 +408,27 @@ int main(int argc, char **argv)
 		fprintf(stderr, "-K: the spectral kurtosis needs all reads of a hop on one worker (fewer hops than workers).\n");
 		return 1;
 	}
+	if (y_filename && !x_filename) {
+		fprintf(stderr, "-Y needs -X.\n");
+		return 1;
+	}
+	if (x_filename && (peak_hold || plan->bin_e == 0 || ws.by_pass)) {
+		fprintf(stderr, "-X: excision needs sums of FFT powers (not -P, not 1-bin hops) and all reads of a hop on one "
+				"worker (not more workers than hops).\n");
+		return 1;
+	}
+	if (x_filename && (!(k_low >= 0.0) || !(k_high >= 0.0))) {
+		fprintf(stderr, "-k: thresholds must be >= 0.\n");
+		return 1;
+	}
+	if (x_filename) {
+		xf = fopen(x_filename, "wb");
+		yf = y_filename ? fopen(y_filename, "wb") : NULL;
+		if (!xf || (y_filename && !yf)) {
+			fprintf(stderr, "Failed to open %s\n", !xf ? x_filename : y_filename);
+			return 1;
+		}
+	}
 	if (sk_filename) {
 		skf = fopen(sk_filename, "wb");
 		if (!skf) {
@@ -413,8 +452,8 @@ int main(int argc, char **argv)
 	cfg.rate = plan->rate;
 	cfg.crop = plan->crop;
 	cfg.window_coefs = window_coefs;
-	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS | (skf ? RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS : 0u) |
-		    (guard_bits ? RTLSDR_GPU_FLAG_GUARD_BITS : 0u);
+	cfg.flags = RTLSDR_GPU_FLAG_SHORT_READS | (skf || xf ? RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS : 0u) |
+		    (guard_bits ? RTLSDR_GPU_FLAG_GUARD_BITS : 0u) | (xf ? RTLSDR_GPU_FLAG_SK_EXCISION : 0u);
 	if (smooth_iir) {
 		const char *a = getenv("RTL_POWER_IIR_ALPHA");
 		cfg.iir_alpha = (a && *a) ? atof(a) : 0.25;
@@ -432,8 +471,13 @@ int main(int argc, char **argv)
 		/* text buffer for the longest stamp this program prints */
 		if ((size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > text_cap)
 			text_cap = (size_t)rtlsdr_gpu_scan_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1);
-		if (skf && (size_t)rtlsdr_gpu_scan_sk_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > sk_cap)
+		if ((skf || yf) && (size_t)rtlsdr_gpu_scan_sk_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1) > sk_cap)
 			sk_cap = (size_t)rtlsdr_gpu_scan_sk_csv_capacity(ws.gpu[w], cfg.tune_count, sizeof(stamp) - 1);
+	}
+	if (xf && excise_sweeps <= 0) {
+		/* the fewest sweeps giving every hop 64 FFT blocks per sub-integration (one read per hop and sweep) */
+		const int blocks = rtlsdr_gpu_scan_blocks_per_read(ws.gpu[0]);
+		excise_sweeps = (64 + blocks - 1) / blocks;
 	}
 	if (ws.count > 1 && ws.by_pass)
 		fprintf(stderr, "GPU workers: %d (all %d hops each, every %d-th sweep; accumulators merged per report)\n",
@@ -456,8 +500,12 @@ int main(int argc, char **argv)
 	text = (char *)rtlsdr_gpu_scan_host_alloc(text_cap);
 	if (skf)
 		sk_text = (char *)rtlsdr_gpu_scan_host_alloc(sk_cap);
+	if (xf)
+		x_text = (char *)rtlsdr_gpu_scan_host_alloc(text_cap);
+	if (yf)
+		y_text = (char *)rtlsdr_gpu_scan_host_alloc(sk_cap);
 	order = (int *)malloc(sizeof(int) * (size_t)plan->tune_count);
-	if (!buf8 || !text || (skf && !sk_text) || !order) {
+	if (!buf8 || !text || (skf && !sk_text) || (xf && !x_text) || (yf && !y_text) || !order) {
 		fprintf(stderr, "Out of memory.\n");
 		return 1;
 	}
@@ -473,9 +521,27 @@ int main(int argc, char **argv)
 		if (rc)
 			break;
 		passes++;
+		/* -X: a sub-integration closes every excise_sweeps sweeps, and the rest of one before each report */
+		since_fold++;
+		if (xf && since_fold == excise_sweeps) {
+			for (w = 0; w < ws.count && !rc; w++)
+				rc = rtlsdr_gpu_scan_excise_fold(ws.gpu[w], k_low, k_high);
+			since_fold = 0;
+			if (rc) {
+				fprintf(stderr, "rtlsdr_gpu_scan_excise_fold: %s\n", rtlsdr_gpu_scan_strerror(rc));
+				break;
+			}
+		}
 		now = time(NULL);
 		if (passes_per_report ? (passes % passes_per_report) != 0 : now < next_tick)
 			continue;
+		for (w = 0; xf && since_fold && w < ws.count && !rc; w++)
+			rc = rtlsdr_gpu_scan_excise_fold(ws.gpu[w], k_low, k_high);
+		since_fold = 0;
+		if (rc) {
+			fprintf(stderr, "rtlsdr_gpu_scan_excise_fold: %s\n", rtlsdr_gpu_scan_strerror(rc));
+			break;
+		}
 		if (fixed_stamp) {
 			snprintf(stamp, sizeof(stamp) - 2, "%s", fixed_stamp);
 		} else {
@@ -504,6 +570,18 @@ int main(int argc, char **argv)
 		}
 		/* -K: the SK rows are formatted beside the power rows, with the same read-and-zero */
 		for (w = 0; w < ws.count && !rc && !ws.by_pass; w++) {
+			/* -X / -Y: the excised report is a peek, so it goes before the worker's read-and-zero */
+			if (xf) {
+				rc = rtlsdr_gpu_scan_excised_csv(ws.gpu[w], stamp, x_text, text_cap, &x_len, y_text, sk_cap, &y_len);
+				if (rc) {
+					fprintf(stderr, "rtlsdr_gpu_scan_excised_csv: %s (%s)\n", rtlsdr_gpu_scan_strerror(rc),
+						rtlsdr_gpu_scan_last_cuda_error(ws.gpu[w]));
+					break;
+				}
+				fwrite(x_text, 1, x_len, xf);
+				if (yf)
+					fwrite(y_text, 1, y_len, yf);
+			}
 			rc = skf ? rtlsdr_gpu_scan_collect_sk_csv(ws.gpu[w], stamp, text, text_cap, &text_len, sk_text, sk_cap,
 								  &sk_len)
 				 : rtlsdr_gpu_scan_collect_csv(ws.gpu[w], stamp, text, text_cap, &text_len);
@@ -519,6 +597,10 @@ int main(int argc, char **argv)
 		fflush(out);
 		if (skf)
 			fflush(skf);
+		if (xf)
+			fflush(xf);
+		if (yf)
+			fflush(yf);
 		if (rc)
 			break;
 		while (time(NULL) >= next_tick)
@@ -537,12 +619,18 @@ int main(int argc, char **argv)
 		fclose(out);
 	if (skf)
 		fclose(skf);
+	if (xf)
+		fclose(xf);
+	if (yf)
+		fclose(yf);
 	for (w = 0; w < ws.count; w++)
 		rtlsdr_gpu_scan_close(ws.gpu[w]);
 	rtlsdr_close(dev);
 	free(buf8);
 	rtlsdr_gpu_scan_host_free(text);
 	rtlsdr_gpu_scan_host_free(sk_text);
+	rtlsdr_gpu_scan_host_free(x_text);
+	rtlsdr_gpu_scan_host_free(y_text);
 	rtlsdr_gpu_scan_host_free(parts);
 	free(order);
 	free(window_coefs);

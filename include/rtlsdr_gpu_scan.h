@@ -145,6 +145,18 @@ typedef struct rtlsdr_gpu_scan_cfg {
  * scale-invariant: its rows have the same meaning.  Combines with every other flag and option; RTLSDR_GPU_ERR_CONFIG
  * at init with bin_e = 0 (the rms path has no transform). */
 #define RTLSDR_GPU_FLAG_GUARD_BITS 16u
+/* cfg.flags: spectral-kurtosis RFI excision (Nita & Gary 2010) on top of RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS, which it
+ * requires (RTLSDR_GPU_ERR_CONFIG at init without it, so every SK restriction applies).  The caller cuts the
+ * interval into sub-integrations with rtlsdr_gpu_scan_excise_fold(); a bin's sub-integration of M FFT blocks joins
+ * the bin's clean average only when its SK lies within [1 - k_low sigma(M), 1 + k_high sigma(M)], and
+ * rtlsdr_gpu_scan_excised_report() / _excised_report_device() / _excised_csv() report the clean average and the
+ * flagged fraction beside the unchanged power and SK reports.  The handle keeps 36 bytes per bin more (S1 and S2 at
+ * the last fold, the clean power sum int64 and the clean block count int32) and the sample counter of every hop at
+ * its last fold.  Every read-and-zero (collect, collect_all, collect_sk, collect_csv, collect_sk_csv,
+ * collect_sk_device) also zeroes this state for the hops it zeroes; reads submitted after the last fold count in the
+ * ordinary rows only, so a driver folds once more before it reports.  merge_device() and merge_sk_device() return
+ * RTLSDR_GPU_ERR_CONFIG on such a handle: merged reads would land in one sub-integration. */
+#define RTLSDR_GPU_FLAG_SK_EXCISION 32u
 
 /* ---- lifecycle --------------------------------------------------------- */
 
@@ -353,6 +365,53 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_format_sk_csv_device(rtlsdr_gpu_scan_t *h, co
 RTLSDR_GPU_API int rtlsdr_gpu_scan_collect_sk_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap,
 		size_t *len, char *sk_text, size_t sk_cap, size_t *sk_len);
 
+/* ---- spectral-kurtosis RFI excision (RTLSDR_GPU_FLAG_SK_EXCISION) ------ */
+
+/*
+ * Close a sub-integration of every hop.  For hop h and bin j (natural FFT order):
+ *   M = (samples[h] - snap_smp[h]) / downsample   FFT blocks since the last fold (exact: each block adds downsample)
+ *   dS1 = S1 - snapS1, dS2 = S2 - snapS2          (an exact 128-bit difference)
+ *   sk = SK of (dS1, dS2, M)                     as collect_sk() evaluates it (rtlsdr_b200/csrc/sk.cuh)
+ *   sigma = sqrt(4 M^2 / ((M-1)(M+2)(M+3)))      the estimator's standard deviation for single-block power,
+ *                                                correctly rounded IEEE steps in a fixed order (sk_sigma())
+ *   flagged iff sk is not NaN and (sk < 1 - k_low sigma or sk > 1 + k_high sigma); otherwise the bin is clean:
+ *   C1 += dS1, B1 += M.  M < 2 and dS1 = 0 never flag.  Then snapS1 = S1, snapS2 = S2, snap_smp = samples.
+ * k_low, k_high >= 0, +inf never flags that side (k_low = +inf keeps steady carriers); NaN or a negative value is
+ * RTLSDR_GPU_ERR_CONFIG, as is a handle without the flag.  Flushes the staging ring first, then runs asynchronously
+ * on the handle's stream.
+ */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_excise_fold(rtlsdr_gpu_scan_t *h, double k_low, double k_high);
+
+/*
+ * The excised report of every hop, a peek (nothing is zeroed); blocks until it is in host memory.  Any pointer may
+ * be NULL:
+ *   clean_avg      int64 [tune_count << bin_e]  C1, natural FFT order like collect()'s avg
+ *   clean_blocks   int32 [tune_count << bin_e]  B1
+ *   folded_samples int32 [tune_count]           the sample counter at the last fold (snap_smp)
+ *   db     double [tune_count * db_count] the dB row's layout -- bin 0 takes bin 1's (C1, B1) (csv_dbm's DC nuke),
+ *          half swap, crop, duplicate of bin i2 -- with collect()'s expressions and the hop's sample count replaced
+ *          by the bin's clean samples s = B1 * downsample: 10 log10(C1 / rate / s), the duplicate
+ *          10 log10(C1 / (rate * s)) (guard-bit bins scaled by 2^-8 first); a quiet NaN (sign bit clear) when
+ *          B1 = 0.  Never smoothed by iir_alpha.
+ *   flagged double [tune_count * db_count] same layout: (F - B1) / F, F = folded_samples / downsample the folded FFT
+ *          blocks, in [0, 1]; NaN when F = 0.
+ * RTLSDR_GPU_ERR_CONFIG on a handle without RTLSDR_GPU_FLAG_SK_EXCISION.
+ */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_excised_report(rtlsdr_gpu_scan_t *h, int64_t *clean_avg, int32_t *clean_blocks,
+		int32_t *folded_samples, double *db, double *flagged);
+/* The dB rows (dev_db, double [tune_count][db_count]), flag fractions (dev_flagged, same shape) and folded samples
+ * (dev_samples, int32 [tune_count]) of excised_report() into device memory, which may be a peer mapping; any pointer
+ * may be NULL.  Asynchronous on the handle's stream.  RTLSDR_GPU_ERR_ALIGN for a misaligned pointer. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_excised_report_device(rtlsdr_gpu_scan_t *h, void *dev_db, void *dev_flagged,
+		void *dev_samples);
+/* The excised report as text, formatted on the GPU (a peek: nothing is zeroed): the excised dB rows like
+ * collect_csv() prints power rows (cap >= csv_capacity(tune_count)) into `text`, and when flag_text is not NULL the
+ * flag fractions printed "%.4f" like collect_sk_csv() prints SK rows (flag_cap >= sk_csv_capacity(tune_count)) into
+ * `flag_text`.  The count column of both is the folded samples.  Needs the csv column table (set_csv_columns());
+ * only the text crosses PCIe; blocks until both texts are in host memory. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_excised_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap,
+		size_t *len, char *flag_text, size_t flag_cap, size_t *flag_len);
+
 /* ---- multi-GPU report hand-off ----------------------------------------- */
 
 /*
@@ -377,6 +436,9 @@ RTLSDR_GPU_API int rtlsdr_gpu_scan_flag_wait(void *cuda_stream, const void *dev_
 
 /* Number of doubles per hop that collect() writes to `db` (= i2 - i1 + 2). */
 RTLSDR_GPU_API int rtlsdr_gpu_scan_db_count(const rtlsdr_gpu_scan_t *h);
+/* FFT blocks one read adds to a hop (each adds `downsample` to its sample count, rtl_power.c:717): the M one read
+ * contributes to a sub-integration of rtlsdr_gpu_scan_excise_fold(); 1 for 1-bin (rms) hops. */
+RTLSDR_GPU_API int rtlsdr_gpu_scan_blocks_per_read(const rtlsdr_gpu_scan_t *h);
 /* Pinned host memory for submit_batch() and fast collect(). */
 RTLSDR_GPU_API void *rtlsdr_gpu_scan_host_alloc(size_t bytes);
 RTLSDR_GPU_API void rtlsdr_gpu_scan_host_free(void *p);

@@ -17,6 +17,7 @@
 #include "scan_kernels.cuh"
 #include "scan_large.cuh"
 #include "scan_guard.cuh"
+#include "excise.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -83,6 +84,12 @@ struct rtlsdr_gpu_scan {
 	unsigned long long *d_level = nullptr; /* [tune_count][2] soft-AGC byte counts (optional) */
 	unsigned long long *d_s2 = nullptr;    /* RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS: [tune_count * N][2] sum pw^2 (lo, hi) */
 	double *d_sk = nullptr;                /* [tune_count][db_count] SK rows of collect_sk() */
+	/* RTLSDR_GPU_FLAG_SK_EXCISION (excise.cuh), one allocation at d_exc_s2: snapS2 [tune_count * N][2], snapS1,
+	 * C1 (int64) [tune_count * N], snap_smp (int64) [tune_count], B1 (int32) [tune_count * N], tickets [tune_count] */
+	unsigned long long *d_exc_s2 = nullptr;
+	long long *d_exc_s1 = nullptr, *d_exc_c1 = nullptr, *d_exc_smp = nullptr;
+	int *d_exc_b1 = nullptr;
+	unsigned *d_exc_ticket = nullptr;
 	std::vector<uint64_t> level_bytes;
 	int2 *d_tw = nullptr;
 	int2 *d_twc = nullptr;          /* small path: per-stage compact twiddles (shared-memory image); large path: round A's */
@@ -1371,6 +1378,7 @@ void free_all(rtlsdr_gpu_scan *h)
 	cudaFree(h->d_level);
 	cudaFree(h->d_s2);
 	cudaFree(h->d_sk);
+	cudaFree(h->d_exc_s2);
 	cudaFree(h->d_done);
 	cudaFree(h->d_twb);
 	cudaFree(h->d_twc);
@@ -1541,6 +1549,66 @@ int run_sk_report(rtlsdr_gpu_scan *h, double *sk)
 	return check_launch(h, "sk_report_kernel");
 }
 
+/* RTLSDR_GPU_FLAG_SK_EXCISION: the read-and-zero of hops [hop0, hop0 + nhops) also clears their excision state */
+int zero_excise(rtlsdr_gpu_scan *h, int hop0, int nhops)
+{
+	if (!h->d_exc_s2)
+		return 0;
+	const size_t N = (size_t)h->shape.N, a = (size_t)hop0 * N, n = (size_t)nhops * N;
+	h->last_was_epilogue = false;
+	if (nhops == h->cfg.tune_count) { /* snapS2, snapS1, C1 and snap_smp are contiguous, then B1 */
+		CU(cudaMemsetAsync(h->d_exc_s2, 0, (n * 4 + (size_t)nhops) * sizeof(long long), h->stream));
+	} else {
+		CU(cudaMemsetAsync(h->d_exc_s2 + 2 * a, 0, n * 2 * sizeof(unsigned long long), h->stream));
+		CU(cudaMemsetAsync(h->d_exc_s1 + a, 0, n * sizeof(long long), h->stream));
+		CU(cudaMemsetAsync(h->d_exc_c1 + a, 0, n * sizeof(long long), h->stream));
+		CU(cudaMemsetAsync(h->d_exc_smp + hop0, 0, (size_t)nhops * sizeof(long long), h->stream));
+	}
+	CU(cudaMemsetAsync(h->d_exc_b1 + a, 0, n * sizeof(int), h->stream));
+	return 0;
+}
+
+/* the excised report of every hop (excise.cuh) into any of its three destinations (device or peer memory) */
+int run_excised_report(rtlsdr_gpu_scan *h, int *samples_out, double *db, double *flagged)
+{
+	ExciseReportParams p;
+	p.c1 = h->d_exc_c1;
+	p.b1 = h->d_exc_b1;
+	p.snap_smp = h->d_exc_smp;
+	p.samples_out = samples_out;
+	p.db = db;
+	p.flagged = flagged;
+	p.bin_e = h->cfg.bin_e;
+	p.i1 = h->shape.db_i1;
+	p.i2 = h->shape.db_i2;
+	p.rate = h->cfg.rate;
+	p.downsample = h->cfg.downsample;
+	const dim3 grid((h->shape.db_count + 255) / 256, h->cfg.tune_count);
+	h->last_was_epilogue = false;
+	if (h->cfg.flags & RTLSDR_GPU_FLAG_GUARD_BITS)
+		excised_report_kernel<true><<<grid, 256, 0, h->stream>>>(p);
+	else
+		excised_report_kernel<false><<<grid, 256, 0, h->stream>>>(p);
+	return check_launch(h, "excised_report_kernel");
+}
+
+/* the device text buffer of collect_text() / excised_csv() and its two lengths, grown to `bytes` */
+int ensure_csv_text(rtlsdr_gpu_scan *h, size_t bytes)
+{
+	if (!h->d_csv_len) { /* [0] the power text's length, [1] the SK text's */
+		CU(cudaMalloc(&h->d_csv_len, 2 * sizeof(long long)));
+		CU(cudaMallocHost(&h->h_csv_len, 2 * sizeof(long long)));
+	}
+	if (bytes > h->csv_text_bytes) {
+		cudaFree(h->d_csv_text);
+		h->d_csv_text = nullptr;
+		h->csv_text_bytes = 0;
+		CU(cudaMalloc(&h->d_csv_text, bytes));
+		h->csv_text_bytes = bytes;
+	}
+	return 0;
+}
+
 } // namespace
 
 /* large-FFT path needs the handle definition */
@@ -1703,6 +1771,17 @@ int rtlsdr_gpu_scan_init(const rtlsdr_gpu_scan_cfg_t *cfg_in, rtlsdr_gpu_scan_t 
 			if (!alloc_fill(&h->d_s2, (size_t)cfg->tune_count * N * 2 * sizeof(unsigned long long), 0, h->stream, &rc) ||
 			    !alloc_fill(&h->d_sk, (size_t)cfg->tune_count * h->shape.db_count * sizeof(double), 0, h->stream, &rc))
 				break;
+		}
+		if (cfg->flags & RTLSDR_GPU_FLAG_SK_EXCISION) { /* 36 B per bin, 12 B per hop (excise.cuh) */
+			const size_t n = (size_t)cfg->tune_count * N, tc = (size_t)cfg->tune_count;
+			if (!alloc_fill(&h->d_exc_s2, (n * 4 + tc) * sizeof(long long) + n * sizeof(int) + tc * sizeof(unsigned), 0,
+					h->stream, &rc))
+				break;
+			h->d_exc_s1 = (long long *)(h->d_exc_s2 + 2 * n);
+			h->d_exc_c1 = h->d_exc_s1 + n;
+			h->d_exc_smp = h->d_exc_c1 + n;
+			h->d_exc_b1 = (int *)(h->d_exc_smp + tc);
+			h->d_exc_ticket = (unsigned *)(h->d_exc_b1 + n);
 		}
 		if (cfg->flags & RTLSDR_GPU_FLAG_LEVEL_STATS) {
 			if (!alloc_fill(&h->d_level, (size_t)cfg->tune_count * 2 * sizeof(unsigned long long), 0, h->stream, &rc))
@@ -2108,6 +2187,11 @@ int rtlsdr_gpu_scan_db_count(const rtlsdr_gpu_scan_t *h)
 	return h ? h->shape.db_count : RTLSDR_GPU_ERR_NULL;
 }
 
+int rtlsdr_gpu_scan_blocks_per_read(const rtlsdr_gpu_scan_t *h)
+{
+	return h ? (h->shape.path == PATH_RMS ? 1 : h->shape.n_blocks) : RTLSDR_GPU_ERR_NULL;
+}
+
 static int collect_range(rtlsdr_gpu_scan_t *h, int hop0, int nhops, int64_t *avg, int *samples, double *db)
 {
 	CU(cudaSetDevice(h->cfg.device));
@@ -2144,6 +2228,8 @@ static int collect_range(rtlsdr_gpu_scan_t *h, int hop0, int nhops, int64_t *avg
 		CU(cudaMemsetAsync(h->d_level + 2 * (size_t)hop0, 0, (size_t)nhops * 2 * sizeof(unsigned long long), h->stream));
 	if (h->d_s2)
 		CU(cudaMemsetAsync(h->d_s2 + 2 * (size_t)hop0 * N, 0, (size_t)nhops * N * 2 * sizeof(unsigned long long), h->stream));
+	if ((rc = zero_excise(h, hop0, nhops)))
+		return rc;
 	CU(cudaStreamSynchronize(h->stream));
 	for (int i = 0; i < nhops; i++) {
 		if (samples)
@@ -2290,7 +2376,7 @@ int rtlsdr_gpu_scan_collect_sk_device(rtlsdr_gpu_scan_t *h, void *dev_avg, void 
 		return rc;
 	h->last_was_epilogue = false;
 	CU(cudaMemsetAsync(h->d_s2, 0, s2_bytes, h->stream));
-	return 0;
+	return zero_excise(h, 0, h->cfg.tune_count);
 }
 
 int rtlsdr_gpu_scan_set_csv_columns(rtlsdr_gpu_scan_t *h, int rows, const int32_t *low, const int32_t *high, double step)
@@ -2356,17 +2442,8 @@ static int collect_text(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, siz
 	int rc = flush_ring(h);
 	if (rc)
 		return rc;
-	if (!h->d_csv_len) { /* [0] the power text's length, [1] the SK text's */
-		CU(cudaMalloc(&h->d_csv_len, 2 * sizeof(long long)));
-		CU(cudaMallocHost(&h->h_csv_len, 2 * sizeof(long long)));
-	}
-	if (bound + sk_bound > h->csv_text_bytes) {
-		cudaFree(h->d_csv_text);
-		h->d_csv_text = nullptr;
-		h->csv_text_bytes = 0;
-		CU(cudaMalloc(&h->d_csv_text, bound + sk_bound));
-		h->csv_text_bytes = bound + sk_bound;
-	}
+	if ((rc = ensure_csv_text(h, bound + sk_bound)))
+		return rc;
 	/* in front of the epilogue: reads S1, the counters and S2 */
 	if (sk_text && (rc = run_sk_report(h, h->d_sk)))
 		return rc;
@@ -2394,6 +2471,8 @@ static int collect_text(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, siz
 		CU(cudaMemsetAsync(h->d_level, 0, (size_t)tc * 2 * sizeof(unsigned long long), h->stream));
 	if (h->d_s2)
 		CU(cudaMemsetAsync(h->d_s2, 0, (size_t)tc * h->shape.N * 2 * sizeof(unsigned long long), h->stream));
+	if ((rc = zero_excise(h, 0, tc)))
+		return rc;
 	CU(cudaStreamSynchronize(h->stream));
 	std::fill(h->samples.begin(), h->samples.end(), 0);
 	if (h->d_level)
@@ -2497,8 +2576,8 @@ int rtlsdr_gpu_scan_merge_sk_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, c
 		return RTLSDR_GPU_ERR_CONFIG;
 	if (((uintptr_t)dev_avg & 7) || ((uintptr_t)dev_samples & 3) || ((uintptr_t)dev_s2 & 7) || (set_stride & 7))
 		return RTLSDR_GPU_ERR_ALIGN;
-	if (!h->d_s2)
-		return RTLSDR_GPU_ERR_CONFIG;
+	if (!h->d_s2 || h->d_exc_s2)
+		return RTLSDR_GPU_ERR_CONFIG; /* excision: merged reads would land in one sub-integration */
 	CU(cudaSetDevice(h->cfg.device));
 	int rc = flush_ring(h);
 	if (rc)
@@ -2519,6 +2598,121 @@ int rtlsdr_gpu_scan_merge_sk_device(rtlsdr_gpu_scan_t *h, const void *dev_avg, c
 	merge_sk_sets_kernel<<<std::max(grid, 1), 256, 0, h->stream>>>(p);
 	h->samples_on_device = true; /* the host mirror of tunes[i].samples no longer knows the totals */
 	return check_launch(h, "merge_sk_sets_kernel");
+}
+
+int rtlsdr_gpu_scan_excise_fold(rtlsdr_gpu_scan_t *h, double k_low, double k_high)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_exc_s2 || !(k_low >= 0.0) || !(k_high >= 0.0)) /* also NaN */
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc = flush_ring(h);
+	if (rc)
+		return rc;
+	ExciseFoldParams p;
+	p.avg = h->d_avg;
+	p.samples = h->d_smp64;
+	p.s2 = h->d_s2;
+	p.snap_s1 = h->d_exc_s1;
+	p.snap_s2 = h->d_exc_s2;
+	p.c1 = h->d_exc_c1;
+	p.b1 = h->d_exc_b1;
+	p.snap_smp = h->d_exc_smp;
+	p.ticket = h->d_exc_ticket;
+	p.k_low = k_low;
+	p.k_high = k_high;
+	p.bin_e = h->cfg.bin_e;
+	p.downsample = h->cfg.downsample;
+	h->last_was_epilogue = false;
+	excise_fold_kernel<<<dim3((h->shape.N + 255) / 256, h->cfg.tune_count), 256, 0, h->stream>>>(p);
+	return check_launch(h, "excise_fold_kernel");
+}
+
+int rtlsdr_gpu_scan_excised_report(rtlsdr_gpu_scan_t *h, int64_t *clean_avg, int32_t *clean_blocks,
+				   int32_t *folded_samples, double *db, double *flagged)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_exc_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	CU(cudaSetDevice(h->cfg.device));
+	const size_t tc = (size_t)h->cfg.tune_count, n = tc * h->shape.N, rows = tc * h->shape.db_count;
+	/* dB rows and flag fractions through the handle's dB and SK row buffers, C1 and B1 straight from the state */
+	int rc;
+	if ((db || flagged || folded_samples) &&
+	    (rc = run_excised_report(h, h->d_samples, db ? h->d_db : nullptr, flagged ? h->d_sk : nullptr)))
+		return rc;
+	if (db)
+		CU(cudaMemcpyAsync(db, h->d_db, rows * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+	if (flagged)
+		CU(cudaMemcpyAsync(flagged, h->d_sk, rows * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+	if (folded_samples)
+		CU(cudaMemcpyAsync(folded_samples, h->d_samples, tc * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+	if (clean_avg)
+		CU(cudaMemcpyAsync(clean_avg, h->d_exc_c1, n * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+	if (clean_blocks)
+		CU(cudaMemcpyAsync(clean_blocks, h->d_exc_b1, n * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+	h->d2h += (uint64_t)((db ? rows * 8 : 0) + (flagged ? rows * 8 : 0) + (folded_samples ? tc * 4 : 0) +
+			     (clean_avg ? n * 8 : 0) + (clean_blocks ? n * 4 : 0));
+	CU(cudaStreamSynchronize(h->stream));
+	return 0;
+}
+
+int rtlsdr_gpu_scan_excised_report_device(rtlsdr_gpu_scan_t *h, void *dev_db, void *dev_flagged, void *dev_samples)
+{
+	if (!h)
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_exc_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	if (((uintptr_t)dev_db & 7) || ((uintptr_t)dev_flagged & 7) || ((uintptr_t)dev_samples & 3))
+		return RTLSDR_GPU_ERR_ALIGN;
+	if (!dev_db && !dev_flagged && !dev_samples)
+		return 0;
+	CU(cudaSetDevice(h->cfg.device));
+	return run_excised_report(h, (int *)dev_samples, (double *)dev_db, (double *)dev_flagged);
+}
+
+int rtlsdr_gpu_scan_excised_csv(rtlsdr_gpu_scan_t *h, const char *stamp, char *text, size_t cap, size_t *len,
+				char *flag_text, size_t flag_cap, size_t *flag_len)
+{
+	if (!h || !stamp || !text || !len || (flag_text && !flag_len))
+		return RTLSDR_GPU_ERR_NULL;
+	if (!h->d_exc_s2)
+		return RTLSDR_GPU_ERR_CONFIG;
+	const size_t stamp_len = strlen(stamp);
+	const int tc = h->cfg.tune_count;
+	if (stamp_len >= (size_t)kCsvStampMax || h->csv_rows < tc)
+		return RTLSDR_GPU_ERR_CONFIG;
+	const size_t bound = csv_bound(h, tc, stamp_len), f_bound = flag_text ? csv_bound(h, tc, stamp_len, true) : 0;
+	if (cap < bound || flag_cap < f_bound)
+		return RTLSDR_GPU_ERR_LENGTH;
+	CU(cudaSetDevice(h->cfg.device));
+	int rc;
+	if ((rc = ensure_csv_text(h, bound + f_bound)))
+		return rc;
+	if ((rc = run_excised_report(h, h->d_samples, h->d_db, flag_text ? h->d_sk : nullptr)))
+		return rc;
+	if ((rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_db, h->shape.db_count, h->d_samples, h->d_csv_text, h->d_csv_len)))
+		return rc;
+	if (flag_text && (rc = run_csv(h, stamp, stamp_len, 0, tc, h->d_sk, h->shape.db_count, h->d_samples,
+					h->d_csv_text + bound, h->d_csv_len + 1, true)))
+		return rc;
+	const int nlen = flag_text ? 2 : 1;
+	CU(cudaMemcpyAsync(h->h_csv_len, h->d_csv_len, nlen * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+	CU(cudaStreamSynchronize(h->stream));
+	const long long nt = h->h_csv_len[0], mt = flag_text ? h->h_csv_len[1] : 0;
+	if (nt < 0 || (size_t)nt > bound || mt < 0 || (size_t)mt > f_bound)
+		return RTLSDR_GPU_ERR_CONFIG; /* cannot happen for the report's values */
+	CU(cudaMemcpyAsync(text, h->d_csv_text, (size_t)nt, cudaMemcpyDeviceToHost, h->stream));
+	if (flag_text)
+		CU(cudaMemcpyAsync(flag_text, h->d_csv_text + bound, (size_t)mt, cudaMemcpyDeviceToHost, h->stream));
+	h->d2h += (uint64_t)nt + (uint64_t)mt + nlen * sizeof(long long);
+	CU(cudaStreamSynchronize(h->stream));
+	*len = (size_t)nt;
+	if (flag_len)
+		*flag_len = (size_t)mt;
+	return 0;
 }
 
 int rtlsdr_gpu_scan_level_stats(rtlsdr_gpu_scan_t *h, int hop, uint64_t *overload, uint64_t *high_level, uint64_t *bytes)

@@ -33,6 +33,9 @@ inline int scan_shape(const rtlsdr_gpu_scan_cfg_t &cfg, ScanShape *out)
 	if ((cfg.flags & RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS) &&
 	    (cfg.peak_hold || cfg.bin_e == 0 || (cfg.flags & RTLSDR_GPU_FLAG_ASYNC_REPORT)))
 		return RTLSDR_GPU_ERR_CONFIG;
+	/* excision folds sub-integrations of the SK moments */
+	if ((cfg.flags & RTLSDR_GPU_FLAG_SK_EXCISION) && !(cfg.flags & RTLSDR_GPU_FLAG_SPECTRAL_KURTOSIS))
+		return RTLSDR_GPU_ERR_CONFIG;
 	/* guard bits widen the transform; the rms path has none */
 	if ((cfg.flags & RTLSDR_GPU_FLAG_GUARD_BITS) && cfg.bin_e == 0)
 		return RTLSDR_GPU_ERR_CONFIG;

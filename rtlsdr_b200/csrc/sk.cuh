@@ -98,6 +98,28 @@ SK_HD double sk_from_moments(long long S1, unsigned long long s2_lo, unsigned lo
 	return sk_mul(e, d);
 }
 
+SK_HD double sk_sqrt(double a)
+{
+#ifdef __CUDA_ARCH__
+	return __dsqrt_rn(a);
+#else
+	return sqrt(a);
+#endif
+}
+
+/* the standard deviation of the estimator over M blocks of single-block power (Nita & Gary 2010, N = d = 1):
+ *   sigma = sqrt(4 M^2 / ((M-1)(M+2)(M+3))), quiet NaN when M < 2,
+ * as m = rn(M); a = (4*m)*m; b = ((m-1)*(m+2))*(m+3); sigma = sqrt(a/b), every step correctly rounded */
+SK_HD double sk_sigma(long long M)
+{
+	if (M < 2)
+		return NAN;
+	const double m = (double)M;
+	const double a = sk_mul(sk_mul(4.0, m), m);
+	const double b = sk_mul(sk_mul(sk_add(m, -1.0), sk_add(m, 2.0)), sk_add(m, 3.0));
+	return sk_sqrt(sk_div(a, b));
+}
+
 /* ---- device accumulation ------------------------------------------------ */
 
 /* pw^2 into a register partial (lo, carry count): exact over up to 2^32 additions */

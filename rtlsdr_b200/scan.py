@@ -66,12 +66,18 @@ def load_library():
     L.rtlsdr_gpu_scan_collect_sk_csv.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t,
                                                  ctypes.POINTER(ctypes.c_size_t), vp, ctypes.c_size_t,
                                                  ctypes.POINTER(ctypes.c_size_t)]
+    L.rtlsdr_gpu_scan_excise_fold.argtypes = [vp, ctypes.c_double, ctypes.c_double]
+    L.rtlsdr_gpu_scan_excised_report.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.rtlsdr_gpu_scan_excised_report_device.argtypes = [vp, vp, vp, vp]
+    L.rtlsdr_gpu_scan_excised_csv.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t),
+                                              vp, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]
     L.rtlsdr_gpu_scan_set_csv_columns.argtypes = [vp, i, vp, vp, ctypes.c_double]
     L.rtlsdr_gpu_scan_csv_capacity.argtypes = [vp, i, ctypes.c_size_t]
     L.rtlsdr_gpu_scan_csv_capacity.restype = i64
     L.rtlsdr_gpu_scan_collect_csv.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]
     L.rtlsdr_gpu_scan_format_csv_device.argtypes = [vp, ctypes.c_char_p, i, i, vp, i64, vp, vp, ctypes.c_size_t, vp]
     L.rtlsdr_gpu_scan_db_count.argtypes = [vp]
+    L.rtlsdr_gpu_scan_blocks_per_read.argtypes = [vp]
     L.rtlsdr_gpu_scan_host_alloc.argtypes = [ctypes.c_size_t]
     L.rtlsdr_gpu_scan_host_alloc.restype = vp
     L.rtlsdr_gpu_scan_host_free.argtypes = [vp]
@@ -168,7 +174,7 @@ class GpuScan:
     def __init__(self, tune_count, bin_e, buf_len, downsample=1, downsample_passes=0, boxcar=1,
                  comp_fir_size=0, peak_hold=0, rate=2400000, crop=0.0, window_coefs=None,
                  sinewave=None, device=0, ring_bytes=0, level_stats=False, iir_alpha=0.0, async_report=False,
-                 short_reads=False, spectral_kurtosis=False, guard_bits=False):
+                 short_reads=False, spectral_kurtosis=False, guard_bits=False, sk_excision=False):
         self.lib = load_library()
         self.tune_count, self.bin_e, self.buf_len = tune_count, bin_e, buf_len
         self.n = 1 << bin_e
@@ -188,9 +194,11 @@ class GpuScan:
             self._s = np.ascontiguousarray(sinewave, dtype=np.int16)
             cfg.sinewave = self._s.ctypes.data
         cfg.ring_bytes = ring_bytes
-        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS / _SPECTRAL_KURTOSIS / _GUARD_BITS
+        # RTLSDR_GPU_FLAG_LEVEL_STATS / _ASYNC_REPORT / _SHORT_READS / _SPECTRAL_KURTOSIS / _GUARD_BITS /
+        # _SK_EXCISION (which needs spectral kurtosis, so sk_excision=True sets both)
         cfg.flags = ((1 if level_stats else 0) | (2 if async_report else 0) | (4 if short_reads else 0)
-                     | (8 if spectral_kurtosis else 0) | (16 if guard_bits else 0))
+                     | (8 if spectral_kurtosis or sk_excision else 0) | (16 if guard_bits else 0)
+                     | (32 if sk_excision else 0))
         cfg.iir_alpha = iir_alpha            # -s iir smoothing of the dB rows across reports (0 = off)
         self.h = ctypes.c_void_p()
         rc = self.lib.rtlsdr_gpu_scan_init(ctypes.byref(cfg), ctypes.byref(self.h))
@@ -198,6 +206,7 @@ class GpuScan:
             self.h = None
             raise ScanError(rc, "rtlsdr_gpu_scan_init", self.lib.rtlsdr_gpu_scan_strerror(rc).decode())
         self.db_count = self.lib.rtlsdr_gpu_scan_db_count(self.h)
+        self.blocks_per_read = self.lib.rtlsdr_gpu_scan_blocks_per_read(self.h)   # FFT blocks (M) one read adds
 
     @classmethod
     def from_plan(cls, plan, window_coefs=None, peak_hold=0, device=0, hops=None, **kw):
@@ -291,6 +300,49 @@ class GpuScan:
         added as exact 128-bit sums"""
         self._check(self.lib.rtlsdr_gpu_scan_merge_sk_device(self.h, dev_avg, dev_samples, dev_s2, sets, set_stride),
                     "merge_sk_device")
+
+    def excise_sweeps(self, min_blocks=64):
+        """the fewest sweeps (reads per hop) whose sub-integration gives every hop at least min_blocks FFT blocks"""
+        return max(1, -(-min_blocks // self.blocks_per_read))
+
+    def excise_fold(self, k_low=3.0, k_high=3.0):
+        """close a sub-integration of every hop (sk_excision=True handles): a bin's sub-integration joins its clean
+        average unless its SK lies below 1 - k_low sigma(M) or above 1 + k_high sigma(M); float('inf') never flags
+        that side.  Async on the handle's stream."""
+        self._check(self.lib.rtlsdr_gpu_scan_excise_fold(self.h, float(k_low), float(k_high)), "excise_fold")
+
+    def excised_report(self):
+        """the excised report, nothing zeroed: (clean_avg int64 [tc, N], clean_blocks int32 [tc, N], folded samples
+        int32 [tc], excised dB float64 [tc, db_count], flag fractions float64 [tc, db_count])"""
+        c1 = np.zeros((self.tune_count, self.n), dtype=np.int64)
+        b1 = np.zeros((self.tune_count, self.n), dtype=np.int32)
+        smp = np.zeros(self.tune_count, dtype=np.int32)
+        db = np.zeros((self.tune_count, self.db_count), dtype=np.float64)
+        fl = np.zeros((self.tune_count, self.db_count), dtype=np.float64)
+        self._check(self.lib.rtlsdr_gpu_scan_excised_report(self.h, c1.ctypes.data, b1.ctypes.data, smp.ctypes.data,
+                                                            db.ctypes.data, fl.ctypes.data), "excised_report")
+        return c1, b1, smp, db, fl
+
+    def excised_report_device(self, dev_db=None, dev_flagged=None, dev_samples=None):
+        """excised dB rows, flag fractions (float64 [tc, db_count]) and folded samples (int32 [tc]) into device
+        memory (may be peer memory); any address may be None; async on the handle's stream"""
+        self._check(self.lib.rtlsdr_gpu_scan_excised_report_device(self.h, dev_db, dev_flagged, dev_samples),
+                    "excised_report_device")
+
+    def excised_csv(self, stamp, flags=True, out=None, flag_out=None):
+        """the excised report's text, formatted on the GPU: (excised dB rows, flag-fraction rows or None without
+        `flags`) as bytes, the folded samples in the count column; nothing is zeroed"""
+        s = stamp.encode() if isinstance(stamp, str) else bytes(stamp)
+        if out is None:
+            out = np.empty(max(1, self.csv_capacity(self.tune_count, len(s))), dtype=np.uint8)
+        if flags and flag_out is None:
+            flag_out = np.empty(max(1, self.sk_csv_capacity(self.tune_count, len(s))), dtype=np.uint8)
+        n, m = ctypes.c_size_t(0), ctypes.c_size_t(0)
+        self._check(self.lib.rtlsdr_gpu_scan_excised_csv(self.h, s, out.ctypes.data, out.nbytes, ctypes.byref(n),
+                                                         flag_out.ctypes.data if flags else None,
+                                                         flag_out.nbytes if flags else 0,
+                                                         ctypes.byref(m) if flags else None), "excised_csv")
+        return out[: n.value].tobytes(), (flag_out[: m.value].tobytes() if flags else None)
 
     def set_csv_columns(self, low, high, step):
         """row table of the CSV formatter: row r prints low[r], high[r], step (Plan.csv_columns())"""

@@ -108,7 +108,10 @@ class SpectrumGather:
 
     A report buffer is `words` int64 words: [avg hmax*N | db hmax*db_count (bit patterns) |
     samples hmax x int32, padded to 8 bytes], hmax = the largest shard; with sk=True (spectral-kurtosis handles)
-    followed by [S2 hmax*N*2 (lo, hi) | SK rows hmax*db_count], at word offsets s2_at and sk_at.  Use per interval j
+    followed by [S2 hmax*N*2 (lo, hi) | SK rows hmax*db_count], at word offsets s2_at and sk_at; with excise=True
+    (spectral-kurtosis excision handles, which implies the SK sections) followed by [excised dB rows hmax*db_count |
+    flag rows hmax*db_count | folded samples hmax x int32, padded to 8 bytes] at xdb_at, xfl_at and xsmp_at, what
+    rtlsdr_gpu_scan_excised_report_device() writes (excise_pointers()).  Use per interval j
     (k = j % SLOTS):
         before_collect(k, stream); collect_device(*pointers(k)); publish(k, stream)
         (sk: collect_sk_device(*pointers(k), *sk_pointers(k)))
@@ -116,7 +119,7 @@ class SpectrumGather:
     """
 
     def __init__(self, tune_count, n_bins, db_count, world, rank, device, mode=None, sizes=None, replicated=False,
-                 sk=False):
+                 sk=False, excise=False):
         self.tune_count, self.n, self.db_count = tune_count, n_bins, db_count
         self.world, self.rank = world, rank
         self.device = torch.device(device)
@@ -128,12 +131,18 @@ class SpectrumGather:
         self.hmax = max(1, max(len(r) for r in self.ranges))
         self.smp_words = (self.hmax + 1) // 2
         self.words = self.hmax * (n_bins + db_count) + self.smp_words
-        self.sk = sk
-        self.s2_at = self.sk_at = None
-        if sk:
+        self.sk = sk or excise
+        self.excise = excise
+        self.s2_at = self.sk_at = self.xdb_at = self.xfl_at = self.xsmp_at = None
+        if self.sk:
             self.s2_at = self.words
             self.sk_at = self.s2_at + self.hmax * n_bins * 2
             self.words = self.sk_at + self.hmax * db_count
+        if excise:
+            self.xdb_at = self.words
+            self.xfl_at = self.xdb_at + self.hmax * db_count
+            self.xsmp_at = self.xfl_at + self.hmax * db_count
+            self.words = self.xsmp_at + self.smp_words
         self.my_hops = self.ranges[rank]
         self.peer = None
         # peer mode: int32 flags behind the report buffers of the symmetric allocation:
@@ -240,10 +249,25 @@ class SpectrumGather:
         assert self.sk
         return slot_base + self.s2_at * 8, slot_base + self.sk_at * 8
 
+    def excise_pointers(self, k=0):
+        """excise: device addresses of the excised dB rows, the flag rows and the folded samples (int32) of report
+        buffer k, for rtlsdr_gpu_scan_excised_report_device()"""
+        return self.excise_sections(self.pointers(k)[0])
+
+    def excise_sections(self, slot_base):
+        """excise: (excised dB rows, flag rows, folded samples) addresses of the slot starting at `slot_base`"""
+        assert self.excise
+        return slot_base + self.xdb_at * 8, slot_base + self.xfl_at * 8, slot_base + self.xsmp_at * 8
+
+    def slot_excise(self, k, r):
+        """rank 0, excise: the three excision sections of rank r's slot in the private copy of buffer k"""
+        return self.excise_sections(self.dev_copy[k].data_ptr() + r * self.words * 8)
+
     def views(self, k=0):
         """(avg [h, N] int64, db [h, db_count] float64, samples [h] int32) views of the LOCAL send buffer k
         sized for this rank's hop count (host mode / tests fill these instead of a GPU epilogue); with sk also
-        (s2 [h, N, 2] uint64, sk [h, db_count] float64)"""
+        (s2 [h, N, 2] uint64, sk [h, db_count] float64); with excise also (excised dB [h, db_count] float64,
+        flag rows [h, db_count] float64, folded samples [h] int32)"""
         h = len(self.my_hops)
         s = self.send[k]
         a = s[: self.hmax * self.n].view(self.hmax, self.n)[:h]
@@ -254,8 +278,13 @@ class SpectrumGather:
         if not self.sk:
             return a, d, c
         s2 = s[self.s2_at: self.sk_at].view(torch.uint64).view(self.hmax, self.n, 2)[:h]
-        sk = s[self.sk_at: self.words].view(torch.float64).view(self.hmax, self.db_count)[:h]
-        return a, d, c, s2, sk
+        sk = s[self.sk_at: self.sk_at + self.hmax * self.db_count].view(torch.float64).view(self.hmax, self.db_count)[:h]
+        if not self.excise:
+            return a, d, c, s2, sk
+        xdb = s[self.xdb_at: self.xfl_at].view(torch.float64).view(self.hmax, self.db_count)[:h]
+        xfl = s[self.xfl_at: self.xsmp_at].view(torch.float64).view(self.hmax, self.db_count)[:h]
+        xsmp = s[self.xsmp_at: self.words].view(torch.int32)[:h]
+        return a, d, c, s2, sk, xdb, xfl, xsmp
 
     def _flag_addr(self, owner, index):
         """device address (as seen from this rank) of int32 flag `index` in rank `owner`'s symmetric buffer"""
@@ -421,8 +450,8 @@ class SpectrumGather:
             smp[hops.start: hops.stop] = b[o: o + self.smp_words].view(np.int32)[:h]
             if self.sk:
                 s2[hops.start: hops.stop] = b[self.s2_at: self.sk_at].view(np.uint64).reshape(self.hmax, self.n, 2)[:h]
-                sk[hops.start: hops.stop] = b[self.sk_at: self.words].view(np.float64).reshape(
-                    self.hmax, self.db_count)[:h]
+                sk[hops.start: hops.stop] = b[self.sk_at: self.sk_at + self.hmax * self.db_count].view(
+                    np.float64).reshape(self.hmax, self.db_count)[:h]
         return IntervalReport(avg, db, smp, s2, sk)
 
     def describe(self):

@@ -24,6 +24,15 @@ collect_sk_device() adds its SK rows to its report slot and rank 0 formats them 
 rank 0 folds all three sums into its handle (rtlsdr_gpu_scan_merge_sk_device) before rtlsdr_gpu_scan_collect_sk_csv
 -- SK rows byte-identical to one GPU's.  The power CSV is the same with and without --sk.  Not with -P or 1-bin
 (rms) hops.
+--excise FILE writes the spectral-kurtosis-excised power rows (RTLSDR_GPU_FLAG_SK_EXCISION, hop-sharded only): every
+interval's sweeps are submitted in chunks of --excise-sweeps K passes with rtlsdr_gpu_scan_excise_fold() after each
+chunk, so a bin's sub-integration of K sweeps enters its clean average only when its SK lies within
+[1 - LOW sigma, 1 + HIGH sigma] (--excise-sigma LOW[:HIGH], default 3:3, inf never flags that side).  Every rank's
+excised_report_device() adds the excised dB rows, the flag fractions and the folded sample counts to its report slot
+(SpectrumGather(excise=True)) in front of its collect_sk_device(); rank 0 formats them like the power rows
+(--excise) and like the SK rows (--excise-flags FILE), with the folded samples as the count column.  The power and
+SK files are the same with and without --excise.  Not with --shard reads (merged reads would land in one
+sub-integration), -P or 1-bin hops.
 """
 import argparse
 import ctypes
@@ -56,6 +65,16 @@ def main(argv=None):
     ap.add_argument("--device", type=int, default=None, help="CUDA device of this rank (default: LOCAL_RANK)")
     ap.add_argument("--sk", dest="sk_out", default=None, metavar="FILE",
                     help="also write each bin's spectral kurtosis to FILE (rows like the power rows, %%.4f values)")
+    ap.add_argument("--excise", dest="excise_out", default=None, metavar="FILE",
+                    help="also write the spectral-kurtosis-excised power rows to FILE (sub-integrations whose SK lies "
+                         "outside the thresholds are left out of a bin's average)")
+    ap.add_argument("--excise-flags", dest="flags_out", default=None, metavar="FILE",
+                    help="with --excise: the flagged fraction of every bin's sub-integrations (%%.4f values)")
+    ap.add_argument("--excise-sweeps", type=int, default=None, metavar="K",
+                    help="with --excise: sweeps per sub-integration (default: the fewest giving every hop 64 FFT "
+                         "blocks)")
+    ap.add_argument("--excise-sigma", default="3:3", metavar="LOW[:HIGH]",
+                    help="with --excise: thresholds 1 - LOW*sigma and 1 + HIGH*sigma (default 3:3)")
     ap.add_argument("--guard-bits", action="store_true",
                     help="fix_fft with 8 fractional guard bits (RTLSDR_GPU_FLAG_GUARD_BITS): the transform rounds "
                          "2^8 below the reference's LSB, so fine-resolution rows show the signal's noise floor")
@@ -63,6 +82,24 @@ def main(argv=None):
     args = ap.parse_args(argv)
     if args.sk_out is not None and args.peak:
         raise SystemExit("sweep_main: --sk needs averaged power bins, not -P peak hold")
+    excise = args.excise_out is not None
+    k_low = k_high = None
+    if args.flags_out is not None and not excise:
+        raise SystemExit("sweep_main: --excise-flags needs --excise")
+    if excise:
+        if args.shard == "reads":
+            raise SystemExit("sweep_main: --excise needs all reads of a hop on one rank, not --shard reads")
+        if args.peak:
+            raise SystemExit("sweep_main: --excise needs averaged power bins, not -P peak hold")
+        if args.excise_sweeps is not None and args.excise_sweeps < 1:
+            raise SystemExit("sweep_main: --excise-sweeps must be >= 1")
+        try:
+            lo, _, hi = args.excise_sigma.partition(":")
+            k_low, k_high = float(lo), float(hi or lo)
+        except ValueError:
+            k_low = k_high = float("nan")
+        if not (k_low >= 0 and k_high >= 0):
+            raise SystemExit("sweep_main: --excise-sigma LOW[:HIGH] needs two values >= 0")
 
     import torch
     import torch.distributed as dist
@@ -91,8 +128,11 @@ def main(argv=None):
     sk = args.sk_out is not None
     if sk and pd["bin_e"] == 0:
         raise SystemExit("sweep_main: --sk needs FFT bins; this scan's hops are 1-bin (rms) power readings")
+    if excise and pd["bin_e"] == 0:
+        raise SystemExit("sweep_main: --excise needs FFT bins; this scan's hops are 1-bin (rms) power readings")
     if args.guard_bits and pd["bin_e"] == 0:
         raise SystemExit("sweep_main: --guard-bits needs FFT bins; this scan's hops are 1-bin (rms) power readings")
+    sk = sk or excise          # an excision handle is an SK handle: its report is collect_sk_device()
     tc, b, n = pd["tune_count"], pd["buf_len"], 1 << pd["bin_e"]
     mine = shard_hops(tc, world, rank)
     mode = ["xorshift", "counter", "const", "biased", "tone"].index(args.synth)
@@ -104,23 +144,29 @@ def main(argv=None):
     if len(mine):
         window = rs.window_coefs(args.window, n) if pd["bin_e"] else None
         g = rs.GpuScan.from_plan(pd, window_coefs=window, device=local, hops=list(mine), spectral_kurtosis=sk,
-                                 guard_bits=args.guard_bits)
+                                 guard_bits=args.guard_bits, sk_excision=excise)
+    # sub-integration length: K passes per fold (the same K on every rank: FFT blocks per read do not depend on the hop)
+    chunk = (args.excise_sweeps or g.excise_sweeps()) if (g and excise) else args.sweeps
     db_count = g.db_count if g else plan.db_count
     gather = SpectrumGather(tc, n, db_count, world, rank, torch.device("cuda", local),
-                            mode=("host" if args.backend == "gloo" and world > 1 else None), sk=sk)
+                            mode=("host" if args.backend == "gloo" and world > 1 else None), sk=sk, excise=excise)
     if rank == 0 and world > 1:
         print("sweep_main: interval reports: " + gather.describe(), file=sys.stderr)
     stream = torch.cuda.ExternalStream(g.get_stream()) if g else torch.cuda.current_stream()
     stamp = args.stamp + ", "
+    groups = ["power"] + (["sk"] if args.sk_out is not None else []) + (["excise"] if excise else []) + \
+        (["flags"] if args.flags_out is not None else [])
     if rank == 0:
         # rank 0 formats every rank's rows from a private device copy of the gathered report, on its handle's
         # stream behind the exchange; one text region and one int64 length per rank slot, copied out together
         gather.keep_device_copy()
         g.set_csv_columns(*plan.csv_columns())
-        # with --sk the SK rows' regions follow the power rows' (slots world..2*world-1), and so do their lengths
-        caps = [g.csv_capacity(len(r), len(stamp.encode())) for r in gather.ranges]
-        if sk:
-            caps += [g.sk_csv_capacity(len(r), len(stamp.encode())) for r in gather.ranges]
+        # one text region per (output, rank slot): the power rows, then with --sk the SK rows, with --excise the
+        # excised rows and, with --excise-flags, the flag rows; group gi's regions are slots gi*world..gi*world+world-1
+        caps = []
+        for name in groups:
+            cap = g.sk_csv_capacity if name in ("sk", "flags") else g.csv_capacity
+            caps += [cap(len(r), len(stamp.encode())) for r in gather.ranges]
         offs = [0] + [int(x) for x in np.cumsum(caps)]
         lens_at = (offs[-1] + 7) // 8 * 8
         dev = torch.device("cuda", local)
@@ -134,7 +180,7 @@ def main(argv=None):
     consumed = [None, None]
 
     rng = np.random.default_rng(args.random_hops + 7919 * rank) if args.random_hops is not None else None
-    rows_out, sk_rows_out = [], []
+    outs = {name: [] for name in groups}
     pending = None          # exchange buffer of the interval whose report has not been printed yet
 
     def format_rows(k):
@@ -146,10 +192,18 @@ def main(argv=None):
                 p_db, p_smp = gather.slot_rows(k, r)
                 g.format_csv_device(stamp, hops.start, len(hops), p_db, g.db_count, p_smp,
                                     text_dev[k].data_ptr() + offs[r], caps[r], lens + 8 * r)
-                if sk:
-                    q = world + r
-                    g.format_sk_csv_device(stamp, hops.start, len(hops), gather.slot_sk(k, r)[1], g.db_count, p_smp,
-                                           text_dev[k].data_ptr() + offs[q], caps[q], lens + 8 * q)
+                for gi, name in enumerate(groups[1:], 1):
+                    q = gi * world + r
+                    at, cap, ln = text_dev[k].data_ptr() + offs[q], caps[q], lens + 8 * q
+                    if name == "sk":
+                        g.format_sk_csv_device(stamp, hops.start, len(hops), gather.slot_sk(k, r)[1], g.db_count, p_smp,
+                                               at, cap, ln)
+                        continue
+                    x_db, x_fl, x_smp = gather.slot_excise(k, r)     # the folded samples are the count column
+                    if name == "excise":
+                        g.format_csv_device(stamp, hops.start, len(hops), x_db, g.db_count, x_smp, at, cap, ln)
+                    else:
+                        g.format_sk_csv_device(stamp, hops.start, len(hops), x_fl, g.db_count, x_smp, at, cap, ln)
         gather.release_copy(k, stream)
         with torch.cuda.stream(stream):
             text_host[k].copy_(text_dev[k], non_blocking=True)
@@ -165,7 +219,7 @@ def main(argv=None):
                 if len(gather.ranges[q % world]):
                     if lens[q] < 0:
                         raise RuntimeError("sweep_main: a report value is outside the CSV formatter's domain")
-                    (rows_out if q < world else sk_rows_out).append(buf[offs[q]: offs[q] + lens[q]].tobytes().decode())
+                    outs[groups[q // world]].append(buf[offs[q]: offs[q] + lens[q]].tobytes().decode())
 
     for interval in range(args.intervals):
         k = interval & 1
@@ -175,7 +229,13 @@ def main(argv=None):
             if rng is None:
                 synth_cube(pinned[k].ptr, mode, args.seed, args.param, tc, mine.start, len(mine),
                            interval * args.sweeps, args.sweeps, b)
-                g.submit_batch(0, len(mine), args.sweeps, pinned[k].ptr, len(mine) * b, b)
+                # --excise: chunks of K passes, a fold behind each (the last, shorter chunk's fold comes before
+                # the report); without it one chunk
+                for p0 in range(0, args.sweeps, chunk):
+                    g.submit_batch(0, len(mine), min(chunk, args.sweeps - p0), pinned[k].ptr + p0 * len(mine) * b,
+                                   len(mine) * b, b)
+                    if excise:
+                        g.excise_fold(k_low, k_high)
             else:
                 # randomised hopping: every sweep visits this rank's hops in its own random order
                 cube = pinned[k].view(np.uint8, (args.sweeps, len(mine), b))
@@ -185,10 +245,17 @@ def main(argv=None):
                         host.synth_generate(mode, ctypes.c_uint64(args.seed), args.param, tc, mine.start + int(lh),
                                             ctypes.c_uint64(interval * args.sweeps + s_), cube[s_, j].ctypes.data,
                                             ctypes.c_size_t(b))
-                g.submit_reads(order.ravel(), pinned[k].ptr, b)
+                for p0 in range(0, args.sweeps, chunk):
+                    g.submit_reads(order[p0: p0 + chunk].ravel(), pinned[k].ptr + p0 * len(mine) * b, b)
+                    if excise:
+                        g.excise_fold(k_low, k_high)
             gather.before_collect(k, stream)
+            if excise:
+                # a peek, in front of the collect's read-and-zero of S1, S2 and the excision state
+                g.excised_report_device(*gather.excise_pointers(k))
             if sk:
-                g.collect_sk_device(*gather.pointers(k), None, gather.sk_pointers(k)[1])
+                g.collect_sk_device(*gather.pointers(k), None,
+                                    gather.sk_pointers(k)[1] if args.sk_out is not None else None)
             else:
                 g.collect_device(*gather.pointers(k))
             consumed[k] = torch.cuda.Event()
@@ -204,7 +271,7 @@ def main(argv=None):
     if pending is not None:
         print_pending()
     if rank == 0:
-        _write_rows(args, rows_out, sk_rows_out)
+        _write_rows(args, outs["power"], outs.get("sk", []), outs.get("excise"), outs.get("flags"))
     if rank == 0:
         # torch's pinned-memory allocator records an event on the stream of the last copy when it frees a block:
         # the text buffers go before the handle's stream does
@@ -218,16 +285,17 @@ def main(argv=None):
     return 0
 
 
-def _write_rows(args, rows_out, sk_rows_out):
+def _write_rows(args, rows_out, sk_rows_out, excise_rows=None, flag_rows=None):
     text = "".join(rows_out)
     if args.out == "-":
         sys.stdout.write(text)
     else:
         with open(args.out, "w") as f:
             f.write(text)
-    if args.sk_out is not None:
-        with open(args.sk_out, "w") as f:
-            f.write("".join(sk_rows_out))
+    for path, rows in ((args.sk_out, sk_rows_out), (args.excise_out, excise_rows), (args.flags_out, flag_rows)):
+        if path is not None:
+            with open(path, "w") as f:
+                f.write("".join(rows))
 
 
 def _main_read_sharded(args, rs, host, plan, pd, mode, world, rank, local, torch, dist,
