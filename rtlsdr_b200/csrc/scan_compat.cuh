@@ -212,6 +212,19 @@ SCAN_DEV void named_bar_sync(int id, int count)
 #endif
 }
 
+/* sum (mod 2^32) over the 32 lanes of a full warp, returned to every lane: one REDUX instead of five
+ * shuffle + add rounds */
+SCAN_DEV unsigned warp_sum(unsigned v)
+{
+#ifdef SCAN_EMU
+	for (int o = 16; o > 0; o >>= 1)
+		v += __shfl_xor_sync(0xffffffffu, v, o);
+	return v;
+#else
+	return __reduce_add_sync(0xffffffffu, v);
+#endif
+}
+
 SCAN_DEV void warp_sync()
 {
 #ifdef SCAN_EMU

@@ -202,6 +202,16 @@ SCAN_DEV int pos(int t, int r)
 
 SCAN_DEV int xch_idx(int p) { return p + (p >> 4); }
 
+/* xch_idx(pos<K>(t, r)) == xch_idx(pos<K>(t, 0)) + xch_step<K>() * r for every t: the three fields of pos<K> are
+ * disjoint, so p >> 4 splits over them, and r adds r << 4K to p and r << (4K - 4) to p >> 4 (nothing for K = 0).
+ * exchange_pk addresses with one per-thread base plus a compile-time offset per register: pos<K> composes with `|`,
+ * through which ptxas cannot distribute the padding term, and would rebuild every address. */
+template <int K>
+SCAN_DEV constexpr int xch_step()
+{
+	return K == 0 ? 1 : (1 << (4 * K)) + (1 << (4 * K - 4));
+}
+
 SCAN_DEV constexpr int brev4(int r)
 {
 	return ((r & 1) << 3) | ((r & 2) << 1) | ((r & 4) >> 1) | ((r & 8) >> 3);
@@ -265,6 +275,8 @@ struct GroupBar { /* the transform threads are one role of a warp-specialised CT
 template <int KA, int KB, bool LEAD, class BAR = BlockBar>
 SCAN_DEV void exchange(X2 (&x)[kPts], c16 *xch, int tw_, int t, const BAR &bar = BAR())
 {
+	/* the large path's transpose keeps per-register addresses: the base + offset form of exchange_pk measured 0.7 %
+	 * slower on config 4 here */
 	if (LEAD)
 		bar.sync();
 #pragma unroll
@@ -281,13 +293,14 @@ SCAN_DEV void exchange(X2 (&x)[kPts], c16 *xch, int tw_, int t, const BAR &bar =
 template <int KA, int KB, class BAR>
 SCAN_DEV void exchange_pk(X2 (&x)[kPts], c16 (&pk)[kPts], c16 *xch, int tw_, int t, const BAR &bar)
 {
+	const int st = xch_idx(pos<KA>(tw_, 0)), ld = xch_idx(pos<KB>(t, 0));
 #pragma unroll
 	for (int r = 0; r < kPts; ++r)
-		xch[xch_idx(pos<KA>(tw_, r))] = x_pack(x[r]);
+		xch[st + xch_step<KA>() * r] = x_pack(x[r]);
 	bar.sync();
 #pragma unroll
 	for (int r = 0; r < kPts; ++r) {
-		pk[r] = xch[xch_idx(pos<KB>(t, r))];
+		pk[r] = xch[ld + xch_step<KB>() * r];
 		if (!RSCAN_PACKED_B || (r & 1) == 0)
 			x[r] = x_unpack(pk[r]);
 	}
@@ -474,11 +487,8 @@ SCAN_DEV void u8_read_dc(const uint8_t *st, int *red, int t, int &kI, int &kQ)
 		sI = __dp4a(q.w, 0x00010001u, sI);
 		sQ = __dp4a(q.w, 0x01000100u, sQ);
 	}
-#pragma unroll
-	for (int o = 16; o > 0; o >>= 1) {
-		sI += __shfl_xor_sync(0xffffffffu, sI, o);
-		sQ += __shfl_xor_sync(0xffffffffu, sQ, o);
-	}
+	sI = warp_sum(sI);
+	sQ = warp_sum(sQ);
 	if ((t & 31) == 0) {
 		red[(t >> 5) * 2 + 0] = (int)sI;
 		red[(t >> 5) * 2 + 1] = (int)sQ;

@@ -22,6 +22,7 @@ CONFIGS = {
     "cfg1": ("100M:102.4M:2400", 0.0, "rectangle", None, 0, 293),
     "cfg4": ("100M:102.4M:19", 0.0, "blackman-harris", None, 1, 256),
     "box28": ("100M:100.1M:100", 0.0, "rectangle", None, 0, 8192),
+    "box14pk": ("100M:100.2M:50", 0.0, "rectangle", None, 1, 4096),  # 4096 bins, ds = 14, peak hold: stream kernel <12,1,2,2>
     "f9": ("100M:100.1M:100", 0.0, "blackman", 9, 0, 8192),
     "rms": ("100M:110M:1M", 0.0, "rectangle", None, 0, 4096),
     "rms1k": ("100M:110M:1M", 0.0, "rectangle", None, 0, 1024),
